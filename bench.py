@@ -2,7 +2,7 @@
 """bench.py — SOS front-end frame-pairs/s on B200 (BASELINE.json metric), with per-kernel roofline fractions and the
 CPU reference path timed beside it.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|tiny] [--batch B]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|tiny] [--batch B] [--dump-outputs DIR]
     python bench.py --impl reference ...          # the reference's CPU path (OpenCV + NumPy) on this box's host cores
 
 A "step" is one pass of the hot path over one batch of B new synthetic frames = B frame pairs (frame i-1 -> frame i):
@@ -331,6 +331,8 @@ def run_gpu(args, rank, local_rank, world):
     launches = ctx.launch_count - launches0
     clocks = sampler.stop()
     stats = fe.buffers()["stats"].cpu().numpy()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(fe.buffers(), args.dump_outputs)
 
     # ---- end to end: pinned host buffers in, poses out, copies overlapped with the previous step's kernels -----------
     fe2 = w.frontend(ctx)
@@ -776,6 +778,37 @@ def run_c4(args, ctx, rank, world, steps=20, warm=3):
     return out
 
 
+DUMP_ARRAY_BYTES = 16 << 20   # per array: the six arrays stay under 64 MB in all
+
+
+def dump_outputs(buf, out_dir):
+    """Write what the last step computed, as a caller of Frontend.step reads it from buffers(), to out_dir/<name>.npy: per
+    frame pair the refitted pose, RANSAC's pose, the stats row (stereo points, correspondences, inliers, winning hypothesis),
+    the inlier mask over the correspondences and the triangulated stereo points of the new frame, and the panoramas.  Rows
+    past a frame's valid count are zeroed, since they hold whatever an earlier step left there.  int32 goes out as float64,
+    the rest as float32 (both exact).  An array above DUMP_ARRAY_BYTES is replaced by a fixed, seeded sample of its elements
+    (flattened, in index order), so the same arguments give the same files from run to run."""
+    import torch
+    B = buf["pose"].shape[0]
+
+    def valid(t, n):
+        keep = torch.arange(t.shape[1], device=t.device)[None, :] < n[:, None]
+        return torch.where(keep.view(keep.shape + (1,) * (t.dim() - 2)), t, torch.zeros((), dtype=t.dtype, device=t.device))
+
+    arrays = {"pose": buf["pose"], "ransac_pose": buf["ransac_pose"], "stats": buf["stats"],
+              "inlier_mask": valid(buf["inlier_mask"], buf["n_corr"]),
+              "points": valid(buf["xyz"][1:B + 1], buf["n"][1:B + 1]),   # slot i + 1 holds frame i of the batch
+              "panoramas": buf["pano"]}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        dtype = torch.float64 if t.dtype == torch.int32 else torch.float32
+        size = 8 if dtype == torch.float64 else 4
+        if t.numel() * size > DUMP_ARRAY_BYTES:
+            idx = np.sort(np.random.default_rng(0).choice(t.numel(), DUMP_ARRAY_BYTES // size, replace=False))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.to(dtype).cpu().numpy())
+
+
 def summarize_kernels(marks, steps):
     """marks: (kernel name, ms) per launch over `steps` eager steps -> average ms per step, keyed `kernel#k` for the k-th
     launch of that kernel within a step (e.g. hamming_mma_kernel#0 = stereo buckets, #1 = temporal matching)."""
@@ -848,7 +881,12 @@ def main():
                     help="share of scene landmarks that move between frames (outliers for RANSAC): 0.79 gives the ~35 %% inlier "
                          "rate SURVEY 8d specifies for config 2; 0 = the clean static scene (~99 %% inliers)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the CPU baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32 / float64, "
+                         "panoramas as a fixed seeded sample, under 64 MB in all) to compare two builds output for output")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.workload in ("c3", "c4")):
+        ap.error("--dump-outputs applies to the frame-pair workloads (c1, c2, tiny) of --impl ours")
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     args.steps_given = args.steps is not None
     if args.steps is None:

@@ -1,5 +1,5 @@
 """CPU: oracle/driver.py (the restatement of the reference's VO loop) against the reference's OWN run_VO
-(pose_est_tools.py:1264-1678), which oracle/gen_vo_golden.py drove unmodified over a rendered 10-frame sequence with a
+(pose_est_tools.py:1264-1678), which oracle/gen_vo_golden.py drove unmodified over a rendered 9-frame sequence with a
 pyopengv stub backed by oracle/p3p.py + oracle/ransac.py.  Fed the features the reference detected, the restated loop must
 produce the same keyframe ids and the same estimated_frame_poses_TUM.txt."""
 import numpy as np
@@ -71,7 +71,7 @@ def test_restated_vo_loop_reproduces_the_reference_run():
     T_ref = [_vo_golden.tum_to_matrix(est[i]) for i in range(n)]
     # per frame: pose relative to its tracking reference (the keyframe current when the frame was tracked) to 2e-7 — the TUM file
     # prints float64 repr, the inputs of RANSAC agree to 1e-9 (checked above), and the Levenberg-Marquardt minimiser is a
-    # function of them; the absolute poses chain up to 9 such links: 2e-6
+    # function of them; the absolute poses chain up to 8 such links: 2e-6
     parent = 0
     for i in range(1, n):
         rel_ref = np.linalg.inv(T_ref[parent]) @ T_ref[i]
