@@ -310,16 +310,33 @@ int sos_ransac_p3d(sos_ctx* ctx, const float* p_ref, const float* p_cur, const f
                    int32_t* best_hyp, int32_t* best_count, uint8_t* inlier_mask, uint64_t* best_key,
                    int32_t* all_counts);
 
-/* Diagnostics of the tensor-core engine of the scores (csrc/score_mma.cuh): sos_ransac_p3d forced onto that engine, which
- * additionally stores what the tensor cores accumulated for every (hypothesis, correspondence) pair:
- * sn [n_problems, n_hyp, ceil(cap/128)*128, 2] float32.  SOS_SCORE_BEARING: (s, N') with s = f . x and N' = |x|^2 + 1.52 max_cam
- * |b|^2, x = Rc^T (R^T (p - t) - tc) (pose_est_tools.py:150-203, 181-185); SOS_SCORE_EUCLID: (s', n2) with s' = |q|^2 - 2 q . x
- * and n2 = |x|^2, q = p_cur, so that s' + n2 = |x - q|^2.  The parity tests bound their error against float64 with it; the
- * guard band of the engine is 4 x that bound. */
+/* Diagnostics of the score engines, two optional outputs (at least one must be given).
+ * sn (may be NULL): sos_ransac_p3d forced onto the tensor-core engine (csrc/score_mma.cuh), which additionally stores what the
+ * tensor cores accumulated for every (hypothesis, correspondence) pair: sn [n_problems, n_hyp, ceil(cap/128)*128, 2] float32.
+ * SOS_SCORE_BEARING: (s, N') with s = f . x and N' = |x|^2 + 1.52 max_cam |b|^2, x = Rc^T (R^T (p - t) - tc)
+ * (pose_est_tools.py:150-203, 181-185); SOS_SCORE_EUCLID: (s', n2) with s' = |q|^2 - 2 q . x and n2 = |x|^2, q = p_cur, so
+ * that s' + n2 = |x - q|^2.  The parity tests bound their error against float64 with it.  With sn NULL the engine is the one
+ * sos_ransac_p3d picks (SOS_SCORE_ENGINE).
+ * stats (may be NULL): DEVICE int32 [SOS_SCORE_STATS], zeroed by the call, then filled with how much work went through the
+ * deferred float64 path of the engine that ran (indices SOS_STAT_*; the other engine's entries stay 0).  Tensor-core engine,
+ * per work item (problem x 128 hypotheses x a range of correspondence tiles): 32-pair chunks with uncertain pairs, queued in
+ * shared memory up to 1536 per item and decided by the scoring thread itself past that; pairs expanded from the queue, in
+ * rounds of at most 2048.  FP32-pipe kernel, per block: (32-correspondence batch, hypothesis) entries with an uncertain pair,
+ * queued up to 2048 per block; a block past that re-decides its whole range in float64.
+ * Counts equal those of sos_ransac_p3d on the same engine. */
+#define SOS_SCORE_STATS 8
+#define SOS_STAT_TC_ITEMS 0              /* tensor-core work items that ran */
+#define SOS_STAT_TC_CHUNKS 1             /* chunks with uncertain pairs, summed over items */
+#define SOS_STAT_TC_CHUNKS_MAX 2         /* largest number of such chunks in one item */
+#define SOS_STAT_TC_CHUNKS_IN_THREAD 3   /* chunks past the 1536 queue entries of their item, decided in-thread */
+#define SOS_STAT_TC_PAIRS 4              /* pairs expanded from the queues and re-decided, summed */
+#define SOS_STAT_TC_ROUNDS_MAX 5         /* largest number of expansion rounds (<= 2048 pairs each) in one item */
+#define SOS_STAT_FMA_ENTRIES 6           /* FP32 kernel: queue entries, summed over blocks, overflowing ones included */
+#define SOS_STAT_FMA_OVERFLOW_BLOCKS 7   /* FP32 kernel: blocks whose queue overflowed */
 int sos_ransac_score_probe(sos_ctx* ctx, const float* p_ref, const float* p_cur, const float* f_cur, const uint8_t* cam,
                            const int32_t* n, int n_problems, int cap, const double* rig, int n_cams, const uint32_t* hyp,
                            int n_hyp, int score_mode, double threshold, float* best_pose, int32_t* best_hyp,
-                           int32_t* best_count, int32_t* all_counts, float* sn);
+                           int32_t* best_count, int32_t* all_counts, float* sn, int32_t* stats);
 
 /* replaces: pyopengv.absolute_pose_noncentral_ransac(bearings, cam_idx, points, cam_offsets, cam_rotations, thr, iters)
  * (pose_est_tools.py:785) and pyopengv.absolute_pose_ransac(bearings, points, algo, thr, iters) (pose_est_tools.py:915)

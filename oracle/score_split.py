@@ -3,9 +3,9 @@
 The engine evaluates the reference's bearing score (pose_est_tools.py:150-203, non-central correction :181-185) as two small-K
 GEMMs in bfloat16: every float32 feature is split into three bfloat16 pieces and six partial products per feature are
 accumulated in float32.  This module restates that arithmetic in NumPy (bfloat16 rounding emulated on the bit pattern,
-float32 accumulation in the order of the K columns), so that the split's exactness and the size of the guard band can be
-checked without a GPU.  The tensor core's internal accumulation order is not specified; the GPU test
-(tests/test_gpu_score_tc.py) measures the real thing."""
+float32 accumulation in the order of the K columns, or one rounding per MMA instruction of 16 columns), so that the split's
+exactness and the size of the guard band can be checked without a GPU.  The tensor core's internal accumulation is not
+specified; the GPU tests (tests/test_gpu_score_tc.py, tests/test_gpu_score_stress.py) measure the real thing."""
 from __future__ import annotations
 
 import numpy as np
@@ -33,15 +33,41 @@ def split3(x: np.ndarray):
     return h, m, l
 
 
-def split_dot(a: np.ndarray, b: np.ndarray) -> np.ndarray:
+def round_f32(x: np.ndarray, mode: str) -> np.ndarray:
+    """float64 -> float32, to nearest ("rn") or toward zero ("tz")."""
+    f = np.asarray(x, np.float64).astype(np.float32)
+    if mode == "tz":
+        over = np.abs(f.astype(np.float64)) > np.abs(x)
+        f[over] = np.nextafter(f[over], np.float32(0))
+    return f
+
+
+def split_dot(a: np.ndarray, b: np.ndarray, accum: str = "column") -> np.ndarray:
     """sum_k a[..., k] * b[..., k] the way the engine forms it: per feature the six products hh, hm, mh, hl, lh, mm (each exact
-    in float32: 8 x 8 mantissa bits), accumulated in float32 column by column."""
+    in float32: 8 x 8 mantissa bits), laid out as six consecutive K columns per feature.
+    accum = "column": float32 accumulation column by column (one rounding per product);
+    accum = "rn16" / "tz16": one rounding per MMA instruction, to nearest / toward zero — the accumulator plus the exact sum
+    of the instruction's 16 K columns (the zero padding of the last one included), which is the hardware model of the band's
+    derivation (csrc/score_mma.cuh)."""
     ah, am, al = split3(a)
     bh, bm, bl = split3(b)
-    acc = np.zeros(np.broadcast_shapes(a.shape, b.shape)[:-1], np.float32)
-    for k in range(a.shape[-1]):
-        for x, y in ((ah, bh), (ah, bm), (am, bh), (ah, bl), (al, bh), (am, bm)):
-            acc = (acc + (x[..., k] * y[..., k]).astype(np.float32)).astype(np.float32)
+    shape = np.broadcast_shapes(a.shape, b.shape)[:-1]
+    if accum == "column":
+        acc = np.zeros(shape, np.float32)
+        for k in range(a.shape[-1]):
+            for x, y in ((ah, bh), (ah, bm), (am, bh), (ah, bl), (al, bh), (am, bm)):
+                acc = (acc + (x[..., k] * y[..., k]).astype(np.float32)).astype(np.float32)
+        return acc
+    if accum not in ("rn16", "tz16"):
+        raise ValueError(accum)
+    prods = [x[..., k].astype(np.float64) * y[..., k].astype(np.float64)
+             for k in range(a.shape[-1]) for x, y in ((ah, bh), (ah, bm), (am, bh), (ah, bl), (al, bh), (am, bm))]
+    acc = np.zeros(shape, np.float32)
+    for s in range(0, len(prods), 16):
+        tot = acc.astype(np.float64)
+        for pr in prods[s:s + 16]:   # products of two bfloat16 values: the float64 sum of 17 terms is exact to 2^-50 or so
+            tot = tot + pr
+        acc = round_f32(tot, accum[:2])
     return acc
 
 

@@ -13,9 +13,9 @@ pytestmark = pytest.mark.gpu
 
 @pytest.fixture(autouse=True, params=["tensor", "fma"])
 def score_engine(request, monkeypatch):
-    """Every test of this file runs with both engines of the bearing score: the bfloat16-split GEMMs on the tensor cores
-    (csrc/score_mma.cuh, default) and the FP32-pipe kernel (SOS_SCORE_ENGINE=fma; the library reads the switch per call).
-    The Euclidean score only has the FP32-pipe kernel."""
+    """Every test of this file runs with both engines of the scores, bearing and Euclidean: the bfloat16-split GEMMs on the
+    tensor cores (csrc/score_mma.cuh, default) and the FP32-pipe kernel (SOS_SCORE_ENGINE=fma; the library reads the switch
+    per call)."""
     if request.param == "fma":
         monkeypatch.setenv("SOS_SCORE_ENGINE", "fma")
     else:

@@ -55,7 +55,7 @@ PROTOTYPES = {
     "sos_arun_batch": (I, [c_ctx, P, P, I, I, I, P, P]),
     "sos_pixel_gate": (I, [c_ctx, P, P, I, D, D, P]),
     "sos_ransac_p3d": (I, [c_ctx, P, P, P, P, P, I, I, P, I, P, I, I, I, D, P, P, P, P, P, P]),
-    "sos_ransac_score_probe": (I, [c_ctx, P, P, P, P, P, I, I, P, I, P, I, I, D, P, P, P, P, P]),
+    "sos_ransac_score_probe": (I, [c_ctx, P, P, P, P, P, I, I, P, I, P, I, I, D, P, P, P, P, P, P]),
     "sos_ransac_p3p": (I, [c_ctx, P, P, P, P, I, I, P, I, P, I, I, D, P, P, P, P, P, P]),
     "sos_ransac_p3d_eval": (I, [c_ctx, P, P, P, P, P, I, I, P, I, P, I, D, P, P, P]),
     "sos_refit_inliers": (I, [c_ctx, P, P, P, P, I, I, P, P]),

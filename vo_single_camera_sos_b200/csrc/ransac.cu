@@ -29,52 +29,48 @@ namespace {
 // ------------------------------------------------------------------------------------------------------------
 // float64 3x3 helpers (row-major)
 // ------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void jacobi_rotate(double* S, double* V, int p, int q) {
-  const double apq = S[p * 3 + q];
-  if (apq == 0.0) return;
-  const double app = S[p * 3 + p], aqq = S[q * 3 + q];
-  const double tau = (aqq - app) / (2.0 * apq);
-  const double t = (tau >= 0.0 ? 1.0 : -1.0) / (fabs(tau) + sqrt(1.0 + tau * tau));
-  const double c = 1.0 / sqrt(1.0 + t * t), s = t * c;
-  // S <- J^T S J
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const double skp = S[k * 3 + p], skq = S[k * 3 + q];
-    S[k * 3 + p] = c * skp - s * skq;
-    S[k * 3 + q] = s * skp + c * skq;
-  }
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const double spk = S[p * 3 + k], sqk = S[q * 3 + k];
-    S[p * 3 + k] = c * spk - s * sqk;
-    S[q * 3 + k] = s * spk + c * sqk;
-  }
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-    const double vkp = V[k * 3 + p], vkq = V[k * 3 + q];
-    V[k * 3 + p] = c * vkp - s * vkq;
-    V[k * 3 + q] = s * vkp + c * vkq;
-  }
-}
-
 // Rotation R (det +1) maximising trace(R^T ... ) for covariance Hm = sum v1_i v0_i^T, i.e. U diag(1,1,det(U V^T)) V^T of
 // Hm = U S V^T (transformations.py:942-953).  Returns false when the second singular value vanishes (rank < 2).
+// V comes from one-sided (Hestenes) Jacobi on the columns of Hm, not from the eigenvectors of Hm^T Hm: forming Hm^T Hm squares
+// the ratio of the singular values, so for a thin sample triangle (sigma2 / sigma1 ~ 1e-2) the second singular vector, and
+// with it the pose, lost six digits against the float64 SVD of the oracle and inlier counts differed from it.
 __device__ bool kabsch_rotation(const double* Hm, double* R) {
-  double S[9], V[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
+  double A[9], V[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
 #pragma unroll
-  for (int i = 0; i < 3; ++i)
+  for (int i = 0; i < 9; ++i) A[i] = Hm[i];
+  for (int sweep = 0; sweep < 30; ++sweep) {
+    bool rotated = false;
 #pragma unroll
-    for (int j = 0; j < 3; ++j) S[i * 3 + j] = Hm[0 * 3 + i] * Hm[0 * 3 + j] + Hm[1 * 3 + i] * Hm[1 * 3 + j] + Hm[2 * 3 + i] * Hm[2 * 3 + j];
-  for (int sweep = 0; sweep < 12; ++sweep) {
-    const double off = fabs(S[1]) + fabs(S[2]) + fabs(S[5]);
-    const double diag = fabs(S[0]) + fabs(S[4]) + fabs(S[8]);
-    if (off <= 1e-300 || off <= 1e-22 * diag) break;
-    jacobi_rotate(S, V, 0, 1);
-    jacobi_rotate(S, V, 0, 2);
-    jacobi_rotate(S, V, 1, 2);
+    for (int pq = 0; pq < 3; ++pq) {
+      const int p = pq == 2 ? 1 : 0, q = pq == 0 ? 1 : 2;
+      double alpha = 0.0, beta = 0.0, gamma = 0.0;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        alpha += A[k * 3 + p] * A[k * 3 + p];
+        beta += A[k * 3 + q] * A[k * 3 + q];
+        gamma += A[k * 3 + p] * A[k * 3 + q];
+      }
+      if (!(fabs(gamma) > 1e-15 * sqrt(alpha * beta))) continue;   // columns orthogonal to working precision
+      rotated = true;
+      const double zeta = (beta - alpha) / (2.0 * gamma);
+      const double t = (zeta >= 0.0 ? 1.0 : -1.0) / (fabs(zeta) + sqrt(1.0 + zeta * zeta));
+      const double c = 1.0 / sqrt(1.0 + t * t), s = t * c;
+#pragma unroll
+      for (int k = 0; k < 3; ++k) {
+        const double ap = A[k * 3 + p], aq = A[k * 3 + q];
+        A[k * 3 + p] = c * ap - s * aq;
+        A[k * 3 + q] = s * ap + c * aq;
+        const double vp = V[k * 3 + p], vq = V[k * 3 + q];
+        V[k * 3 + p] = c * vp - s * vq;
+        V[k * 3 + q] = s * vp + c * vq;
+      }
+    }
+    if (!rotated) break;
   }
-  // pick the two largest eigenvalues
-  double lam[3] = {S[0], S[4], S[8]};
+  // pick the two largest singular values (squared: the column norms of Hm V)
+  double lam[3];
+#pragma unroll
+  for (int j = 0; j < 3; ++j) lam[j] = A[j] * A[j] + A[3 + j] * A[3 + j] + A[6 + j] * A[6 + j];
   int i0 = 0;
   if (lam[1] > lam[i0]) i0 = 1;
   if (lam[2] > lam[i0]) i0 = 2;
@@ -704,7 +700,7 @@ template <int MODE, int HPT, int CHUNK, int MINB>
 __global__ void __launch_bounds__(RS_THREADS, MINB)
 score_kernel(const float* __restrict__ p_ref, const float* __restrict__ q_arr, const uint8_t* __restrict__ cam,
              const int32_t* __restrict__ n_arr, int cap, const HypRec* __restrict__ recs, int n_hyp, ScoreConst k,
-             const __grid_constant__ Rig rig, int32_t* __restrict__ counts) {
+             const __grid_constant__ Rig rig, int32_t* __restrict__ counts, int32_t* __restrict__ stats) {
   __shared__ PointRec pts[CHUNK];
   __shared__ unsigned char pcam[CHUNK];
   __shared__ float pguard[CHUNK];
@@ -809,7 +805,11 @@ score_kernel(const float* __restrict__ p_ref, const float* __restrict__ q_arr, c
   }
   __syncthreads();
   int nq = queue_n;
-  if (nq > RS_QCAP) {  // block-uniform; queue overflow has never been observed: redo the whole chunk in float64
+  if (stats && threadIdx.x == 0) {   // sos_ransac_score_probe
+    atomicAdd(&stats[SOS_STAT_FMA_ENTRIES], nq);
+    if (nq > RS_QCAP) atomicAdd(&stats[SOS_STAT_FMA_OVERFLOW_BLOCKS], 1);
+  }
+  if (nq > RS_QCAP) {  // block-uniform; near-threshold pairs in most batches of most hypotheses: redo the whole chunk in float64
     nq = 0;
 #pragma unroll 1
     for (int r = 0; r < HPT; ++r) {
@@ -1072,7 +1072,7 @@ bool use_tensor_score(int score_mode, int n_hyp, int cap) {
 }
 
 int launch_score_tc(sos_ctx* ctx, int mode, const Rig& rig, const RansacScratch& s, const float* p_ref, const float* f_cur, const uint8_t* cam,
-                    const int32_t* n, int n_problems, int cap, int n_hyp, ScoreConst k, float* probe) {
+                    const int32_t* n, int n_problems, int cap, int n_hyp, ScoreConst k, float* probe, int32_t* stats) {
   using namespace score_tc;
   const int ht = sos_div_up(n_hyp, TILE), ct = sos_div_up(cap, TILE);
   corr_expand_kernel<<<dim3(ct, n_problems), TILE, 0, ctx->stream>>>(mode, p_ref, f_cur, cam, n, cap, rig.n_cams, ct, s.tc_b, s.tc_meta);
@@ -1098,11 +1098,12 @@ int launch_score_tc(sos_ctx* ctx, int mode, const Rig& rig, const RansacScratch&
     splits = best;
   }
   a.splits = splits;
-  a.recs = s.recs; a.counts = s.counts; a.p_ref = p_ref; a.f_cur = f_cur; a.cam = cam; a.k = k; a.probe = probe;
+  a.recs = s.recs; a.counts = s.counts; a.p_ref = p_ref; a.f_cur = f_cur; a.cam = cam; a.k = k; a.probe = probe; a.stats = stats;
   static bool attr_set[64][4] = {};     // per device: the opt-in to > 48 KB of dynamic shared memory
   const bool euclid = mode == SOS_SCORE_EUCLID;
-  const int dev = ctx->device & 63, v = (probe ? 1 : 0) + (euclid ? 2 : 0);
-  auto kern = probe ? (euclid ? score_mma_kernel<true, SOS_SCORE_EUCLID> : score_mma_kernel<true, SOS_SCORE_BEARING>)
+  const bool diag = probe || stats;
+  const int dev = ctx->device & 63, v = (diag ? 1 : 0) + (euclid ? 2 : 0);
+  auto kern = diag ? (euclid ? score_mma_kernel<true, SOS_SCORE_EUCLID> : score_mma_kernel<true, SOS_SCORE_BEARING>)
                     : (euclid ? score_mma_kernel<false, SOS_SCORE_EUCLID> : score_mma_kernel<false, SOS_SCORE_BEARING>);
   if (!attr_set[dev][v]) {
     SOS_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
@@ -1116,12 +1117,12 @@ int launch_score_tc(sos_ctx* ctx, int mode, const Rig& rig, const RansacScratch&
 
 template <int MODE>
 int launch_score(sos_ctx* ctx, const Rig& rig, dim3 grid, const float* p_ref, const float* q, const uint8_t* cam,
-                 const int32_t* n, int cap, const HypRec* recs, int n_hyp, ScoreConst k, int32_t* counts) {
+                 const int32_t* n, int cap, const HypRec* recs, int n_hyp, ScoreConst k, int32_t* counts, int32_t* stats) {
   // 4 hypotheses per thread, 512 correspondences per block, 4 blocks per SM.  Measured against higher-occupancy shapes in
   // round 2 (profiles/r02/score_variants_and_ring_depth_ab.log: 2 hypotheses per thread with 6-8 blocks per SM, 256-point
   // chunks): all slower (0.74 - 0.81 ms against 0.72 ms) — fewer hypotheses per shared-memory read and more block prologues
   // cost more than the extra warps hide.
-  score_kernel<MODE, RS_HPT, RS_CHUNK, 4><<<grid, RS_THREADS, 0, ctx->stream>>>(p_ref, q, cam, n, cap, recs, n_hyp, k, rig, counts);
+  score_kernel<MODE, RS_HPT, RS_CHUNK, 4><<<grid, RS_THREADS, 0, ctx->stream>>>(p_ref, q, cam, n, cap, recs, n_hyp, k, rig, counts, stats);
   SOS_LAUNCHED_AS(ctx, "score_kernel");
   return SOS_OK;
 }
@@ -1146,7 +1147,8 @@ int ransac_run(sos_ctx* ctx, int solver, const float* p_ref, const float* p_cur,
                               const uint8_t* cam, const int32_t* n, int n_problems, int cap, const double* rig,
                               int n_cams, const uint32_t* hyp, int n_hyp, int hyp_offset, int score_mode,
                               double threshold, float* best_pose, int32_t* best_hyp, int32_t* best_count,
-                              uint8_t* inlier_mask, uint64_t* best_key, int32_t* all_counts, float* tc_probe = nullptr) {
+                              uint8_t* inlier_mask, uint64_t* best_key, int32_t* all_counts, float* tc_probe = nullptr,
+                              int32_t* stats = nullptr) {
   SOS_CHECK_ARG(ctx, "ctx is NULL");
   SOS_CHECK_ARG(n_problems >= 0 && cap >= 0 && n_hyp >= 0, "negative size");
   SOS_CHECK_ARG(score_mode == SOS_SCORE_EUCLID || score_mode == SOS_SCORE_BEARING, "unknown score mode");
@@ -1164,6 +1166,7 @@ int ransac_run(sos_ctx* ctx, int solver, const float* p_ref, const float* p_cur,
   RansacScratch s;
   const int n_hyp_alloc = n_hyp > 0 ? n_hyp : 1;
   const bool tc = tc_probe != nullptr || use_tensor_score(score_mode, n_hyp, cap);
+  if (stats) SOS_CUDA(cudaMemsetAsync(stats, 0, SOS_SCORE_STATS * sizeof(int32_t), ctx->stream));
   int rc = ransac_scratch(ctx, n_problems, n_hyp_alloc, tc ? cap : 0, s);
   if (rc != SOS_OK) return rc;
   if (n_hyp > 0) {
@@ -1175,14 +1178,14 @@ int ransac_run(sos_ctx* ctx, int solver, const float* p_ref, const float* p_cur,
     SOS_LAUNCHED_AS(ctx, "hypothesize_kernel");
     if (cap > 0 && tc) {
       rc = launch_score_tc(ctx, score_mode, r, s, p_ref, score_mode == SOS_SCORE_EUCLID ? p_cur : f_cur, cam, n, n_problems, cap, n_hyp, k,
-                           tc_probe);
+                           tc_probe, stats);
       if (rc != SOS_OK) return rc;
     } else if (cap > 0) {
       dim3 sgrid(sos_div_up(n_hyp, RS_TILE_H), sos_div_up(cap, RS_CHUNK), n_problems);
       const float* q = score_mode == SOS_SCORE_EUCLID ? p_cur : f_cur;
       rc = score_mode == SOS_SCORE_EUCLID
-               ? launch_score<SOS_SCORE_EUCLID>(ctx, r, sgrid, p_ref, q, cam, n, cap, s.recs, n_hyp, k, s.counts)
-               : launch_score<SOS_SCORE_BEARING>(ctx, r, sgrid, p_ref, q, cam, n, cap, s.recs, n_hyp, k, s.counts);
+               ? launch_score<SOS_SCORE_EUCLID>(ctx, r, sgrid, p_ref, q, cam, n, cap, s.recs, n_hyp, k, s.counts, stats)
+               : launch_score<SOS_SCORE_BEARING>(ctx, r, sgrid, p_ref, q, cam, n, cap, s.recs, n_hyp, k, s.counts, stats);
       if (rc != SOS_OK) return rc;
     }
   }
@@ -1215,10 +1218,10 @@ extern "C" int sos_ransac_score_probe(sos_ctx* ctx, const float* p_ref, const fl
                                       const uint8_t* cam, const int32_t* n, int n_problems, int cap, const double* rig,
                                       int n_cams, const uint32_t* hyp, int n_hyp, int score_mode, double threshold,
                                       float* best_pose, int32_t* best_hyp, int32_t* best_count, int32_t* all_counts,
-                                      float* sn) {
-  SOS_CHECK_ARG(sn, "sn is NULL");
+                                      float* sn, int32_t* stats) {
+  SOS_CHECK_ARG(sn || stats, "sn and stats are both NULL");
   return ransac_run(ctx, 0, p_ref, p_cur, f_cur, cam, n, n_problems, cap, rig, n_cams, hyp, n_hyp, 0, score_mode,
-                    threshold, best_pose, best_hyp, best_count, nullptr, nullptr, all_counts, sn);
+                    threshold, best_pose, best_hyp, best_count, nullptr, nullptr, all_counts, sn, stats);
 }
 
 extern "C" int sos_ransac_p3p(sos_ctx* ctx, const float* p_ref, const float* f_cur, const uint8_t* cam, const int32_t* n,

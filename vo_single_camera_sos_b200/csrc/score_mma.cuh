@@ -22,8 +22,20 @@
 //     one FFMA (s|s| + a constant of the hypothesis), one packed FFMA2 per two pairs for each of t = D - band and
 //     u = D + band, and two SHF that collect their sign bits; 32 pairs are counted with one POPC.
 // Exactness: a band bounds the error of D from the split, the accumulation and the two float32 operations:
-// |err D| <= BAND_REL (|p|^2 + |b|^2) (measured on every pair of the test problems by tests/test_gpu_score_tc.py through the
-// PROBE instantiation: 1.4e-6, BAND_REL is 9 x that).  Since x = A p + b with A orthogonal, |p|^2 <= 2 n2 + 2 |b|^2, so the
+// |err D| <= BAND_REL (|p|^2 + |b|^2).  Worst-case model (u = 2^-24; T = the sum of |terms| of an accumulator):
+//   * float32 features: the hypothesis feature and the correspondence feature are each one rounding of a float64 value: 2u T;
+//   * the split: the dropped products mid*lo, lo*mid, lo*lo are below 2^-24 + 2^-24 + 2^-32 of a term: 2u T;
+//   * accumulation — the HARDWARE ASSUMPTION, not documented by NVIDIA: each tcgen05.mma kind::f16 instruction adds the exact
+//     sum of its 16 products to the float32 accumulator and rounds once, to nearest (e = u) or toward zero (e = 2u); every
+//     partial sum is at most T, so m instructions add m e T (m = 5 for s, 4 for n2).
+//   So |err s| <= (4u + 5e) T_s and |err n2| <= (4u + 4e) T_n.  Bearing score (|f| = 1, A orthogonal, b of the pair's camera,
+//   B = max_cam |b|, S = |p|^2 + B^2): T_s <= sqrt(3) |p| + |b|, |s| <= |p| + |b|, hence |err s|s|| <= 2|s| |err s| <=
+//   6.2 S (4u + 5e); T_n <= (|p| + |b|)^2 + 1.52 B^2 <= 3.52 S; the epilogue adds the rounding of w (3.52 u S), of the constants
+//   c^2 + BETA (2 x 3.52 u S) and of K_h against the shift inside N' (12.2 u S; the rounding of t itself cannot flip its sign).
+//   Total 107 u S = 6.4e-6 S (0.49 BAND_REL) to nearest, 152 u S = 9.1e-6 S (0.70 BAND_REL) toward zero.
+//   Measured through the PROBE instantiation on every pair of the test problems (tests/test_gpu_score_tc.py,
+//   tests/test_gpu_score_stress.py: large motion, far points, points at the camera centre, s ~ 0 and s < 0, millimetres)
+//   the error stays below a quarter of BAND_REL, which those tests assert.  Since x = A p + b with A orthogonal, |p|^2 <= 2 n2 + 2 |b|^2, so the
 // band is at most BETA n2 + G_h with BETA = 2 BAND_REL and G_h = 3 BAND_REL |b_h|^2 = BETA * 1.5 |b_h|^2.  The constant of
 // the hypothesis rides through the MMA: the n2 GEMM delivers N' = n2 + 1.5 |b_h|^2 (added to the hypothesis feature that
 // multiplies the correspondence's constant 1), so the band is BETA N' and D = (s|s| + c^2 1.5 |b_h|^2) - c^2 N':
@@ -34,7 +46,10 @@
 // Euclidean score (|A p + b - q| < thr, q = the current frame's 3D point): r^2 = s' + n2 with s' = |q|^2 - 2 q.(A p + b) — the
 // same 13 hypothesis features against (-2 q_i p_k, -2 q_i, |q|^2) — and the same n2 GEMM, so both scores share tiles, MMA
 // issue and pipeline; only the correspondence features and the epilogue arithmetic differ.  r^2 is a difference of large
-// terms, so its band scales with |p|^2 + |q|^2 + |b|^2, not with r^2 — but both accumulators bound those: |p|^2 <= 2 n2 +
+// terms, so its band scales with |p|^2 + |q|^2 + |b|^2 =: S, not with r^2 (worst case, model above: T_s' <= 2 sqrt(3) |q||p| +
+// 2 |q||b| + |q|^2 <= 3.73 S and T_n <= (|p| + |b|)^2 <= 2 S, so |err r^2| <= 49.6 u S = 3.0e-6 S (0.59 BAND_EUCLID) to nearest,
+// 76.2 u S = 4.5e-6 S (0.91 BAND_EUCLID) toward zero; the epilogue's roundings scale with r^2 and thr^2, far inside the band's
+// 2 B r^2 term; measured below a quarter of the band, as for the bearing score) — but both accumulators bound S: |p|^2 <= 2 n2 +
 // 2 |b|^2 and, because r^2 = |q - x|^2 >= (|q| - |x|)^2, |q|^2 <= 2 n2 + 2 r^2.  So band <= B (4 n2 + 2 r^2 + 3 |b_h|^2) per
 // pair: t = (thr^2 - 3B|b|^2) - (1 + 2B) r^2 - 4B n2 >= 0 is a certain inlier, u = (thr^2 + 3B|b|^2) - (1 - 2B) r^2 + 4B n2 < 0
 // a certain outlier.
@@ -65,12 +80,11 @@ constexpr int ECAP = 1536;                      // chunks with uncertain pairs p
 constexpr int PCAP = 2048;                      // uncertain pairs expanded per round of the deferred pass
 constexpr int SMEM_BYTES = (2 + STAGES) * TILE_BYTES + 256 + ECAP * 8 + PCAP * 4 + TILE * 4;
 constexpr float PAD_N2 = 1e30f;                 // n2 feature of a padding correspondence: D = -c^2 1e30, a certain outlier
-// |err D| <= BAND_REL (|p|^2 + max_cam |b|^2): 13 eps + 5e-7 with eps = 2^-20 for the relative error of an accumulated term
-// sum (tests/test_gpu_score_tc.py measures 1.4e-6 for the whole expression and asserts a 4x margin)
+// |err D| <= BAND_REL (|p|^2 + max_cam |b|^2) (derivation at the top of this file: worst case 0.49 / 0.70 of it for rounding to
+// nearest / toward zero per MMA instruction; the tests measure below a quarter of it and assert that)
 constexpr float BAND_REL = 13.0f * 9.5367431640625e-07f + 5e-7f;
 constexpr float BETA = 2.02f * BAND_REL;        // band <= BETA (n2 + B2_SHIFT |b|^2)
-// Euclidean score: |err r^2| <= BAND_EUCLID (|p|^2 + |q|^2 + |b|^2); tests/test_gpu_score_tc.py measures 5.8e-7 (the sum has
-// fewer and better conditioned terms than the bearing score's D) and asserts the 4x margin
+// Euclidean score: |err r^2| <= BAND_EUCLID (|p|^2 + |q|^2 + |b|^2) (worst case 0.59 / 0.91 of it; measured below a quarter)
 constexpr float BAND_EUCLID = 5e-6f;
 constexpr double B2_SHIFT = 1.52;               // (3 / 2 of the derivation, padded for the float32 rounding of |b|^2 in the epilogue)
 
@@ -232,7 +246,8 @@ struct Args {
   const float *p_ref, *f_cur;   // f_cur: bearings, or the current frame's points (Euclidean score)
   const uint8_t* cam;
   ScoreConst k;
-  float* probe;          // PROBE: (s, N') of every pair, [problem][hypothesis][ct * 128][2]
+  float* probe;          // PROBE (may be NULL): (s, N') of every pair, [problem][hypothesis][ct * 128][2]
+  int32_t* stats;        // PROBE (may be NULL): deferred-path counters, SOS_SCORE_STATS layout (include/sosfront.h)
 };
 
 // one deferred pair, decided exactly like score_kernel's deferred pass
@@ -436,7 +451,7 @@ __global__ void __launch_bounds__(THREADS, 1) score_mma_kernel(const Args a, con
           mt = __funnelshift_l(__float_as_uint(t.y), mt, 1);
           mu = __funnelshift_l(__float_as_uint(u.x), mu, 1);
           mu = __funnelshift_l(__float_as_uint(u.y), mu, 1);
-          if (PROBE && valid_h) {
+          if (PROBE && valid_h && a.probe) {
             float* o = a.probe + (((size_t)b * a.n_hyp + h) * ((size_t)a.ct * TILE) + (size_t)k * TILE + chunk * 32 + i) * 2;
             o[0] = s0; o[1] = n2.x; o[2] = s1; o[3] = n2.y;
           }
@@ -449,7 +464,7 @@ __global__ void __launch_bounds__(THREADS, 1) score_mma_kernel(const Args a, con
           if (slot < ECAP) {
             qent[slot] = ((uint32_t)k << 9) | ((uint32_t)chunk << 7) | (uint32_t)row;
             qmask[slot] = unsure;
-          } else {   // queue full (never observed): this thread decides its uncertain pairs on its own
+          } else {   // queue full (far-field Euclidean batches): this thread decides its uncertain pairs on its own
             for (int i = 0; i < 32; ++i)
               if ((unsure >> (31 - i)) & 1u) cnt += exact_pair<MODE>(a, rig, b, h, k * TILE + chunk * 32 + i, n);
           }
@@ -462,6 +477,7 @@ __global__ void __launch_bounds__(THREADS, 1) score_mma_kernel(const Args a, con
     const int te = tid;
     asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
     const int nq = min(*q_n, ECAP);
+    int rounds = 0, expanded = 0;   // PROBE statistics
     for (bool more = nq > 0; more;) {
       if (te == 0) *p_n = 0;
       asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
@@ -484,7 +500,18 @@ __global__ void __launch_bounds__(THREADS, 1) score_mma_kernel(const Args a, con
         if (exact_pair<MODE>(a, rig, b, ht * TILE + r, k * TILE + chunk * 32 + (int)(v & 31u), n)) atomicAdd(&fixcnt[r], 1);
       }
       more = np > PCAP;
+      ++rounds;
+      expanded += min(np, PCAP);
       asm volatile("bar.sync 1, %0;" ::"n"(EPI_WARPS * 32) : "memory");
+    }
+    if (PROBE && a.stats && te == 0) {
+      const int queued = *q_n;
+      atomicAdd(&a.stats[SOS_STAT_TC_ITEMS], 1);
+      atomicAdd(&a.stats[SOS_STAT_TC_CHUNKS], queued);
+      atomicMax(&a.stats[SOS_STAT_TC_CHUNKS_MAX], queued);
+      atomicAdd(&a.stats[SOS_STAT_TC_CHUNKS_IN_THREAD], max(queued - ECAP, 0));
+      atomicAdd(&a.stats[SOS_STAT_TC_PAIRS], expanded);
+      atomicMax(&a.stats[SOS_STAT_TC_ROUNDS_MAX], rounds);
     }
     if (g == 0) cnt += fixcnt[row];
     if (valid_h && cnt != 0) atomicAdd(&a.counts[(size_t)b * a.n_hyp + h], cnt);

@@ -541,10 +541,14 @@ class Context:
         return pose, best_hyp, best_count, mask, key
 
     def ransac_score_probe(self, p_ref, p_cur, f_cur, n, hyp, threshold: float, cam=None, rig=None, n_cams: int = 0,
-                           score_mode: int = 1):
-        """A score on the tensor-core engine, dumping its two accumulators per pair (sos_ransac_score_probe).
-        Returns (all_counts [B, H] int32, sn [B, H, ceil(cap / 128) * 128, 2] float32)."""
+                           score_mode: int = 1, want_sn: bool = True, stats=None):
+        """Diagnostics of the score engines (sos_ransac_score_probe).  want_sn: run on the tensor-core engine and dump its two
+        accumulators per pair; otherwise the engine is the one ransac_p3d picks.  stats: an optional DEVICE int32 tensor of
+        SOS_SCORE_STATS (8) entries that receives the deferred-path counters (include/sosfront.h, SOS_STAT_*).
+        Returns (all_counts [B, H] int32, sn [B, H, ceil(cap / 128) * 128, 2] float32 or None)."""
         self._sync_stream()
+        if not want_sn and stats is None:
+            raise ValueError("ransac_score_probe needs want_sn or stats")
         B, cap, _ = p_ref.shape
         H = hyp.shape[0]
         r, n_cams = self._rig(rig, n_cams)
@@ -552,12 +556,15 @@ class Context:
         best_hyp = self.empty((B,), torch.int32)
         best_count = self.empty((B,), torch.int32)
         counts = self.empty((B, H), torch.int32)
-        sn = torch.zeros((B, H, (cap + 127) // 128 * 128, 2), dtype=torch.float32, device=self.device)
+        sn = torch.zeros((B, H, (cap + 127) // 128 * 128, 2), dtype=torch.float32, device=self.device) if want_sn else None
+        if stats is not None and stats.numel() != 8:
+            raise ValueError("stats must hold SOS_SCORE_STATS = 8 int32 entries")
         check(self.lib.sos_ransac_score_probe(
             self._h, self._t(p_ref, torch.float32, "p_ref"), self._t(p_cur, torch.float32, "p_cur"),
             self._t(f_cur, torch.float32, "f_cur", optional=True), self._t(cam, torch.uint8, "cam", optional=True),
             self._t(n, torch.int32, "n"), B, cap, _ptr(r), n_cams, self._t(hyp, torch.int32, "hyp"), H, int(score_mode),
-            float(threshold), pose.data_ptr(), best_hyp.data_ptr(), best_count.data_ptr(), counts.data_ptr(), sn.data_ptr()))
+            float(threshold), pose.data_ptr(), best_hyp.data_ptr(), best_count.data_ptr(), counts.data_ptr(),
+            sn.data_ptr() if want_sn else None, self._t(stats, torch.int32, "stats", optional=True)))
         return counts, sn
 
     def ransac_p3p(self, p_ref, f_cur, n, hyp, threshold: float, cam=None, rig=None, n_cams: int = 0, hyp_offset: int = 0,
