@@ -84,7 +84,8 @@ int sos_memset(sos_ctx* ctx, void* dst_dev, int value, size_t bytes);
  *   bits 32..36  ax  = cvRound(32*map_x) & 31        bits 37..41  ay = cvRound(32*map_y) & 31
  *   bits 48..51  tap i lies inside the source image  (i = 0:(y0,x0) 1:(y0,x0+1) 2:(y0+1,x0) 3:(y0+1,x0+1))
  *   bits 52..55  tap i is inside AND its mask byte is non-zero (mask == NULL: same as inside)
- *   bit  56      all four taps usable and the 16-byte windows of the 3-channel fast path end inside the image
+ *   bit  56      all four taps usable and the 16 bytes from tap 2 of a 3-channel frame lie inside it: gates the
+ *                fast taps of remap3b_kernel (aligned 32-bit window loads)
  * NaN / |32*x| >= 2^31 map to INT_MIN exactly as cvtps2dq does inside cv::remap. */
 typedef uint64_t sos_lut_entry;
 

@@ -1,8 +1,7 @@
 #!/usr/bin/env python
 """Kernel micro-benchmarks at C2 sizes (CUDA events, warm-up, inputs rotated): python scripts/kbench.py [hamming|ransac|remap|dense|rgbd|all]
 
-Variants are selected through environment variables read once per process (SOS_HAMMING_VARIANT, SOS_REMAP_BYTE_LOADS),
-so A/B runs are separate processes.  Prints one JSON line per kernel.
+Prints one JSON line per kernel and input variant.
 """
 import json
 import os
@@ -40,7 +39,7 @@ def bench_hamming(ctx, popc_peak, n=4500, segs=32, top2=False):
     ms = timeit(lambda: ctx.hamming_top2(q, t, start, ln, start, ln, cap, cap, want_second=top2, out=out))
     pairs = segs * n * n
     tp = pairs * 8 / (ms * 1e-3) / 1e12
-    return dict(kernel="hamming", variant=os.environ.get("SOS_HAMMING_VARIANT", "default"), top2=top2, ms=ms,
+    return dict(kernel="hamming", top2=top2, ms=ms,
                 pairs_per_s=pairs / (ms * 1e-3), tpopc_equiv=tp, frac_of_popc_peak=tp / popc_peak)
 
 
@@ -97,9 +96,12 @@ def bench_ransac(ctx, ffma_peak, n=8700, B=16, H=4096, mode=ops.SCORE_BEARING):
                 tflops=fl / (ms * 1e-3) / 1e12, frac_of_ffma_peak=fl / (ms * 1e-3) / 1e12 / ffma_peak)
 
 
-def bench_remap(ctx, hbm_peak, B=16, H=2048, W=2048, rows=849, cols=2400):
+def bench_remap(ctx, hbm_peak, B=16, H=2048, W=2048, rows=849, cols=2400, offset=False):
+    """offset: the sources start one byte into their buffers, so the generic remap_kernel<3> runs instead of remap3b_kernel
+    (which needs a 4-byte aligned source with src_w % 4 == 0)."""
     g = torch.Generator(device="cuda").manual_seed(2)
-    srcs = [torch.randint(0, 256, (B, H, W, 3), dtype=torch.uint8, device="cuda", generator=g) for _ in range(2)]
+    n, o = B * H * W * 3, int(offset)
+    srcs = [torch.randint(0, 256, (n + o,), dtype=torch.uint8, device="cuda", generator=g)[o:].view(B, H, W, 3) for _ in range(2)]
     # annular LUTs like the real ones: pano (r, c) -> circle of radius growing with r
     r = torch.arange(rows, device="cuda", dtype=torch.float64)[:, None]
     c = torch.arange(cols, device="cuda", dtype=torch.float64)[None, :]
@@ -120,7 +122,7 @@ def bench_remap(ctx, hbm_peak, B=16, H=2048, W=2048, rows=849, cols=2400):
     ms = timeit(run)
     alg = B * (2 * rows * cols * (8 + 3) + H * W * 3)
     dram = B * (2 * rows * cols * 3 + H * W * 3)
-    return dict(kernel="remap", byte_loads=bool(os.environ.get("SOS_REMAP_BYTE_LOADS")), ms=ms, gbps_algorithmic=alg / (ms * 1e-3) / 1e9,
+    return dict(kernel="remap", src_w=W, src_offset=o, ms=ms, gbps_algorithmic=alg / (ms * 1e-3) / 1e9,
                 frac_of_hbm_peak=alg / (ms * 1e-3) / 1e9 / hbm_peak, gbps_src_plus_dst=dram / (ms * 1e-3) / 1e9)
 
 
@@ -162,6 +164,8 @@ def main():
         res.append(bench_ransac(ctx, pk, mode=ops.SCORE_EUCLID))
     if what in ("remap", "all"):
         res.append(bench_remap(ctx, 6451.2))
+        res.append(bench_remap(ctx, 6451.2, offset=True))
+        res.append(bench_remap(ctx, 6451.2, W=2046))   # rows not a multiple of 4 bytes: generic kernel from an aligned source
     if what in ("dense", "all"):
         res.append(bench_dense(ctx, 6451.2))
     if what in ("rgbd", "all"):

@@ -13,8 +13,6 @@
 // Layout: block = 8 warps = 8 panorama rows x 128 columns, a thread owns 4 consecutive pixels, so LUT reads
 // are 2 x LDG.128 per thread, stores are 4*ch contiguous bytes per thread, and neighbouring rows/columns of
 // the tile hit the same source cache lines in L1.
-#include <stdlib.h>
-
 #include "sos_common.cuh"
 
 namespace {
@@ -50,7 +48,8 @@ lut_pack_kernel(const T* __restrict__ map_x, const T* __restrict__ map_y, int n,
       if (mask == nullptr || mask[(size_t)y * src_w + x] != 0) live |= 1u << tap;
     }
   }
-  // bit 56: all four taps usable AND the two 16-byte windows the 3-channel fast path loads stay inside the image
+  // bit 56: all four taps usable AND the 16 bytes from tap 2 of a 3-channel frame lie inside it; gates remap3b_kernel's
+  // fast taps, whose three aligned 32-bit loads per tap row end at most 12 bytes past the tap
   uint32_t wide3 = 0;
   if (live == 15u) {
     const long long p1 = (((long long)y0 + 1) * src_w + x0) * 3;
@@ -61,44 +60,16 @@ lut_pack_kernel(const T* __restrict__ map_x, const T* __restrict__ map_y, int n,
   lut[i] = lo | (hi << 32);
 }
 
-struct Px4 {
-  uint32_t acc[4];
-};
-
 template <int CH>
 __device__ __forceinline__ void load_tap(const uint8_t* __restrict__ p, uint32_t w, uint32_t* acc) {
 #pragma unroll
   for (int c = 0; c < CH; ++c) acc[c] += w * (uint32_t)__ldg(p + c);
 }
 
-// Six consecutive bytes (two horizontally adjacent BGR taps) starting at p, fetched as two aligned 64-bit words and
-// funnel-shifted: 2 load instructions instead of 6.  Requires p + 16 <= end of the allocation (checked by the caller).
-__device__ __forceinline__ uint64_t load6(const uint8_t* __restrict__ p) {
-  const uintptr_t a = (uintptr_t)p;
-  const uint64_t* w = (const uint64_t*)(a & ~(uintptr_t)7);
-  const uint64_t w0 = __ldg(w), w1 = __ldg(w + 1);
-  const uint32_t sh = (uint32_t)(a & 7) * 8u;
-  return (w0 >> sh) | ((w1 << 1) << (63u - sh));  // (w1 << (64 - sh)) without the undefined shift by 64
-}
-
-// Fast path for 3-channel pixels whose four taps are inside the image and unmasked.  Horizontal then vertical
-// interpolation with the 6-bit weights: sum_i w_i p_i = 32 * V, so (sum + 16384) >> 15 == (V + 512) >> 10 exactly.
-__device__ __forceinline__ void remap_pixel3_fast(const uint8_t* __restrict__ p, size_t row_bytes, uint32_t ax, uint32_t ay,
-                                                  uint32_t* out) {
-  const uint64_t r0 = load6(p), r1 = load6(p + row_bytes);
-  const uint32_t wl = 32u - ax, wt = 32u - ay;
-#pragma unroll
-  for (int c = 0; c < 3; ++c) {
-    const uint32_t h0 = wl * (uint32_t)((r0 >> (8 * c)) & 0xFF) + ax * (uint32_t)((r0 >> (8 * c + 24)) & 0xFF);
-    const uint32_t h1 = wl * (uint32_t)((r1 >> (8 * c)) & 0xFF) + ax * (uint32_t)((r1 >> (8 * c + 24)) & 0xFF);
-    out[c] = (wt * h0 + ay * h1 + 512u) >> 10;
-  }
-}
-
 // One output pixel: returns CH bytes in out[].
 template <int CH>
-__device__ __forceinline__ void remap_pixel(const uint8_t* __restrict__ src, const uint8_t* __restrict__ wide_end, int src_w,
-                                            uint64_t e, const uint32_t* border, const uint32_t* bg, uint32_t* out) {
+__device__ __forceinline__ void remap_pixel(const uint8_t* __restrict__ src, int src_w, uint64_t e, const uint32_t* border,
+                                            const uint32_t* bg, uint32_t* out) {
   const int x0 = (int)(int16_t)(e & 0xFFFF);
   const int y0 = (int)(int16_t)((e >> 16) & 0xFFFF);
   const uint32_t hi = (uint32_t)(e >> 32);
@@ -114,10 +85,6 @@ __device__ __forceinline__ void remap_pixel(const uint8_t* __restrict__ src, con
 #pragma unroll
   for (int c = 0; c < CH; ++c) acc[c] = 16384u;
   const uint8_t* p = src + ((size_t)y0 * src_w + x0) * CH;
-  if (CH == 3 && live == 15u && p + (size_t)src_w * 3 + 16 <= wide_end) {
-    remap_pixel3_fast(p, (size_t)src_w * 3, ax, ay, out);
-    return;
-  }
   if (live == 15u) {
     load_tap<CH>(p, w[0], acc);
     load_tap<CH>(p + CH, w[1], acc);
@@ -147,8 +114,8 @@ struct RemapConst {
 
 template <int CH>
 __global__ void __launch_bounds__(256)
-remap_kernel(const uint8_t* __restrict__ src, const uint8_t* __restrict__ wide_end, int src_h, int src_w,
-             const uint64_t* __restrict__ lut, int views, int rows, int cols, RemapConst k, uint8_t* __restrict__ dst) {
+remap_kernel(const uint8_t* __restrict__ src, int src_h, int src_w, const uint64_t* __restrict__ lut, int views, int rows,
+             int cols, RemapConst k, uint8_t* __restrict__ dst) {
   const int lane_col = blockIdx.x * RM_TILE_COLS + (threadIdx.x & 31) * RM_PX;
   const int row = blockIdx.y * RM_TILE_ROWS + (threadIdx.x >> 5);
   if (row >= rows || lane_col >= cols) return;
@@ -171,7 +138,7 @@ remap_kernel(const uint8_t* __restrict__ src, const uint8_t* __restrict__ wide_e
   uint32_t o[RM_PX][CH];
 #pragma unroll
   for (int i = 0; i < RM_PX; ++i) {
-    if (i < n) remap_pixel<CH>(s, wide_end, src_w, e[i], k.border, k.bg, o[i]);
+    if (i < n) remap_pixel<CH>(s, src_w, e[i], k.border, k.bg, o[i]);
   }
   if (n == RM_PX && (((uintptr_t)d) & 3) == 0) {
     // RM_PX * CH bytes = CH 32-bit words
@@ -200,107 +167,24 @@ remap_kernel(const uint8_t* __restrict__ src, const uint8_t* __restrict__ wide_e
 }
 
 
-// ---------------------------------------------------------------------------------------------------------------------
-// 3-channel kernel (the hot case).  A warp produces 128 consecutive pixels of one panorama row in 4 passes; in a pass
-// LANE l owns pixel 32*pass + l, so the 32 source positions of one load instruction are neighbours on the mirror
-// circle and share a handful of 32-byte sectors (the 4-pixels-per-thread layout touched ~28 sectors per request and
-// saturated L1).  Per pixel: 4 aligned LDG.64 + 32-bit funnel shifts give the two 6-byte tap pairs; horizontal
-// interpolation is one PRMT + DP4A per row and channel, the vertical one a DP2A:  V + 512 = wt*h0 + ay*h1 + 512,
-// dst = (V + 512) >> 10  ==  (sum_i w_i p_i + 16384) >> 15 of cv::remap because sum_i w_i p_i = 32 V exactly.
-// Results go through shared memory so that the row segment leaves as 16-byte stores.
-// ---------------------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void load6_32(const uint8_t* __restrict__ p, uint32_t& lo, uint32_t& hi) {
-  const uintptr_t a = (uintptr_t)p;
-  const uint2* w = (const uint2*)(a & ~(uintptr_t)7);
-  const uint2 w0 = __ldg(w), w1 = __ldg(w + 1);
-  const uint32_t o = (uint32_t)a & 7u, sh = (o & 3u) * 8u;
-  const bool k = o >= 4u;
-  const uint32_t A = k ? w0.y : w0.x, B = k ? w1.x : w0.y, C = k ? w1.y : w1.x;
-  lo = __funnelshift_r(A, B, sh);
-  hi = __funnelshift_r(B, C, sh);
-}
-
-// ---- patch-mapped variant -------------------------------------------------------------------------------------------
+// ---- lane mapping of the 3-channel kernel -----------------------------------------------------------------------------
 // A warp-wide gather costs one L1 wavefront per distinct 128-byte line it touches.  32 consecutive pixels of ONE panorama
 // row follow an arc in the omni image that crosses ~14 source rows (top mirror at C2) -> ~14 wavefronts per tap load; a
 // lane-per-pixel-along-the-row kernel is bound by exactly that (l1tex data-pipe 87 % busy, DRAM 11 %).  Mapping the 32 lanes onto a compact
 // 4-row x 8-column panorama patch halves the distinct lines (measured on the C2 LUT: 13.7 -> 6.1 top, 4.5 -> 1.9 bottom).
-// Warp tile = 4 rows x 32 columns in 4 passes; the 4 x 96 output bytes are staged in shared memory and written as
-// 16-byte vectors.  Same arithmetic for every lane mapping (bit-exact).
+// Warp tile = 4 rows x 32 columns in 4 passes (lane l: row l / 8, column 8 * pass + l % 8); the 4 x 96 output bytes are
+// staged in shared memory and written as 16-byte vectors.
 constexpr int RP_ROWS = 4;                 // rows per warp tile
 constexpr int RP_COLS = 32;                // columns per warp tile
 constexpr int RP_WARPS_X = 4, RP_WARPS_Y = 2;
-
-__global__ void __launch_bounds__(RP_WARPS_X * RP_WARPS_Y * 32)
-remap3p_kernel(const uint8_t* __restrict__ src, int wide_ok, int src_h, int src_w, const uint64_t* __restrict__ lut, int views,
-               int rows, int cols, RemapConst k, uint8_t* __restrict__ dst) {
-  __shared__ __align__(16) uint8_t sout[RP_WARPS_X * RP_WARPS_Y][RP_ROWS][RP_COLS * 3];
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int col0 = (blockIdx.x * RP_WARPS_X + (warp % RP_WARPS_X)) * RP_COLS;
-  const int row0 = (blockIdx.y * RP_WARPS_Y + (warp / RP_WARPS_X)) * RP_ROWS;
-  if (row0 >= rows || col0 >= cols) return;  // whole warps leave together; only __syncwarp below
-  const int img = blockIdx.z;
-  const int view = img % views, b = img / views;
-  const uint8_t* s = src + (size_t)b * src_h * src_w * 3;
-  const int npx = min(RP_COLS, cols - col0);
-  const int nrows = min(RP_ROWS, rows - row0);
-  const size_t row_bytes = (size_t)src_w * 3;
-  const int r = lane >> 3, cc = lane & 7;
-  const uint64_t* l = lut + ((size_t)view * rows + row0 + r) * cols + col0;
-  uint8_t* so = sout[warp][r];
-  if (r < nrows) {
-#pragma unroll
-    for (int pass = 0; pass < RP_COLS / 8; ++pass) {
-      const int c = pass * 8 + cc;
-      if (c < npx) {
-        const uint64_t e = __ldg(l + c);
-        const uint32_t hi = (uint32_t)(e >> 32);
-        uint32_t o[3];
-        if (wide_ok && (hi & (1u << 24))) {
-          const int x0 = (int)(int16_t)(e & 0xFFFF), y0 = (int)(int16_t)((e >> 16) & 0xFFFF);
-          const uint32_t ax = hi & 31u, ay = (hi >> 5) & 31u;
-          const uint8_t* p = s + ((size_t)y0 * src_w + x0) * 3;
-          uint32_t r0l, r0h, r1l, r1h;
-          load6_32(p, r0l, r0h);
-          load6_32(p + row_bytes, r1l, r1h);
-          const uint32_t wx = (32u - ax) | (ax << 8), wy = (32u - ay) | (ay << 8);
-          const uint32_t h0 = __dp4a(__byte_perm(r0l, r0h, 0x0030), wx, __dp4a(__byte_perm(r1l, r1h, 0x0030), wx, 0u) << 16);
-          const uint32_t h1 = __dp4a(__byte_perm(r0l, r0h, 0x0041), wx, __dp4a(__byte_perm(r1l, r1h, 0x0041), wx, 0u) << 16);
-          const uint32_t h2 = __dp4a(__byte_perm(r0l, r0h, 0x0052), wx, __dp4a(__byte_perm(r1l, r1h, 0x0052), wx, 0u) << 16);
-          o[0] = __dp2a_lo(h0, wy, 512u) >> 10;
-          o[1] = __dp2a_lo(h1, wy, 512u) >> 10;
-          o[2] = __dp2a_lo(h2, wy, 512u) >> 10;
-        } else {
-          remap_pixel<3>(s, nullptr, src_w, e, k.border, k.bg, o);
-        }
-        so[c * 3 + 0] = (uint8_t)o[0];
-        so[c * 3 + 1] = (uint8_t)o[1];
-        so[c * 3 + 2] = (uint8_t)o[2];
-      }
-    }
-  }
-  __syncwarp();
-  // write-out: 6 lanes per row, 16 bytes each (row r2 = lane / 6 for lanes 0..23); ragged / unaligned rows byte-wise
-  const int nbytes = npx * 3;
-  uint8_t* d0 = dst + (((size_t)img * rows + row0) * cols + col0) * 3;
-  const size_t drow = (size_t)cols * 3;
-  if (nbytes == RP_COLS * 3 && ((((uintptr_t)d0) | drow) & 15) == 0) {
-    const int r2 = lane / 6, ch = lane - r2 * 6;
-    if (lane < 24 && r2 < nrows) ((uint4*)(d0 + r2 * drow))[ch] = ((const uint4*)sout[warp][r2])[ch];
-  } else {
-    for (int r2 = 0; r2 < nrows; ++r2)
-      for (int i = lane; i < nbytes; i += 32) d0[r2 * drow + i] = sout[warp][r2][i];
-  }
-}
-
 
 // ---- batch-looped kernel with TMA-staged LUT tiles (the default 3-channel path) --------------------------------------------
 // The LUT depends on (view, row, col) only, so a block that owns one 8 x 128 LUT tile serves that tile for EVERY frame of
 // its share of the batch: the tile is fetched once (8 KB, one cp.async.bulk row copy per panorama row, completion on an
 // mbarrier), each lane decodes its four entries ONCE into registers (32-bit source offset, alignment shift, weights), and
 // the per-frame loop is nothing but 16 tap loads, the alignment funnel, dp4a arithmetic and the staged store:
-//   * ~45 instructions per pixel and frame instead of ~100 (ncu, round 1: the per-frame patch kernel is issue bound and
-//     spends more than half of its instructions on LUT decode, 64-bit address arithmetic, per-warp prologue and branches);
+//   * ~45 instructions per pixel and frame instead of ~100 (ncu, round 1: a per-frame 4 x 8-patch kernel was issue bound
+//     and spent more than half of its instructions on LUT decode, 64-bit address arithmetic, per-warp prologue and branches);
 //   * all 16 loads of a lane are in flight before the first use: no LUT-load -> tap-load dependency in the loop;
 //   * rows outside the mirror's field of view (38 % of the C2 panorama: whole rows of the LUT are "dead") never touch the
 //     source image: the warp stages the border colour once and only stores;
@@ -310,7 +194,7 @@ remap3p_kernel(const uint8_t* __restrict__ src, int wide_ok, int src_h, int src_
 // weights (32 - ay, ay, 0, 0) / (0, 0, 32 - ay, ay) gives vL and vR, then (wl * vL + ax * vR + 512) >> 10 — the same integer
 // as cv::remap's (sum_i w_i p_i + 16384) >> 15 because the Q15 weights are 32 * (6-bit x 6-bit products).
 // Requires a 4-byte aligned source whose rows are a multiple of 4 bytes (src_w % 4 == 0), so that the alignment of a tap
-// address is the same for every frame and both rows; other shapes take remap3p_kernel.
+// address is the same for every frame and both rows; other shapes take remap_kernel<3>.
 constexpr int RB_TILE_ROWS = RP_ROWS * RP_WARPS_Y;   // 8
 constexpr int RB_TILE_COLS = RP_COLS * RP_WARPS_X;   // 128
 constexpr int RB_NP = RP_COLS / 8;                   // passes per lane
@@ -458,7 +342,7 @@ remap3b_kernel(const uint8_t* __restrict__ src, int batch, int frames_per_block,
         if ((slowm >> pass) & 1u) {
           const int c = pass * 8 + cc;
           uint32_t o[3];
-          remap_pixel<3>(s, nullptr, src_w, slut[wy * RP_ROWS + r][wx * RP_COLS + c], k.border, k.bg, o);
+          remap_pixel<3>(s, src_w, slut[wy * RP_ROWS + r][wx * RP_COLS + c], k.border, k.bg, o);
           so[c * 3 + 0] = (uint8_t)o[0];
           so[c * 3 + 1] = (uint8_t)o[1];
           so[c * 3 + 2] = (uint8_t)o[2];
@@ -518,39 +402,27 @@ extern "C" int sos_remap_u8(sos_ctx* ctx, const uint8_t* src, int batch, int src
     k.border[c] = (border && c < channels) ? border[c] : 0;
     k.bg[c] = (background && c < channels) ? background[c] : 0;
   }
-  dim3 grid(sos_div_up(cols, RM_TILE_COLS), sos_div_up(rows, RM_TILE_ROWS), batch * views);
-  // the wide (2 x 64-bit) tap loads may touch up to 15 bytes past the taps: allowed only inside [src, wide_end)
-  const bool aligned8 = ((uintptr_t)src & 7) == 0;
-  const uint8_t* wide_end = aligned8 ? src + (size_t)batch * src_h * src_w * channels : nullptr;
-  if (channels == 3) {
-    // Default: batch-looped blocks with TMA-staged LUT tiles (remap3b_kernel).  It needs tap addresses whose alignment is
-    // the same in every frame and row (4-byte aligned source, src_w % 4 == 0) and 32-bit offsets inside a frame; anything
-    // else, or SOS_REMAP_TMA=0, takes the per-frame patch kernel.  tests/test_gpu_remap.py runs every case on both.
-    const char* e = getenv("SOS_REMAP_TMA");
-    const bool want_tma = e == nullptr || e[0] != '0';
-    const bool tma_kernel = want_tma && ((uintptr_t)src & 3) == 0 && (src_w % 4) == 0 && (size_t)src_h * src_w * 3 < (1ull << 32);
-    if (tma_kernel) {
-      const int tiles = sos_div_up(cols, RB_TILE_COLS) * sos_div_up(rows, RB_TILE_ROWS) * views;
-      // enough blocks for ~5 waves of 3 blocks per SM; every block decodes its LUT tile once for its share of the batch
-      const int want_blocks = ctx->sm_count * 3 * 5;
-      int splits = (want_blocks + tiles - 1) / tiles;
-      splits = splits < 1 ? 1 : (splits > batch ? batch : splits);
-      const int fpb = sos_div_up(batch, splits);
-      splits = sos_div_up(batch, fpb);
-      SOS_CHECK_ARG((long long)views * splits <= 65535, "views * batch splits exceeds 65535");
-      dim3 gb(sos_div_up(cols, RB_TILE_COLS), sos_div_up(rows, RB_TILE_ROWS), views * splits);
-      remap3b_kernel<<<gb, RP_WARPS_X * RP_WARPS_Y * 32, 0, ctx->stream>>>(src, batch, fpb, src_h, src_w, lut, views, rows, cols, k, dst);
-      SOS_LAUNCHED_AS(ctx, "remap3b_kernel");
-    } else {
-      dim3 gp(sos_div_up(cols, RP_COLS * RP_WARPS_X), sos_div_up(rows, RP_ROWS * RP_WARPS_Y), batch * views);
-      remap3p_kernel<<<gp, RP_WARPS_X * RP_WARPS_Y * 32, 0, ctx->stream>>>(src, aligned8 ? 1 : 0, src_h, src_w, lut, views, rows,
-                                                                           cols, k, dst);
-      SOS_LAUNCHED_AS(ctx, "remap3p_kernel");
-    }
-  } else {
-    if (channels == 1) remap_kernel<1><<<grid, 256, 0, ctx->stream>>>(src, wide_end, src_h, src_w, lut, views, rows, cols, k, dst);
-    else remap_kernel<4><<<grid, 256, 0, ctx->stream>>>(src, wide_end, src_h, src_w, lut, views, rows, cols, k, dst);
-    SOS_LAUNCHED_AS(ctx, "remap_kernel");
+  // Batch-looped blocks with TMA-staged LUT tiles (remap3b_kernel) need tap addresses whose alignment is the same in every
+  // frame and row (4-byte aligned source, src_w % 4 == 0) and 32-bit offsets inside a frame.  Every other 3-channel call,
+  // and every 1- or 4-channel call, takes the generic kernel.  tests/test_gpu_remap.py runs every case on both.
+  if (channels == 3 && ((uintptr_t)src & 3) == 0 && (src_w % 4) == 0 && (size_t)src_h * src_w * 3 < (1ull << 32)) {
+    const int tiles = sos_div_up(cols, RB_TILE_COLS) * sos_div_up(rows, RB_TILE_ROWS) * views;
+    // enough blocks for ~5 waves of 3 blocks per SM; every block decodes its LUT tile once for its share of the batch
+    const int want_blocks = ctx->sm_count * 3 * 5;
+    int splits = (want_blocks + tiles - 1) / tiles;
+    splits = splits < 1 ? 1 : (splits > batch ? batch : splits);
+    const int fpb = sos_div_up(batch, splits);
+    splits = sos_div_up(batch, fpb);
+    SOS_CHECK_ARG((long long)views * splits <= 65535, "views * batch splits exceeds 65535");
+    dim3 gb(sos_div_up(cols, RB_TILE_COLS), sos_div_up(rows, RB_TILE_ROWS), views * splits);
+    remap3b_kernel<<<gb, RP_WARPS_X * RP_WARPS_Y * 32, 0, ctx->stream>>>(src, batch, fpb, src_h, src_w, lut, views, rows, cols, k, dst);
+    SOS_LAUNCHED_AS(ctx, "remap3b_kernel");
+    return SOS_OK;
   }
+  dim3 grid(sos_div_up(cols, RM_TILE_COLS), sos_div_up(rows, RM_TILE_ROWS), batch * views);
+  if (channels == 1) remap_kernel<1><<<grid, 256, 0, ctx->stream>>>(src, src_h, src_w, lut, views, rows, cols, k, dst);
+  else if (channels == 3) remap_kernel<3><<<grid, 256, 0, ctx->stream>>>(src, src_h, src_w, lut, views, rows, cols, k, dst);
+  else remap_kernel<4><<<grid, 256, 0, ctx->stream>>>(src, src_h, src_w, lut, views, rows, cols, k, dst);
+  SOS_LAUNCHED_AS(ctx, "remap_kernel");
   return SOS_OK;
 }
