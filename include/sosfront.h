@@ -171,6 +171,26 @@ int sos_l2_top2(sos_ctx* ctx, const float* q, const float* t, int dim, const int
                 const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int32_t* idx0,
                 float* d0, int32_t* idx1, float* d1, int32_t* not_integer_flag);
 
+/* replaces: cv2.BFMatcher() (NORM_L2) .match / .knnMatch(k = 2) on ANY finite float descriptors (SURF, KAZE, RootSIFT, ...) —
+ * the SIFT / SURF branch of FeatureMatcher (camera_models.py:397-399, 417-442) when the values are not integers in [0, 255].
+ * Results are those of a float64 reference with a fixed evaluation order, bit for bit:
+ *   d^2(q, t) = sum_k (double(q_k) - double(t_k))^2, summed for k = 0 .. dim-1 in order, without fused multiply-add;
+ *   the two smallest d^2 per query, ties to the lowest train row; distance = float32(sqrt(d^2)) rounded from double.
+ * On integer-valued inputs this equals cv2 (and sos_l2_top2).  On other inputs cv2's float32 SIMD sum is build-dependent;
+ * its distances may differ from these by an ulp.
+ * The tensor cores rank the candidates (each value split into two bfloat16 pieces, float32 accumulators); a query whose
+ * nearest rows are closer together than a derived error band, or whose magnitudes could leave the float32 range, is
+ * re-decided by a float64 brute force over its segment, so the result never depends on the band.
+ *   q, t [*, dim] float32 rows, 1 <= dim <= 128; segments, idx0 / idx1 / d0 / d1 as in sos_l2_top2 (idx1 / d1 may be NULL)
+ *   nonfinite_flag: DEVICE int32 [1], set non-zero when a value is NaN or +-Inf (the outputs are then meaningless)
+ *   stats (may be NULL): DEVICE int32 [SOS_L2F_STATS], zeroed by the call, indices SOS_L2F_STAT_*. */
+#define SOS_L2F_STATS 2
+#define SOS_L2F_STAT_REDECIDED 0   /* queries re-decided by the float64 brute force */
+#define SOS_L2F_STAT_BAND_PPM 1    /* largest |approximate - float64 d^2| / band over the winners decided from the GEMM, ppm */
+int sos_l2f_top2(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start, const int32_t* q_len,
+                 const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int32_t* idx0,
+                 float* d0, int32_t* idx1, float* d1, int32_t* nonfinite_flag, int32_t* stats);
+
 #define SOS_MATCH_NN 0    /* 1-NN, the reference default (k_best = 1, pose_est_tools.py:686) */
 #define SOS_MATCH_RATIO 1 /* keep m0 iff d0 < ratio * d1 (camera_models.py:421-436) */
 #define SOS_MATCH_CROSS 2 /* mutual nearest neighbours (BFMatcher crossCheck, camera_models.py:401) */

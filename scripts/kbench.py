@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Kernel micro-benchmarks at C2 sizes (CUDA events, warm-up, inputs rotated): python scripts/kbench.py [hamming|ransac|remap|dense|rgbd|all]
+"""Kernel micro-benchmarks at C2 sizes (CUDA events, warm-up, inputs rotated): python scripts/kbench.py [hamming|ransac|remap|dense|rgbd|l2|all]
 
 Prints one JSON line per kernel and input variant.
 """
@@ -149,6 +149,73 @@ def bench_rgbd(ctx, hbm_peak, B=256, h=480, w=640, n=1000):
                 ms_backproject=ms_bp, keypoints_per_s=B * n / (ms_bp * 1e-3), frames_per_s_both=B / ((ms_z + ms_bp) * 1e-3))
 
 
+def card():
+    """The card's name and power limit, read in the same run as the numbers they qualify."""
+    import subprocess
+    try:
+        pl = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", "0"],
+                            capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError):
+        pl = "unknown"
+    return dict(gpu=torch.cuda.get_device_name(0), power_limit=pl)
+
+
+def bench_l2(ctx, dim, sizes, engine):
+    """Both float-descriptor L2 engines on the same segment shapes: "int" = sos_l2_top2 on integer-valued SIFT-like rows,
+    "float" = sos_l2f_top2 on RootSIFT-like rows (non-integer).  Executed bf16 FLOP/s counts the padded tiles and the MMA
+    instructions each engine issues (9 x K16 per tile pair, resp. 3 ceil(dim / 16) + 1)."""
+    rng = np.random.default_rng(dim)
+    nq = np.array([a for a, _ in sizes], np.int32)
+    nt = np.array([b for _, b in sizes], np.int32)
+    h = rng.gamma(0.7, 28.0, (int(nq.sum() + nt.sum()), dim))
+    if engine == "int":
+        x = np.clip(h, 0, 255).round().astype(np.float32)
+    else:
+        x = np.sqrt(h / h.sum(1, keepdims=True)).astype(np.float32)
+    tq, tt = x[:nq.sum()], x[nq.sum():]
+    q_start = np.concatenate([[0], np.cumsum(nq)[:-1]]).astype(np.int32)
+    t_start = np.concatenate([[0], np.cumsum(nt)[:-1]]).astype(np.int32)
+    d = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()
+    args = (d(tq), d(tt), d(q_start), d(nq), d(t_start), d(nt), int(nq.max()), int(nt.max()))
+    stats = torch.zeros(ops.L2F_STATS, dtype=torch.int32, device="cuda")
+    fn = (lambda: ctx.l2_top2(*args)) if engine == "int" else (lambda: ctx.l2f_top2(*args, stats=stats))
+    ms = timeit(fn, iters=20)
+    n_mma = 9 if engine == "int" else 3 * -(-dim // 16) + 1
+    flops = sum(2.0 * (-(-a // 256) * 256) * (-(-b // 128) * 128) * 16 * n_mma for a, b in sizes)
+    r = dict(kernel="l2_top2" if engine == "int" else "l2f_top2", dim=dim, segments=len(sizes),
+             shape=f"{sizes[0][0]}x{sizes[0][1]}" if len(set(sizes)) == 1 else "mixed", ms=ms,
+             bf16_tflops_executed=flops / (ms * 1e-3) / 1e12)
+    if engine == "float":
+        r["redecided_share"] = int(stats[ops.L2F_STAT_REDECIDED]) / int(nq.sum())
+        r["band_ratio_max"] = int(stats[ops.L2F_STAT_BAND_PPM]) * 1e-6
+    return r
+
+
+def bench_l2_real(ctx):
+    """Re-decided share of sos_l2f_top2 on live cv2 KAZE and RootSIFT descriptors of a seeded synthetic frame pair."""
+    import cv2
+    rng = np.random.default_rng(21)
+    img = cv2.GaussianBlur((rng.random((960, 1280)) * 255).astype(np.uint8), (0, 0), 2.0)
+    for _ in range(200):
+        c = tuple(int(v) for v in rng.integers(0, [1280, 960]))
+        cv2.circle(img, c, int(rng.integers(4, 40)), int(rng.integers(0, 255)), -1)
+    rot = cv2.warpAffine(img, cv2.getRotationMatrix2D((640, 480), 12.0, 1.05), (1280, 960))
+    sift = cv2.SIFT_create(nfeatures=8000)
+    root = lambda v: np.sqrt(v / np.maximum(v.sum(1, keepdims=True), 1e-12)).astype(np.float32)
+    out = []
+    for name, det, post in (("KAZE", cv2.KAZE_create(), lambda v: v), ("RootSIFT", sift, root)):
+        q, t = post(det.detectAndCompute(img, None)[1]), post(det.detectAndCompute(rot, None)[1])
+        d = lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda()
+        z = d(np.zeros(1, np.int32))
+        stats = torch.zeros(ops.L2F_STATS, dtype=torch.int32, device="cuda")
+        args = (d(q), d(t), z, d(np.array([len(q)], np.int32)), z, d(np.array([len(t)], np.int32)), len(q), len(t))
+        ms = timeit(lambda: ctx.l2f_top2(*args, stats=stats), iters=10)
+        out.append(dict(kernel="l2f_top2", descriptors=name, dim=q.shape[1], nq=len(q), nt=len(t), ms=ms,
+                        redecided_share=int(stats[ops.L2F_STAT_REDECIDED]) / len(q),
+                        band_ratio_max=int(stats[ops.L2F_STAT_BAND_PPM]) * 1e-6))
+    return out
+
+
 def main():
     what = sys.argv[1] if len(sys.argv) > 1 else "all"
     ctx = ops.Context(0)
@@ -170,6 +237,14 @@ def main():
         res.append(bench_dense(ctx, 6451.2))
     if what in ("rgbd", "all"):
         res.append(bench_rgbd(ctx, 6451.2))
+    if what == "l2":
+        res.append(card())
+        stereo = [(700 - 5 * s, 700 + 5 * s) for s in range(12)]
+        for dim in (64, 128):
+            for sizes in (stereo, [(8000, 8000)]):
+                res.append(bench_l2(ctx, dim, sizes, "int"))
+                res.append(bench_l2(ctx, dim, sizes, "float"))
+        res.extend(bench_l2_real(ctx))
     for r in res:
         print(json.dumps(r))
 

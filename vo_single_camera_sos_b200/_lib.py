@@ -40,6 +40,7 @@ PROTOTYPES = {
     "sos_lut_build": (I, [c_ctx, P, I, I, D, D, D, D, P, P]),
     "sos_hamming_top2": (I, [c_ctx, P, P, P, P, P, P, I, I, I, P, P, P, P]),
     "sos_l2_top2": (I, [c_ctx, P, P, I, P, P, P, P, I, I, I, P, P, P, P, P]),
+    "sos_l2f_top2": (I, [c_ctx, P, P, I, P, P, P, P, I, I, I, P, P, P, P, P, P]),
     "sos_hamming_radius": (I, [c_ctx, P, I, P, I, I, P, P, P, P]),
     "sos_match_select": (I, [c_ctx, I, D, P, P, P, P, P, P, P, I, P, P, D, D, P, P, P, P]),
     "sos_lift_pano": (I, [c_ctx, P, P, I, P, P, P]),

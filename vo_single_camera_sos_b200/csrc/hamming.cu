@@ -29,6 +29,12 @@ int sos_l2_mma_launch(sos_ctx* ctx, const float* q, const float* t, int dim, con
                       const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* exp,
                       ulonglong2* partial, int32_t* flag);
 
+size_t sos_l2f_scratch_bytes(int n_seg, int max_nq, int max_nt, int dim, int splits);
+int sos_l2f_launch(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start, const int32_t* q_len,
+                   const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int splits,
+                   const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* scratch,
+                   int32_t* idx0, float* d0, int32_t* idx1, float* d1, int32_t* flag, int32_t* stats);
+
 namespace {
 
 constexpr int HB_THREADS = 128;  // threads per block
@@ -511,6 +517,42 @@ extern "C" int sos_l2_top2(sos_ctx* ctx, const float* q, const float* t, int dim
   l2_merge_kernel<<<mgrid, 256, 0, ctx->stream>>>((const ulonglong2*)ws, q_start, q_len, max_nq, splits, idx0, d0, idx1, d1);
   SOS_LAUNCHED_AS(ctx, "l2_merge_kernel");
   return SOS_OK;
+}
+
+// Any finite float descriptors: the split-bfloat16 GEMM ranks, float64 decides (hamming_mma.cu: band, kernels).
+extern "C" int sos_l2f_top2(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start,
+                            const int32_t* q_len, const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq,
+                            int max_nt, int32_t* idx0, float* d0, int32_t* idx1, float* d1, int32_t* nonfinite_flag,
+                            int32_t* stats) {
+  SOS_CHECK_ARG(ctx, "ctx is NULL");
+  SOS_CHECK_ARG(n_seg >= 0 && max_nq >= 0 && max_nt >= 0, "negative size");
+  SOS_CHECK_ARG(dim >= 1 && dim <= 128, "descriptor length must be 1..128");
+  SOS_CHECK_ARG(n_seg <= 65535, "at most 65535 segments per call");
+  SOS_CHECK_ARG(max_nt < (1 << 30), "segment has too many train rows");
+  if (n_seg == 0 || max_nq == 0) return SOS_OK;
+  SOS_CHECK_ARG(q && t && q_start && q_len && t_start && t_len && idx0 && d0 && nonfinite_flag, "NULL array");
+  SOS_CUDA(cudaSetDevice(ctx->device));
+  const int q_tiles = sos_div_up(max_nq, HB_TILE_Q);
+  SOS_CHECK_ARG(q_tiles <= (1 << ITEM_TILE_BITS), "segment has too many query rows (limit 262144)");
+  const bool top2 = idx1 != nullptr || d1 != nullptr;
+  const int t_tiles = sos_div_up(max_nt > 0 ? max_nt : 1, 128);
+  int splits = sos_div_up(2 * ctx->sm_count, q_tiles * n_seg);
+  if (splits > t_tiles / 4) splits = t_tiles / 4;
+  if (splits > (1 << ITEM_SPLIT_BITS)) splits = 1 << ITEM_SPLIT_BITS;
+  if (splits < 1) splits = 1;
+  void* ws = nullptr;
+  const size_t max_items = (size_t)q_tiles * splits * n_seg;
+  SOS_CHECK_ARG(max_items < ((size_t)1 << 31), "too many work items");
+  const size_t items_bytes = sos_align_up(max_items * sizeof(uint32_t), 256);
+  int rc = sos_arena_get(ctx, items_bytes + 256 + sos_l2f_scratch_bytes(n_seg, max_nq, max_nt, dim, splits), &ws);
+  if (rc != SOS_OK) return rc;
+  uint32_t* items = (uint32_t*)ws;
+  int32_t* n_items = (int32_t*)((char*)ws + items_bytes);
+  SOS_CUDA(cudaMemsetAsync(nonfinite_flag, 0, sizeof(int32_t), ctx->stream));
+  hamming_plan_kernel<<<1, 256, 0, ctx->stream>>>(q_len, n_seg, max_nq, splits, items, n_items);
+  SOS_LAUNCHED_AS(ctx, "hamming_plan_kernel");
+  return sos_l2f_launch(ctx, q, t, dim, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, splits, items, n_items,
+                        (unsigned)max_items, top2, (char*)ws + items_bytes + 256, idx0, d0, idx1, d1, nonfinite_flag, stats);
 }
 
 extern "C" int sos_match_select(sos_ctx* ctx, int mode, double ratio, const int32_t* idx0, const int32_t* d0,

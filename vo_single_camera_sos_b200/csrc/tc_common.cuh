@@ -46,8 +46,8 @@ __device__ __forceinline__ void tc_commit(uint32_t bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 // D[tmem] (+)= A[smem] * B[smem], M128 N128, 32 bytes of K per instruction:
-//   KIND_HAMMING: int8 x int8 -> int32 (K32);   KIND_L2: bf16 x bf16 -> float32 (K16)
-constexpr int KIND_HAMMING = 0, KIND_L2 = 1;
+//   KIND_HAMMING: int8 x int8 -> int32 (K32);   KIND_L2, KIND_L2F: bf16 x bf16 -> float32 (K16)
+constexpr int KIND_HAMMING = 0, KIND_L2 = 1, KIND_L2F = 2;
 template <int KIND>
 __device__ __forceinline__ void tc_mma(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
   if (KIND == KIND_HAMMING)

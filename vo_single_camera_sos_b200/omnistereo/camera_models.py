@@ -21,7 +21,8 @@ class FeatureMatcher(object):
     are Hamming distances computed by sos_hamming_top2; results are ordered like sorted(matches, key=distance), i.e.
     stably by (distance, queryIdx), with ties between train rows going to the lowest trainIdx (cv2.BFMatcher).
     method "SIFT" / "SURF" selects the L2 norm on float descriptors like the reference (camera_models.py:397-399): the
-    tensor-core matcher sos_l2_top2, exact for integer-valued descriptors (cv2's SIFT output)."""
+    tensor-core matcher sos_l2_top2 for integer-valued descriptors in [0, 255] (cv2's SIFT output, exact), sos_l2f_top2 for
+    any other finite values (SURF, KAZE, RootSIFT: bit-equal to a float64 reference)."""
 
     def __init__(self, method, matcher_type, k_best, *args, **kwargs):
         self.feature_detection_method = method
@@ -114,7 +115,8 @@ class FeatureMatcher(object):
         """The SIFT / SURF branch (camera_models.py:397-399, 417-442): cv2.BFMatcher() = NORM_L2.  k_best = 1: the nearest
         train row per query; k_best = 2: knnMatch(k = 2), for "SIFT" filtered by Lowe's ratio test m0.distance <
         0.75 * m1.distance (len(m) == 2 required, :423), otherwise both neighbours flattened; then sorted(key=distance).
-        Distances are float32 like cv2's."""
+        Distances are float32 like cv2's.  The engine follows the values: integers in [0, 255] go to l2_top2 (9 MMAs per
+        tile pair, no re-decision), everything else to l2f_top2 (13 to 25 MMAs and a float64 decision)."""
         q = np.ascontiguousarray(query_descriptors, np.float32)
         t = np.ascontiguousarray(train_descriptors, np.float32)
         if q.ndim != 2 or t.ndim != 2 or q.shape[1] != t.shape[1] or q.shape[1] > 128:
@@ -125,7 +127,9 @@ class FeatureMatcher(object):
         ctx = device_context()
         i32 = lambda v: torch.tensor([v], dtype=torch.int32, device=ctx.device)
         zero = i32(0)
-        i0, d0, i1, d1 = (x.cpu().numpy() for x in ctx.l2_top2(to_device(q), to_device(t), zero, i32(nq), zero, i32(nt), nq, nt))
+        integer = all(np.array_equal(x, np.floor(x)) and x.min() >= 0 and x.max() <= 255 for x in (q, t))
+        top2 = ctx.l2_top2 if integer else ctx.l2f_top2
+        i0, d0, i1, d1 = (x.cpu().numpy() for x in top2(to_device(q), to_device(t), zero, i32(nq), zero, i32(nt), nq, nt))
         qi = np.arange(nq, dtype=np.int32)
         if self.k_best == 2 and str(self.feature_detection_method).upper() == "SIFT":
             keep = (i1 >= 0) & (d0.astype(np.float64) < d1.astype(np.float64) * 0.75)      # Python floats in the reference

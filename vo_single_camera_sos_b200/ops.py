@@ -19,6 +19,7 @@ from ._lib import SosError, check  # noqa: F401  (re-exported)
 MATCH_NN, MATCH_RATIO, MATCH_CROSS = 0, 1, 2
 SCORE_EUCLID, SCORE_BEARING = 0, 1
 SOLVER_ARUN, SOLVER_P3P = 0, 1
+L2F_STATS, L2F_STAT_REDECIDED, L2F_STAT_BAND_PPM = 2, 0, 1   # sosfront.h SOS_L2F_*
 REFINE_NONE, REFINE_ARUN, REFINE_LM = 0, 1, 2
 
 GUM_FIELDS = ("xi1", "xi2", "xi3", "k1", "k2", "k3", "gamma1", "gamma2", "alpha_c", "u_center", "v_center",
@@ -203,6 +204,34 @@ class Context:
         if int(flag.item()):
             raise ValueError("float descriptors must hold integers in [0, 255] (cv2 SIFT); other values are not supported "
                              "by the exact tensor-core L2 matcher")
+        return idx0, d0, idx1, d1
+
+    def l2f_top2(self, q: torch.Tensor, t: torch.Tensor, q_start, q_len, t_start, t_len, max_nq: int, max_nt: int,
+                 want_second: bool = True, stats: Optional[torch.Tensor] = None):
+        """Any finite float descriptors (SURF, KAZE, RootSIFT, ...): q [Nq, dim], t [Nt, dim] float32, 1 <= dim <= 128.
+        -> (idx0 int32, d0 float32, idx1, d1) like l2_top2, equal bit for bit to a float64 reference: d^2 summed over k in
+        order without FMA, ties to the lowest train row, distance = float32(sqrt(d^2)).  Raises ValueError on NaN / Inf.
+        stats: optional DEVICE int32 [L2F_STATS] -> queries re-decided in float64, largest error / band in ppm."""
+        self._sync_stream()
+        nq, dim = q.shape
+        if t.dim() != 2 or t.shape[1] != dim or not 1 <= dim <= 128:
+            raise ValueError("q / t must be [N, dim] with the same 1 <= dim <= 128")
+        if stats is not None and stats.numel() < L2F_STATS:
+            raise ValueError(f"stats needs {L2F_STATS} int32 entries")
+        n_seg = q_start.numel()
+        idx0 = torch.full((nq,), -1, dtype=torch.int32, device=self.device)
+        d0 = torch.full((nq,), -1.0, dtype=torch.float32, device=self.device)
+        idx1 = torch.full((nq,), -1, dtype=torch.int32, device=self.device) if want_second else None
+        d1 = torch.full((nq,), -1.0, dtype=torch.float32, device=self.device) if want_second else None
+        flag = torch.zeros((1,), dtype=torch.int32, device=self.device)
+        check(self.lib.sos_l2f_top2(self._h, self._t(q, torch.float32, "q"), self._t(t, torch.float32, "t"), int(dim),
+                                    self._t(q_start, torch.int32, "q_start"), self._t(q_len, torch.int32, "q_len"),
+                                    self._t(t_start, torch.int32, "t_start"), self._t(t_len, torch.int32, "t_len"), n_seg,
+                                    int(max_nq), int(max_nt), idx0.data_ptr(), d0.data_ptr(),
+                                    idx1.data_ptr() if idx1 is not None else None, d1.data_ptr() if d1 is not None else None,
+                                    flag.data_ptr(), self._t(stats, torch.int32, "stats", optional=True)))
+        if int(flag.item()):
+            raise ValueError("float descriptors must be finite (a value is NaN or Inf)")
         return idx0, d0, idx1, d1
 
     def hamming_radius(self, q: torch.Tensor, t: torch.Tensor, max_distance: int):
