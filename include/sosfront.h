@@ -419,7 +419,9 @@ int sos_orb_describe(sos_ctx* ctx, const uint8_t* gray, int n_images, int height
 
 /* replaces: cv2.cornerMinEigenVal(gray, blockSize = 3, ksize = 3) — the corner measure inside goodFeaturesToTrack.
  * gray uint8 [n_images, height, width] -> eig float32 [n_images, height, width].  Same float32 arithmetic as OpenCV 4.13
- * (bit-equal except at cv2's own SIMD tail columns, where its last bit depends on the image width). */
+ * (written out at the top of csrc/gft.cu; the Sobel rows are smoothed in cv2's tap order).  Bit-equal to cv2 except in
+ * its SIMD tail columns (the last <= 16 of a row) and, on sharp images, at a few pixels where cv2's sliding-window box
+ * sums round differently (at most half a unit in the last place of the image's largest measure). */
 int sos_corner_min_eigenval(sos_ctx* ctx, const uint8_t* gray, int n_images, int height, int width, float* eig);
 
 /* replaces: cv2.goodFeaturesToTrack(image = gray, maxCorners, qualityLevel, minDistance, mask = masks[m],
@@ -428,8 +430,10 @@ int sos_corner_min_eigenval(sos_ctx* ctx, const uint8_t* gray, int n_images, int
  *   out_xy    float32 [n_images, n_masks, max_corners, 2] corner (x, y), strongest first
  *   out_count int32 [n_images, n_masks]
  *   eig_out   float32 [n_images, height, width] (nullable) receives the corner measure
- * More than 16384 local maxima above the quality threshold in one (image, mask) cannot be ranked reproducibly: with
- * several masks the call fails with SOS_ERR_INVALID, with one mask out_count of that list is set to -(candidates). */
+ * max_corners must be >= 1 (cv2's maxCorners <= 0, "no limit", has no fixed output size).  More than 16384 local maxima
+ * above the quality threshold in one (image, mask) cannot be ranked reproducibly: the call then fails with
+ * SOS_ERR_INVALID, whatever the number of masks.  The call reads the candidate counts back, so it returns only after the
+ * candidate stage has run on ctx's stream. */
 int sos_gft_detect(sos_ctx* ctx, const uint8_t* gray, const uint8_t* masks, int n_images, int height, int width,
                    int n_masks, int max_corners, double quality_level, double min_distance, float* out_xy,
                    int32_t* out_count, float* eig_out);

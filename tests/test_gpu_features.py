@@ -1,10 +1,13 @@
 """GPU: the image-in front-end (SURVEY §8f N3 chained in front of the hot path): feature arrays produced on the device
-from rendered omni images equal what the reference's OpenCV calls give on the same panoramas, and the poses that come out
+from rendered omni images equal what the reference's OpenCV calls give on the same panoramas (the corner lists exactly
+those of oracle/gft.py on cv2's median and gray), and the poses that come out
 of Frontend.step on them follow the ground-truth motion."""
 import cv2
 import numpy as np
 import pytest
 import torch
+
+from oracle import gft as ogft
 
 pytestmark = pytest.mark.gpu
 
@@ -40,8 +43,16 @@ def test_image_in_front_end(ctx):
                 px, ds, boff = px.cpu().numpy(), ds.cpu().numpy(), boff.cpu().numpy()
                 gray = cv2.cvtColor(cv2.medianBlur(pano[0, view], 11), cv2.COLOR_BGR2GRAY)
                 orb = cv2.ORB_create(nfeatures=N)
+                eig = ogft.corner_min_eigenval(gray)
                 total = same = 0
                 for k in range(12):
+                    # exactly: cv2 median and gray, then the oracle's Shi-Tomasi, then ORB.compute
+                    want, _ = ogft.good_features(eig, masks[view][k], N, 0.01, 5.0)
+                    got_px, got_ds = px[0, boff[0, k]:boff[0, k + 1]], ds[0, boff[0, k]:boff[0, k + 1]]
+                    ko, do = orb.compute(gray, list(cv2.KeyPoint_convert(want))) if len(want) else ([], np.zeros((0, 32), np.uint8))
+                    assert np.array_equal(got_px, np.array([kp.pt for kp in ko], np.float32).reshape(-1, 2)), (view, k)
+                    assert np.array_equal(got_ds, do), (view, k)
+                    # against cv2's own corner lists (its SIMD tail columns may decide a near-tie differently)
                     pts = cv2.goodFeaturesToTrack(image=gray, maxCorners=N, qualityLevel=0.01, minDistance=5, mask=masks[view][k],
                                                   useHarrisDetector=False)
                     if pts is None:

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from conftest import load_golden, sub
+from oracle import gft as ogft
 
 pytestmark = pytest.mark.gpu
 
@@ -286,8 +287,14 @@ def test_detect_sparse_features_gft_on_device(gums):
             pano_obj.panoramic_img, pano_obj.azimuthal_masks = saved
         blurred = cv2.cvtColor(cv2.medianBlur(pano, 11), cv2.COLOR_BGR2GRAY)
         orb = cv2.ORB_create(nfeatures=60)
+        eig = ogft.corner_min_eigenval(blurred)
         total = same = 0
         for m, k_got, d_got in zip(masks, kl, dl):
+            # exactly: cv2 median and gray, then the oracle's Shi-Tomasi, then ORB.compute
+            want, _ = ogft.good_features(eig, m, 60, 0.01, 5.0)
+            k_or, d_or = orb.compute(blurred, list(cv2.KeyPoint_convert(want)))
+            assert [k.pt for k in k_got] == [k.pt for k in k_or] and np.array_equal(d_got, d_or)
+            # against cv2's own corner lists (its SIMD tail columns may decide a near-tie differently)
             pts = cv2.goodFeaturesToTrack(image=blurred, maxCorners=60, qualityLevel=0.01, minDistance=5, mask=m,
                                           useHarrisDetector=False)
             k_ref, d_ref = orb.compute(blurred, list(cv2.KeyPoint_convert(pts.reshape(-1, 2))))
@@ -299,3 +306,22 @@ def test_detect_sparse_features_gft_on_device(gums):
                     same += 1
                     assert np.array_equal(da, db) and a.angle == b.angle == -1 and a.octave == b.octave == 0
         assert total > 60 and same >= 0.98 * total, (same, total)
+
+
+def test_detect_sparse_features_gft_refuses_overflow(gums):
+    """Without azimuthal masks the whole panorama is one list; a textured 849 x 2400 panorama has far more than the 16 384
+    candidates the selection can rank, and the call raises instead of returning fewer keypoints."""
+    from vo_single_camera_sos_b200._lib import SosError
+    gs, _ = gums
+    pano = cv2.GaussianBlur(np.random.default_rng(12).integers(0, 256, (849, 2400, 3), dtype=np.uint8), (0, 0), 1.0)
+    gray = cv2.cvtColor(cv2.medianBlur(pano, 11), cv2.COLOR_BGR2GRAY)
+    assert len(ogft.candidates(ogft.corner_min_eigenval(gray), None, 0.01)) > 16384
+    pano_obj = gs.top_model.panorama
+    saved = pano_obj.panoramic_img, pano_obj.azimuthal_masks
+    pano_obj.panoramic_img, pano_obj.azimuthal_masks = pano, []
+    try:
+        with pytest.raises(SosError):
+            gs.top_model.detect_sparse_features_on_panorama(feature_detection_method="GFT", num_of_features=60,
+                                                            median_win_size=11, show=False)
+    finally:
+        pano_obj.panoramic_img, pano_obj.azimuthal_masks = saved

@@ -5,11 +5,15 @@
 //           (camera_models.py:1737), i.e. cv::cornerMinEigenVal (blockSize 3, Sobel 3) + threshold at
 //           quality * max over the mask + 3x3 non-maximum suppression + strongest-first minimum-distance selection.
 //
-// Arithmetic of cornerMinEigenVal, identified against cv2 (scratch probes, see DESIGN.md): Sobel in float32 with the scale
-// 1/(4*3*255) folded into the smoothing taps and one fused multiply-add, dx = fma(s, r[-1] + r[+1], 2s * r[0]); covariance
-// products in float32; the 3x3 box sums accumulate in float64 and are rounded once; eigenvalue (a + c) - sqrt((a - c)^2 + b^2)
-// in float32 without contraction.  cv2's own SIMD tail columns skip the FMA, so a handful of pixels per row end differ
-// in the last bit from cv2 — the detected corners are the same except for exact near-ties.
+// Arithmetic of cornerMinEigenVal, identified against cv2 (the tests restate it operation by operation in NumPy): Sobel in
+// float32 with the scale s = 1/(4*3*255) folded into the smoothing taps.  dx: rows differentiated exactly, then smoothed
+// down the column with one fused multiply-add, dx = fma(s, d[-1] + d[+1], 2s * d[0]).  dy: each row smoothed in tap order
+// as cv2's row filter accumulates it, fma(s, g[x+1], fma(2s, g[x], s * g[x-1])), then the row above subtracted from the
+// row below.  Covariance products in float32; the 3x3 box sums accumulate in float64 ((p[-1] + p[0]) + p[+1] along the
+// row, then down the column) and are rounded once; eigenvalue (a + c) - sqrt((a - c)^2 + b^2) in float32 without
+// contraction.  cv2 itself differs in its SIMD tail columns (the last <= 16 of a row, which skip the FMA) and, on sharp
+// images, at a few interior pixels where its sliding-window box sums round differently (by at most half a unit of the
+// image's largest measure).
 //
 // Selection: candidates of one (image, mask) are sorted by (strength desc, pixel index desc) — cv2's comparator — and the
 // strongest-first greedy of cv2 is evaluated in parallel rounds (a candidate is accepted once every stronger candidate
@@ -31,9 +35,9 @@ __device__ __forceinline__ int refl(int p, int n) {
   return p;
 }
 
-// Corner measure + (optionally) the maximum over each mask, fused.  Per pixel: Sobel derivatives (cv2's arithmetic: rows
-// differentiated exactly, columns smoothed with (s, 2s, s), one FMA), covariance terms dx^2, dx dy, dy^2 in float32, their
-// 3 x 3 box sums in double (cv2's RowSum<float,double> / ColumnSum<double,float>), smaller eigenvalue without contraction.
+// Corner measure + (optionally) the maximum over each mask, fused.  Per pixel: Sobel derivatives (cv2's arithmetic, see the
+// top of the file), covariance terms dx^2, dx dy, dy^2 in float32, their 3 x 3 box sums in double (cv2's
+// RowSum<float,double> / ColumnSum<double,float>), smaller eigenvalue without contraction.
 // Every thread walks down its column with the 3-tap row sums of the last three rows in registers and recomputes the
 // covariance terms of its three columns from the gray image, so nothing but the gray image is read and nothing but the
 // measure is written.  (First version: a covariance image of 12 bytes per pixel written by one kernel and pulled through L2
@@ -74,8 +78,8 @@ gft_eig_kernel(const uint8_t* __restrict__ gray, int H, int W, float* __restrict
       const float a20 = rd[cx[j][0]], a21 = rd[cx[j][1]], a22 = rd[cx[j][2]];
       const float du = a02 - a00, d0 = a12 - a10, dd = a22 - a20;
       const float dx = __fmaf_rn(s, du + dd, __fmul_rn(s2, d0));
-      const float su = __fmaf_rn(s, a00 + a02, __fmul_rn(s2, a01));
-      const float sd = __fmaf_rn(s, a20 + a22, __fmul_rn(s2, a21));
+      const float su = __fmaf_rn(s, a02, __fmaf_rn(s2, a01, __fmul_rn(s, a00)));
+      const float sd = __fmaf_rn(s, a22, __fmaf_rn(s2, a21, __fmul_rn(s, a20)));
       const float dy = __fsub_rn(sd, su);
       pxx[j] = __fmul_rn(dx, dx);
       pxy[j] = __fmul_rn(dx, dy);
@@ -86,8 +90,8 @@ gft_eig_kernel(const uint8_t* __restrict__ gray, int H, int W, float* __restrict
     cc = ((double)pyy[0] + (double)pyy[1]) + (double)pyy[2];
   };
   // Fast path (warp-uniform): no reflection anywhere in the strip.  Per gray row and column, D = g[x+1] - g[x-1] and
-  // S = fma(s, g[x-1] + g[x+1], 2s g[x]) are computed once and serve the three product rows that touch the row (same
-  // operations, same order as the generic path: bit-identical).
+  // S = fma(s, g[x+1], fma(2s, g[x], s g[x-1])) are computed once and serve the three product rows that touch the row
+  // (same operations, same order as the generic path: bit-identical).
   const bool fast = __all_sync(0xFFFFFFFFu, in && x >= 2 && x + 2 < W) && y0 >= 2 && y1 <= H - 2;
   float D[3][3], S[3][3];
   uint8_t raw[5];                                  // the gray row after next, loaded one iteration ahead of its use
@@ -103,7 +107,7 @@ gft_eig_kernel(const uint8_t* __restrict__ gray, int H, int W, float* __restrict
 #pragma unroll
     for (int j = 0; j < 3; ++j) {
       Dr[j] = v[j + 2] - v[j];
-      Sr[j] = __fmaf_rn(s, v[j] + v[j + 2], __fmul_rn(s2, v[j + 1]));
+      Sr[j] = __fmaf_rn(s, v[j + 2], __fmaf_rn(s2, v[j + 1], __fmul_rn(s, v[j])));
     }
   };
   auto fast_sums = [&](double& a, double& b, double& cc) {
@@ -301,8 +305,8 @@ gft_select_kernel(const unsigned long long* __restrict__ keys_in, const int32_t*
   const int list = img * n_masks + mk;
   const int tag = mk << 16;
   if (counts[list] > cap) {
-    // more local maxima than the candidate buffer holds: the atomics that filled it kept a schedule-dependent subset, so
-    // refuse instead of returning a corner set that can change from run to run (out_count < 0 = -candidates)
+    // more local maxima than the candidate buffer holds (the host refuses the call before launching; this keeps the
+    // kernel inside its shared memory whatever it is given)
     if (threadIdx.x == 0) out_count[list] = -counts[list];
     return;
   }
@@ -525,10 +529,12 @@ extern "C" int sos_gft_detect(sos_ctx* ctx, const uint8_t* gray, const uint8_t* 
                               int n_masks, int max_corners, double quality_level, double min_distance, float* out_xy,
                               int32_t* out_count, float* eig_out) {
   SOS_CHECK_ARG(ctx, "ctx is NULL");
-  SOS_CHECK_ARG(n_images >= 0 && height >= 0 && width >= 0 && n_masks >= 1 && n_masks <= 32 && max_corners >= 0, "bad size (at most 32 masks)");
+  SOS_CHECK_ARG(n_images >= 0 && height >= 0 && width >= 0 && n_masks >= 1 && n_masks <= 32, "bad size (at most 32 masks)");
+  // cv2 reads maxCorners <= 0 as "no limit"; here it sizes out_xy, so a limit is required
+  SOS_CHECK_ARG(max_corners >= 1, "max_corners must be >= 1");
   SOS_CHECK_ARG(quality_level > 0.0 && min_distance >= 0.0 && min_distance < 64.0, "bad quality level / minimum distance");
   if (n_images == 0) return SOS_OK;
-  SOS_CHECK_ARG(gray && out_count && (out_xy || max_corners == 0), "NULL array");
+  SOS_CHECK_ARG(gray && out_count && out_xy, "NULL array");
   SOS_CHECK_ARG(height >= 3 && width >= 3 && (size_t)height * width < (1ull << 31), "image size out of range");
   SOS_CHECK_ARG((long long)n_images * n_masks <= 65535, "too many (image, mask) lists");
   SOS_CUDA(cudaSetDevice(ctx->device));
@@ -575,29 +581,28 @@ extern "C" int sos_gft_detect(sos_ctx* ctx, const uint8_t* gray, const uint8_t* 
   const double md2 = min_distance * min_distance;
   const int min_dist_sq = min_distance >= 1.0 ? (int)ceil(md2) : 0;   // integer offsets: dx^2 + dy^2 < minDistance^2
   const int reach = (int)ceil(min_distance);
+  // One small read-back on every call: the overlap flag and the candidate counts.  A list with more candidates than the
+  // buffer holds is refused (the atomics that filled the buffer kept a schedule-dependent subset), and the largest count
+  // sizes the selection's shared memory (a block sorts next_pow2(count) keys: 64 KB instead of 128 KB lets three blocks
+  // share an SM).
+  int overlap = 0;
+  std::vector<int32_t> hc(lists);
+  SOS_CUDA(cudaMemcpyAsync(&overlap, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  SOS_CUDA(cudaMemcpyAsync(hc.data(), counts, sizeof(int32_t) * lists, cudaMemcpyDeviceToHost, ctx->stream));
+  SOS_CUDA(cudaStreamSynchronize(ctx->stream));
+  int mx = 1;
+  for (int v : hc) {
+    if (v > GFT_CAP) {
+      sos_set_error("sos_gft_detect: %d corner candidates in one mask, the selection holds %d: raise quality_level", v, GFT_CAP);
+      return SOS_ERR_INVALID;
+    }
+    mx = std::max(mx, v);
+  }
+  int np2 = 1024;
+  while (np2 < mx) np2 <<= 1;
+  const size_t sel_smem = gft_select_smem(np2);
   // pixel-disjoint masks (the reference's default, overlap_degrees = 0): every list at once.  Overlapping masks: a pixel can
   // be a candidate of two lists and each selection needs the rank image of its image to itself -> one launch per mask.
-  int overlap = 0;
-  size_t sel_smem = smem;
-  if (masks && n_masks > 1) {
-    // one small read-back: the overlap flag and the candidate counts, which size the selection's shared memory (a block
-    // sorts next_pow2(count) keys: 64 KB instead of 128 KB lets three blocks share an SM)
-    std::vector<int32_t> hc(lists);
-    SOS_CUDA(cudaMemcpyAsync(&overlap, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-    SOS_CUDA(cudaMemcpyAsync(hc.data(), counts, sizeof(int32_t) * lists, cudaMemcpyDeviceToHost, ctx->stream));
-    SOS_CUDA(cudaStreamSynchronize(ctx->stream));
-    int mx = 1;
-    for (int v : hc) {
-      if (v > GFT_CAP) {
-        sos_set_error("sos_gft_detect: %d corner candidates in one mask, the selection holds %d: raise quality_level", v, GFT_CAP);
-        return SOS_ERR_INVALID;
-      }
-      mx = std::max(mx, v);
-    }
-    int np2 = 1024;
-    while (np2 < mx) np2 <<= 1;
-    sel_smem = gft_select_smem(np2);
-  }
   if (!overlap) {
     gft_select_kernel<<<lists, GFT_THREADS, sel_smem, ctx->stream>>>(keys, counts, GFT_CAP, height, width, n_masks, -1, max_corners,
                                                                  min_dist_sq, reach, rank_img, out_xy, out_count);
