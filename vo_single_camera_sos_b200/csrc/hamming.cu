@@ -14,26 +14,7 @@
 //     the per-split partial keys are merged by a second, tiny kernel.
 #include <stdlib.h>
 
-#include "sos_common.cuh"
-
-// tensor-core engine (hamming_mma.cu)
-size_t sos_hamming_mma_scratch_bytes(int n_seg, int max_nq, int max_nt);
-int sos_hamming_mma_launch(sos_ctx* ctx, const uint32_t* q, const uint32_t* t, const int32_t* q_start, const int32_t* q_len,
-                           const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int splits,
-                           const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* exp,
-                           uint2* partial);
-
-size_t sos_l2_mma_scratch_bytes(int n_seg, int max_nq, int max_nt);
-int sos_l2_mma_launch(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start, const int32_t* q_len,
-                      const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int splits,
-                      const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* exp,
-                      ulonglong2* partial, int32_t* flag);
-
-size_t sos_l2f_scratch_bytes(int n_seg, int max_nq, int max_nt, int dim, int splits);
-int sos_l2f_launch(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start, const int32_t* q_len,
-                   const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int splits,
-                   const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* scratch,
-                   int32_t* idx0, float* d0, int32_t* idx1, float* d1, int32_t* flag, int32_t* stats);
+#include "match_common.cuh"
 
 namespace {
 
@@ -41,8 +22,7 @@ constexpr int HB_THREADS = 128;  // threads per block
 constexpr int HB_QPT = 2;        // query descriptors per thread
 constexpr int HB_TILE_Q = HB_THREADS * HB_QPT;
 constexpr int HB_TILE_T = 256;   // train descriptors per shared-memory tile (8 KB)
-constexpr int KEY_IDX_BITS = 22; // up to 4M train rows per segment; distance <= 256 needs 9 bits
-constexpr uint32_t KEY_NONE = 0xFFFFFFFFu;
+static_assert(HB_TILE_Q == ITEM_QROWS, "a block covers the query rows of one work item");
 
 // carry-save adder on 32 bit lanes: a + b + c = sum + 2 * carry (one LOP3 each)
 // Written as two explicit LOP3s (truth tables 0x96 = a^b^c, 0xE8 = majority): left to itself the compiler re-factors
@@ -68,45 +48,6 @@ __device__ __forceinline__ uint32_t hamming_key(const uint4& qa, const uint4& qb
   const uint32_t ones = __popc(s3) + __popc(x7);
   const uint32_t twos = __popc(c1) + __popc(c2) + __popc(c3);
   return twos * (2u << KEY_IDX_BITS) + (ones * (1u << KEY_IDX_BITS) + tj);
-}
-
-// Work list: segment lengths live on the device, so the host can only size the grid for the worst case.  Launching
-// that grid directly leaves the SMs unevenly loaded (blocks of short segments exit at once and everything fits in
-// one wave: measured 66 % average SM activity).  Instead one small block compacts the ACTIVE (segment, query tile,
-// train split) items into a list; block i of the main kernel takes item i, so the active blocks are contiguous in
-// launch order and the hardware scheduler balances them.
-constexpr int ITEM_SPLIT_BITS = 6, ITEM_TILE_BITS = 10;  // item = seg << 16 | tile << 6 | split
-
-__global__ void __launch_bounds__(256)
-hamming_plan_kernel(const int32_t* __restrict__ q_len, int n_seg, int max_nq, int splits, uint32_t* __restrict__ items,
-                    int32_t* __restrict__ n_items) {
-  __shared__ int warp_tot[8];
-  __shared__ int carry_sh;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  if (tid == 0) carry_sh = 0;
-  __syncthreads();
-  for (int base = 0; base < n_seg; base += 256) {
-    const int seg = base + tid;
-    const int tiles = seg < n_seg ? (min(q_len[seg], max_nq) + HB_TILE_Q - 1) / HB_TILE_Q : 0;
-    const int cnt = tiles * splits;
-    int incl = cnt;
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-      const int v = __shfl_up_sync(0xFFFFFFFFu, incl, off);
-      if (lane >= off) incl += v;
-    }
-    if (lane == 31) warp_tot[warp] = incl;
-    __syncthreads();
-    int before = carry_sh;
-    for (int w = 0; w < warp; ++w) before += warp_tot[w];
-    const int first = before + incl - cnt;
-    for (int k = 0; k < cnt; ++k)
-      items[first + k] = ((uint32_t)seg << 16) | ((uint32_t)(k / splits) << ITEM_SPLIT_BITS) | (uint32_t)(k % splits);
-    __syncthreads();
-    if (tid == 255) carry_sh = before + incl;
-    __syncthreads();
-  }
-  if (tid == 0) *n_items = carry_sh;
 }
 
 template <bool TOP2>
@@ -179,30 +120,6 @@ hamming_partial_kernel(const uint4* __restrict__ q, const uint4* __restrict__ t,
     const int row = q_tile + r * HB_THREADS + threadIdx.x;
     if (row < nq) partial[((size_t)seg * max_nq + row) * splits + split] = make_uint2(k0[r], k1[r]);
   }
-}
-
-__global__ void __launch_bounds__(256)
-hamming_merge_kernel(const uint2* __restrict__ partial, const int32_t* __restrict__ q_start,
-                     const int32_t* __restrict__ q_len, int max_nq, int splits, int32_t* __restrict__ idx0,
-                     int32_t* __restrict__ d0, int32_t* __restrict__ idx1, int32_t* __restrict__ d1) {
-  const int seg = blockIdx.y;
-  const int q0 = q_start[seg], nq = min(q_len[seg], max_nq);
-  const int row = blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= nq) return;
-  const uint2* p = partial + ((size_t)seg * max_nq + row) * splits;
-  uint32_t k0 = KEY_NONE, k1 = KEY_NONE;
-  for (int s = 0; s < splits; ++s) {
-    const uint2 v = p[s];
-    // merge two sorted pairs: v.x <= v.y
-    k1 = min(k1, max(k0, v.x));
-    k0 = min(k0, v.x);
-    k1 = min(k1, v.y);  // v.y >= v.x, so it can only compete for second place
-  }
-  const uint32_t mask = (1u << KEY_IDX_BITS) - 1u;
-  idx0[q0 + row] = (k0 == KEY_NONE) ? -1 : (int32_t)(k0 & mask);
-  d0[q0 + row] = (k0 == KEY_NONE) ? -1 : (int32_t)(k0 >> KEY_IDX_BITS);
-  if (idx1) idx1[q0 + row] = (k1 == KEY_NONE) ? -1 : (int32_t)(k1 & mask);
-  if (d1) d1[q0 + row] = (k1 == KEY_NONE) ? -1 : (int32_t)(k1 >> KEY_IDX_BITS);
 }
 
 // ---------------------------------------------------------------------------------------------------
@@ -332,9 +249,8 @@ extern "C" int sos_hamming_top2(sos_ctx* ctx, const uint32_t* q, const uint32_t*
   SOS_CHECK_ARG(((uintptr_t)q & 15) == 0 && ((uintptr_t)t & 15) == 0, "descriptor arrays must be 16-byte aligned");
   SOS_CUDA(cudaSetDevice(ctx->device));
 
-  const int q_tiles = sos_div_up(max_nq, HB_TILE_Q);
+  const int q_tiles = sos_div_up(max_nq, ITEM_QROWS);
   SOS_CHECK_ARG(q_tiles <= (1 << ITEM_TILE_BITS), "segment has too many query rows (limit 262144)");
-  const bool top2 = idx1 != nullptr || d1 != nullptr;
   // engine: "popc" = XOR + POPC on the integer pipe, "mma" = int8 tensor cores (hamming_mma.cu).  Default: the tensor-core
   // engine once a segment can fill a few 128 x 128 tiles; below that its fixed cost (expansion, 180 KB of shared memory per
   // CTA, TMEM allocation) is not repaid.  SOS_HAMMING_ENGINE overrides (read per call; both engines run the same tests).
@@ -342,34 +258,26 @@ extern "C" int sos_hamming_top2(sos_ctx* ctx, const uint32_t* q, const uint32_t*
   bool use_mma = max_nq >= 256 && max_nt >= 512;
   if (eng && eng[0] == 'p') use_mma = false;
   if (eng && eng[0] == 'm') use_mma = max_nt > 0;
+  if (use_mma)
+    return sos_tc_match(ctx, sos_tc::KIND_HAMMING, q, t, 0, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, idx0, d0,
+                        idx1, d1, nullptr, nullptr);
 
-  int splits;
-  if (use_mma) {
-    // a work item is 256 query rows x (train tiles / splits); keep >= 4 train tiles per item (the two query tiles of an
-    // item are fetched once per item) unless that starves the SMs
-    const int t_tiles = sos_div_up(max_nt, 128);
-    splits = sos_div_up(2 * ctx->sm_count, q_tiles * n_seg);
-    if (splits > t_tiles / 4) splits = t_tiles / 4;
-  } else {
-    // split the train range so that a work item is ~256 x 1024 descriptor pairs and small problems still give every SM
-    // several items; never finer than one shared-memory tile
-    const int t_tiles = sos_div_up(max_nt > 0 ? max_nt : 1, HB_TILE_T);
-    splits = sos_div_up(max_nt > 0 ? max_nt : 1, 1024);
-    const int fill = sos_div_up(4 * ctx->sm_count, q_tiles * n_seg);
-    if (splits < fill) splits = fill;
-    if (splits > t_tiles) splits = t_tiles;
-  }
+  // split the train range so that a work item is ~256 x 1024 descriptor pairs and small problems still give every SM
+  // several items; never finer than one shared-memory tile
+  const int t_tiles = sos_div_up(max_nt > 0 ? max_nt : 1, HB_TILE_T);
+  int splits = sos_div_up(max_nt > 0 ? max_nt : 1, 1024);
+  const int fill = sos_div_up(4 * ctx->sm_count, q_tiles * n_seg);
+  if (splits < fill) splits = fill;
+  if (splits > t_tiles) splits = t_tiles;
   if (splits > (1 << ITEM_SPLIT_BITS)) splits = 1 << ITEM_SPLIT_BITS;
   if (splits < 1) splits = 1;
 
   void* ws = nullptr;
-  const size_t rows_bound = (size_t)max_nq * (size_t)n_seg;
   const size_t max_items = (size_t)q_tiles * splits * n_seg;
   SOS_CHECK_ARG(max_items < ((size_t)1 << 31), "too many work items");
-  const size_t partial_bytes = sos_align_up(rows_bound * splits * sizeof(uint2), 256);
+  const size_t partial_bytes = sos_align_up((size_t)max_nq * n_seg * splits * sizeof(uint2), 256);
   const size_t items_bytes = sos_align_up(max_items * sizeof(uint32_t), 256);
-  const size_t exp_bytes = use_mma ? sos_hamming_mma_scratch_bytes(n_seg, max_nq, max_nt) : 0;
-  int rc = sos_arena_get(ctx, partial_bytes + items_bytes + 256 + exp_bytes, &ws);
+  int rc = sos_arena_get(ctx, partial_bytes + items_bytes + 256, &ws);
   if (rc != SOS_OK) return rc;
   uint32_t* items = (uint32_t*)((char*)ws + partial_bytes);
   int32_t* n_items = (int32_t*)((char*)ws + partial_bytes + items_bytes);
@@ -377,21 +285,15 @@ extern "C" int sos_hamming_top2(sos_ctx* ctx, const uint32_t* q, const uint32_t*
   hamming_plan_kernel<<<1, 256, 0, ctx->stream>>>(q_len, n_seg, max_nq, splits, items, n_items);
   SOS_LAUNCHED_AS(ctx, "hamming_plan_kernel");
   const unsigned grid = (unsigned)max_items;
-  if (use_mma) {
-    rc = sos_hamming_mma_launch(ctx, q, t, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, splits, items, n_items,
-                                grid, top2, (char*)ws + partial_bytes + items_bytes + 256, (uint2*)ws);
-    if (rc != SOS_OK) return rc;
-  } else {
 #define HB_LAUNCH(T2)                                                                                                  \
   hamming_partial_kernel<T2><<<grid, HB_THREADS, 0, ctx->stream>>>((const uint4*)q, (const uint4*)t, q_start, q_len,    \
                                                                    t_start, t_len, max_nq, max_nt, splits, items,      \
                                                                    n_items, (uint2*)ws)
-    if (top2) HB_LAUNCH(true); else HB_LAUNCH(false);
+  if (idx1 || d1) HB_LAUNCH(true); else HB_LAUNCH(false);
 #undef HB_LAUNCH
-    SOS_LAUNCHED_AS(ctx, "hamming_partial_kernel");
-  }
-  dim3 mgrid(sos_div_up(max_nq, 256), n_seg);
-  hamming_merge_kernel<<<mgrid, 256, 0, ctx->stream>>>((const uint2*)ws, q_start, q_len, max_nq, splits, idx0, d0, idx1, d1);
+  SOS_LAUNCHED_AS(ctx, "hamming_partial_kernel");
+  merge_kernel<<<dim3(sos_div_up(max_nq, 256), n_seg), 256, 0, ctx->stream>>>((const uint2*)ws, q_start, q_len, max_nq, splits,
+                                                                               idx0, d0, idx1, d1);
   SOS_LAUNCHED_AS(ctx, "hamming_merge_kernel");
   return SOS_OK;
 }
@@ -454,31 +356,6 @@ extern "C" int sos_hamming_radius(sos_ctx* ctx, const uint32_t* q, int nq, const
 // ---------------------------------------------------------------------------------------------------
 // Float descriptors, L2 norm (cv2.BFMatcher() of the SIFT / SURF branch, camera_models.py:397-399): tensor-core engine only.
 // ---------------------------------------------------------------------------------------------------
-namespace {
-__global__ void __launch_bounds__(256)
-l2_merge_kernel(const ulonglong2* __restrict__ partial, const int32_t* __restrict__ q_start, const int32_t* __restrict__ q_len,
-                int max_nq, int splits, int32_t* __restrict__ idx0, float* __restrict__ d0, int32_t* __restrict__ idx1,
-                float* __restrict__ d1) {
-  const int seg = blockIdx.y;
-  const int q0 = q_start[seg], nq = min(q_len[seg], max_nq);
-  const int row = blockIdx.x * blockDim.x + threadIdx.x;
-  if (row >= nq) return;
-  const ulonglong2* p = partial + ((size_t)seg * max_nq + row) * splits;
-  unsigned long long k0 = ~0ull, k1 = ~0ull;
-  for (int s = 0; s < splits; ++s) {
-    const ulonglong2 v = p[s];
-    k1 = min(k1, max(k0, v.x));
-    k0 = min(k0, v.x);
-    k1 = min(k1, v.y);
-  }
-  // cv2 reports sqrt of the float32 sum of squared differences; the sum is an exact integer < 2^24 here
-  idx0[q0 + row] = (k0 == ~0ull) ? -1 : (int32_t)(k0 & 0xFFFFFFFFull);
-  d0[q0 + row] = (k0 == ~0ull) ? -1.f : sqrtf((float)(uint32_t)(k0 >> 32));
-  if (idx1) idx1[q0 + row] = (k1 == ~0ull) ? -1 : (int32_t)(k1 & 0xFFFFFFFFull);
-  if (d1) d1[q0 + row] = (k1 == ~0ull) ? -1.f : sqrtf((float)(uint32_t)(k1 >> 32));
-}
-}  // namespace
-
 extern "C" int sos_l2_top2(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start,
                            const int32_t* q_len, const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq,
                            int max_nt, int32_t* idx0, float* d0, int32_t* idx1, float* d1, int32_t* not_integer_flag) {
@@ -489,34 +366,10 @@ extern "C" int sos_l2_top2(sos_ctx* ctx, const float* q, const float* t, int dim
   if (n_seg == 0 || max_nq == 0) return SOS_OK;
   SOS_CHECK_ARG(q && t && q_start && q_len && t_start && t_len && idx0 && d0 && not_integer_flag, "NULL array");
   SOS_CUDA(cudaSetDevice(ctx->device));
-  const int q_tiles = sos_div_up(max_nq, HB_TILE_Q);
-  SOS_CHECK_ARG(q_tiles <= (1 << ITEM_TILE_BITS), "segment has too many query rows (limit 262144)");
-  const bool top2 = idx1 != nullptr || d1 != nullptr;
-  const int t_tiles = sos_div_up(max_nt > 0 ? max_nt : 1, 128);
-  int splits = sos_div_up(2 * ctx->sm_count, q_tiles * n_seg);
-  if (splits > t_tiles / 4) splits = t_tiles / 4;
-  if (splits > (1 << ITEM_SPLIT_BITS)) splits = 1 << ITEM_SPLIT_BITS;
-  if (splits < 1) splits = 1;
-  void* ws = nullptr;
-  const size_t max_items = (size_t)q_tiles * splits * n_seg;
-  SOS_CHECK_ARG(max_items < ((size_t)1 << 31), "too many work items");
-  const size_t partial_bytes = sos_align_up((size_t)max_nq * n_seg * splits * sizeof(ulonglong2), 256);
-  const size_t items_bytes = sos_align_up(max_items * sizeof(uint32_t), 256);
-  int rc = sos_arena_get(ctx, partial_bytes + items_bytes + 256 + sos_l2_mma_scratch_bytes(n_seg, max_nq, max_nt), &ws);
-  if (rc != SOS_OK) return rc;
-  uint32_t* items = (uint32_t*)((char*)ws + partial_bytes);
-  int32_t* n_items = (int32_t*)((char*)ws + partial_bytes + items_bytes);
+  SOS_CHECK_ARG(sos_div_up(max_nq, ITEM_QROWS) <= (1 << ITEM_TILE_BITS), "segment has too many query rows (limit 262144)");
   SOS_CUDA(cudaMemsetAsync(not_integer_flag, 0, sizeof(int32_t), ctx->stream));
-  hamming_plan_kernel<<<1, 256, 0, ctx->stream>>>(q_len, n_seg, max_nq, splits, items, n_items);
-  SOS_LAUNCHED_AS(ctx, "hamming_plan_kernel");
-  rc = sos_l2_mma_launch(ctx, q, t, dim, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, splits, items, n_items,
-                         (unsigned)max_items, top2, (char*)ws + partial_bytes + items_bytes + 256, (ulonglong2*)ws,
-                         not_integer_flag);
-  if (rc != SOS_OK) return rc;
-  dim3 mgrid(sos_div_up(max_nq, 256), n_seg);
-  l2_merge_kernel<<<mgrid, 256, 0, ctx->stream>>>((const ulonglong2*)ws, q_start, q_len, max_nq, splits, idx0, d0, idx1, d1);
-  SOS_LAUNCHED_AS(ctx, "l2_merge_kernel");
-  return SOS_OK;
+  return sos_tc_match(ctx, sos_tc::KIND_L2, q, t, dim, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, idx0, d0, idx1, d1,
+                      not_integer_flag, nullptr);
 }
 
 // Any finite float descriptors: the split-bfloat16 GEMM ranks, float64 decides (hamming_mma.cu: band, kernels).
@@ -532,27 +385,10 @@ extern "C" int sos_l2f_top2(sos_ctx* ctx, const float* q, const float* t, int di
   if (n_seg == 0 || max_nq == 0) return SOS_OK;
   SOS_CHECK_ARG(q && t && q_start && q_len && t_start && t_len && idx0 && d0 && nonfinite_flag, "NULL array");
   SOS_CUDA(cudaSetDevice(ctx->device));
-  const int q_tiles = sos_div_up(max_nq, HB_TILE_Q);
-  SOS_CHECK_ARG(q_tiles <= (1 << ITEM_TILE_BITS), "segment has too many query rows (limit 262144)");
-  const bool top2 = idx1 != nullptr || d1 != nullptr;
-  const int t_tiles = sos_div_up(max_nt > 0 ? max_nt : 1, 128);
-  int splits = sos_div_up(2 * ctx->sm_count, q_tiles * n_seg);
-  if (splits > t_tiles / 4) splits = t_tiles / 4;
-  if (splits > (1 << ITEM_SPLIT_BITS)) splits = 1 << ITEM_SPLIT_BITS;
-  if (splits < 1) splits = 1;
-  void* ws = nullptr;
-  const size_t max_items = (size_t)q_tiles * splits * n_seg;
-  SOS_CHECK_ARG(max_items < ((size_t)1 << 31), "too many work items");
-  const size_t items_bytes = sos_align_up(max_items * sizeof(uint32_t), 256);
-  int rc = sos_arena_get(ctx, items_bytes + 256 + sos_l2f_scratch_bytes(n_seg, max_nq, max_nt, dim, splits), &ws);
-  if (rc != SOS_OK) return rc;
-  uint32_t* items = (uint32_t*)ws;
-  int32_t* n_items = (int32_t*)((char*)ws + items_bytes);
+  SOS_CHECK_ARG(sos_div_up(max_nq, ITEM_QROWS) <= (1 << ITEM_TILE_BITS), "segment has too many query rows (limit 262144)");
   SOS_CUDA(cudaMemsetAsync(nonfinite_flag, 0, sizeof(int32_t), ctx->stream));
-  hamming_plan_kernel<<<1, 256, 0, ctx->stream>>>(q_len, n_seg, max_nq, splits, items, n_items);
-  SOS_LAUNCHED_AS(ctx, "hamming_plan_kernel");
-  return sos_l2f_launch(ctx, q, t, dim, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, splits, items, n_items,
-                        (unsigned)max_items, top2, (char*)ws + items_bytes + 256, idx0, d0, idx1, d1, nonfinite_flag, stats);
+  return sos_tc_match(ctx, sos_tc::KIND_L2F, q, t, dim, q_start, q_len, t_start, t_len, n_seg, max_nq, max_nt, idx0, d0, idx1,
+                      d1, nonfinite_flag, stats);
 }
 
 extern "C" int sos_match_select(sos_ctx* ctx, int mode, double ratio, const int32_t* idx0, const int32_t* d0,

@@ -29,11 +29,11 @@
 //                   shared-memory stage and publishes the accumulator
 //   warp 2        : tensor-memory allocation
 //   warps 4..11   : epilogue, one thread per (query tile, row)
-// The per-split partial keys use the POPC engine's format and are merged by the same hamming_merge_kernel.
+// The per-split partial keys use the POPC engine's format and are merged by the same merge_kernel (match_common.cuh).
+// The two float-descriptor L2 engines (sos_l2_top2, sos_l2f_top2) are the same kernel with bfloat16 operands: see KIND.
 #include <cuda_bf16.h>
 
-#include "sos_common.cuh"
-#include "tc_common.cuh"
+#include "match_common.cuh"
 
 namespace sos_hamming_mma {
 
@@ -45,9 +45,7 @@ constexpr int TILE_BYTES = (TILE / 8) * GROUP_BYTES;  // 36864
 constexpr int THREADS = 384;
 constexpr int smem_bytes(int stages) { return (2 + stages) * TILE_BYTES + 256; }
 constexpr int PAD_DROP = 30 * 127 * 128;         // what the 30 pad columns subtract from a padding row's accumulator
-constexpr int KEY_IDX_BITS = 22;                 // must match hamming.cu
-constexpr uint32_t KEY_NONE = 0xFFFFFFFFu;
-constexpr int ITEM_SPLIT_BITS = 6, ITEM_TILE_BITS = 10;   // item = seg << 16 | tile << 6 | split (hamming.cu)
+static_assert(ITEM_QROWS == 2 * TILE, "a work item is two query tiles");
 
 // ---- expansion ------------------------------------------------------------------------------------------------------
 // four descriptor bits -> four int8 values: bit 0 -> +16, bit 1 -> -16
@@ -119,6 +117,28 @@ __device__ __forceinline__ uint64_t smem_desc(uint32_t addr) { return sos_tc::sm
 constexpr uint32_t IDESC = (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TILE >> 3) << 17) | ((uint32_t)(TILE >> 4) << 24);
 // the float-descriptor L2 engine: D = F32 (1 << 4), A = B = BF16 (1 << 7, 1 << 10), both K-major, N = 128, M = 128
 constexpr uint32_t IDESC_L2 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(TILE >> 3) << 17) | ((uint32_t)(TILE >> 4) << 24);
+
+// The MMAs of one (query tile, train sub-tile j) pair into the accumulator at d.  Hamming and L2: one sub-tile per tile,
+// 9 instructions over the 288 bytes of K.  L2F: sub-tile j of a row holds [hi (64) | mid (64) | 16 more] bf16 of the values
+// 64 j .. 64 j + 63; the products hi*hi, hi*mid and mid*hi of each 16-value block come from the same two tiles at different
+// K offsets (descriptor + 16 per 256 bytes), and sub-tile 0 adds the |t|^2 columns: for dim = 64 that is 4 x 3 + 1 = 13
+// instructions per tile pair, for dim = 128 25.
+template <int KIND>
+__device__ __forceinline__ void issue_tile_pair(uint32_t d, uint64_t da, uint64_t db, int j, int dim) {
+  if (KIND == KIND_L2F) {
+    const int nk = (min(64, dim - 64 * j) + 15) >> 4;
+    if (j == 0) tc_mma<KIND>(d, da + 128u, db + 128u, IDESC_L2, 0u);     // 1 x (-|t|^2 pieces)
+    for (int kk = 0; kk < nk; ++kk) {
+      tc_mma<KIND>(d, da + (uint64_t)(16 * kk), db + (uint64_t)(16 * kk), IDESC_L2, 1u);            // hi * hi
+      tc_mma<KIND>(d, da + (uint64_t)(16 * kk), db + (uint64_t)(16 * (4 + kk)), IDESC_L2, 1u);      // hi * mid
+      tc_mma<KIND>(d, da + (uint64_t)(16 * (4 + kk)), db + (uint64_t)(16 * kk), IDESC_L2, 1u);      // mid * hi
+    }
+  } else {
+#pragma unroll
+    for (int kk = 0; kk < KB / 32; ++kk)
+      tc_mma<KIND>(d, da + (uint64_t)(16 * kk), db + (uint64_t)(16 * kk), KIND == KIND_L2 ? IDESC_L2 : IDESC, kk > 0);
+  }
+}
 
 template <bool TOP2>
 __device__ __forceinline__ void reduce32(const int (&v)[32], int& m0, int& m1) {
@@ -235,16 +255,20 @@ __device__ __forceinline__ Item decode_item(const Args& a, uint32_t item) {
 // buffer, query tiles) live across items, so in the persistent shape the tensor pipe only idles while the next item's query
 // tiles land (the train tiles of the next item are already streaming into the ring by then).  The roles agree on every
 // counter because they walk the same items in the same order:
-//   t  = train tiles consumed so far by this CTA -> ring stage t % STAGES, accumulator buffer t & 1
-//   ic = items with work so far                  -> phase of the query-tile barriers
+//   t  = train tiles consumed so far by this CTA     -> accumulator buffer t & 1
+//   r  = train sub-tiles consumed so far (t * nsub + j for sub-tile j of tile t) -> ring stage r % ns
+//   ic = items with work so far                      -> phase of the query-tile barriers
 template <bool TOP2, int STAGES, int KIND>
 __global__ void __launch_bounds__(THREADS, 1) mma_kernel(Args a) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const int n_items = *a.n_items;
   if ((int)blockIdx.x >= n_items) return;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  // A 128-row tile is nsub 288-byte sub-tiles (36 KB each): 1 for Hamming and L2, 1 or 2 for L2F (dim <= 64, dim <= 128).
+  // The two query tiles of an item take 2 nsub of the STAGES + 2 buffers, the ring of train sub-tiles the remaining ns.
+  const int nsub = KIND == KIND_L2F ? a.nsub : 1, ns = STAGES + 2 - 2 * nsub;
   uint8_t* sA = smem;
-  uint8_t* sB = smem + 2 * TILE_BYTES;
+  uint8_t* sB = smem + 2 * nsub * TILE_BYTES;
   uint64_t* bars = (uint64_t*)(smem + (2 + STAGES) * TILE_BYTES);
   // bars: FULL + s (train stage landed), EMPTY + s (stage consumed), TFULL + b (accumulator complete), TEMPTY + b
   // (accumulator drained), AFULL (query tiles landed), AEMPTY (query tiles no longer read by the tensor core)
@@ -269,22 +293,19 @@ __global__ void __launch_bounds__(THREADS, 1) mma_kernel(Args a) {
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
 
-  if (KIND == KIND_L2F && warp == 0) {
-    // producer of the general float engine: a 128-row tile is nsub 288-byte sub-tiles (36 KB each); the two query tiles of
-    // an item take 2 nsub of the six 36 KB buffers, the ring of train sub-tiles the remaining 6 - 2 nsub
-    const int nsub = a.nsub, ns = STAGES + 2 - 2 * nsub;
+  if (warp == 0) {
+    // producer: the whole (converged) warp walks the items, the elected lane issues the copies (tc_common.cuh: elect_one)
     uint32_t r = 0, ic = 0;
     for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
       const Item it = decode_item(a, a.items[w]);
       if (it.n_iter <= 0) continue;
       const uint8_t* gb = a.b_exp + ((size_t)it.seg * a.t_tiles_per_seg + it.tile_begin) * nsub * TILE_BYTES;
-      uint8_t* sB2 = smem + 2 * nsub * TILE_BYTES;
-      auto load_b = [&](int k) {                 // k-th sub-tile of this item
+      auto load_b = [&](int k) {                 // k-th train sub-tile of this item
         const uint32_t s = r % ns;
         mbar_wait(BAR(EMPTY + s), ((r / ns) & 1) ^ 1);
         if (elect_one()) {
           mbar_expect_tx(BAR(FULL + s), TILE_BYTES);
-          const uint32_t dst = smem_u32(sB2) + s * TILE_BYTES;
+          const uint32_t dst = smem_u32(sB) + s * TILE_BYTES;
 #pragma unroll
           for (int p = 0; p < 4; ++p)
             bulk_g2s(dst + p * (TILE_BYTES / 4), gb + (size_t)k * TILE_BYTES + (size_t)p * (TILE_BYTES / 4), TILE_BYTES / 4, BAR(FULL + s));
@@ -292,6 +313,8 @@ __global__ void __launch_bounds__(THREADS, 1) mma_kernel(Args a) {
         __syncwarp();
         ++r;
       };
+      // the first train tiles of this item go into the ring as soon as stages free up, i.e. while the previous item is still
+      // being multiplied; only then wait for the tensor core to be done with the previous item's query tiles and fetch ours
       const int n_sub = it.n_iter * nsub, pre = min(n_sub, ns);
       for (int k = 0; k < pre; ++k) load_b(k);
       mbar_wait(BAR(AEMPTY), (ic & 1) ^ 1);
@@ -304,88 +327,12 @@ __global__ void __launch_bounds__(THREADS, 1) mma_kernel(Args a) {
       ++ic;
       for (int k = pre; k < n_sub; ++k) load_b(k);
     }
-  } else if (KIND == KIND_L2F && (warp == 1 || warp == 3)) {
-    // MMA issuers of the general float engine.  Sub-tile j of a row holds [hi (64) | mid (64) | 16 more] bf16 of the values
-    // 64 j .. 64 j + 63; the products hi*hi, hi*mid and mid*hi of each 16-value block come from the same two tiles at
-    // different K offsets (descriptor + 16 per 256 bytes), and sub-tile 0 adds the |t|^2 columns: for dim = 64 that is
-    // 4 x 3 + 1 = 13 instructions per tile pair, for dim = 128 25, against the integer engine's 9.
-    const int qt = warp == 1 ? 0 : 1, nsub = a.nsub, ns = STAGES + 2 - 2 * nsub;
-    uint8_t* sB2 = smem + 2 * nsub * TILE_BYTES;
-    uint32_t t = 0, r = 0, ic = 0;
-    for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-      const Item it = decode_item(a, a.items[w]);
-      if (it.n_iter <= 0) continue;
-      mbar_wait(BAR(AFULL), ic & 1);
-      ++ic;
-      for (int k = 0; k < it.n_iter; ++k, ++t) {
-        const uint32_t b = t & 1;
-        mbar_wait(BAR(TEMPTY + b), ((t >> 1) & 1) ^ 1);
-        for (int j = 0; j < nsub; ++j, ++r) {
-          const uint32_t s = r % ns;
-          mbar_wait(BAR(FULL + s), (r / ns) & 1);
-          tc_fence_after();
-          const uint64_t da = smem_desc(smem_u32(sA) + (qt * nsub + j) * TILE_BYTES);
-          const uint64_t db = smem_desc(smem_u32(sB2) + s * TILE_BYTES);
-          const int nk = (min(64, a.dim - 64 * j) + 15) >> 4;
-          const uint32_t d = tmem + (b * 2 + qt) * TILE;
-          if (elect_one()) {
-            if (j == 0) tc_mma<KIND>(d, da + 128u, db + 128u, IDESC_L2, 0u);     // 1 x (-|t|^2 pieces)
-            for (int kk = 0; kk < nk; ++kk) {
-              tc_mma<KIND>(d, da + (uint64_t)(16 * kk), db + (uint64_t)(16 * kk), IDESC_L2, 1u);            // hi * hi
-              tc_mma<KIND>(d, da + (uint64_t)(16 * kk), db + (uint64_t)(16 * (4 + kk)), IDESC_L2, 1u);      // hi * mid
-              tc_mma<KIND>(d, da + (uint64_t)(16 * (4 + kk)), db + (uint64_t)(16 * kk), IDESC_L2, 1u);      // mid * hi
-            }
-            tc_commit(BAR(EMPTY + s));
-            if (j == nsub - 1) tc_commit(BAR(TFULL + b));
-          }
-          __syncwarp();
-        }
-      }
-      if (elect_one()) tc_commit(BAR(AEMPTY));
-      __syncwarp();
-    }
-  } else if (warp == 0) {
-    // producer: the whole (converged) warp walks the items, the elected lane issues the copies (tc_common.cuh: elect_one)
-    uint32_t t = 0, ic = 0;
-    for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
-      const Item it = decode_item(a, a.items[w]);
-      if (it.n_iter <= 0) continue;
-      const uint8_t* gb = a.b_exp + ((size_t)it.seg * a.t_tiles_per_seg + it.tile_begin) * TILE_BYTES;
-      auto load_b = [&](int k) {
-        const uint32_t s = t % STAGES;
-        mbar_wait(BAR(EMPTY + s), ((t / STAGES) & 1) ^ 1);
-        if (elect_one()) {
-          mbar_expect_tx(BAR(FULL + s), TILE_BYTES);
-          const uint32_t dst = smem_u32(sB) + s * TILE_BYTES;
-#pragma unroll
-          for (int p = 0; p < 4; ++p)
-            bulk_g2s(dst + p * (TILE_BYTES / 4), gb + (size_t)k * TILE_BYTES + (size_t)p * (TILE_BYTES / 4), TILE_BYTES / 4, BAR(FULL + s));
-        }
-        __syncwarp();
-        ++t;
-      };
-      // the first train tiles of this item go into the ring as soon as stages free up, i.e. while the previous item is still
-      // being multiplied; only then wait for the tensor core to be done with the previous item's query tiles and fetch ours
-      const int pre = min(it.n_iter, STAGES);
-      for (int k = 0; k < pre; ++k) load_b(k);
-      mbar_wait(BAR(AEMPTY), (ic & 1) ^ 1);
-      const uint8_t* ga = a.a_exp + ((size_t)it.seg * a.q_tiles_per_seg + (size_t)it.q_tile * 2) * TILE_BYTES;
-      if (elect_one()) {
-        mbar_expect_tx(BAR(AFULL), 2u * TILE_BYTES);
-#pragma unroll
-        for (int p = 0; p < 8; ++p) bulk_g2s(smem_u32(sA) + p * (TILE_BYTES / 4), ga + (size_t)p * (TILE_BYTES / 4), TILE_BYTES / 4, BAR(AFULL));
-      }
-      __syncwarp();
-      ++ic;
-      for (int k = pre; k < it.n_iter; ++k) load_b(k);
-    }
   } else if (warp == 1 || warp == 3) {
     // MMA issuers: converged warps, elected lane — issued from `if (lane == 0)` every tcgen05.mma was wrapped in an
     // elect / broadcast loop of ~13 instructions and the issuing thread, not the tensor pipe, set the pace.  Two of them (on
     // different sub-partitions), one per query tile = accumulator: the issue loop of a single warp sharing its scheduler
     // with busy epilogue warps was still slower than the tensor pipe (found on the score engine, score_mma.cuh).
     const int qt = warp == 1 ? 0 : 1;
-    const uint64_t da = smem_desc(smem_u32(sA) + qt * TILE_BYTES);
     uint32_t t = 0, ic = 0;
     for (int w = blockIdx.x; w < n_items; w += gridDim.x) {
       const Item it = decode_item(a, a.items[w]);
@@ -393,19 +340,24 @@ __global__ void __launch_bounds__(THREADS, 1) mma_kernel(Args a) {
       mbar_wait(BAR(AFULL), ic & 1);
       ++ic;
       for (int k = 0; k < it.n_iter; ++k, ++t) {
-        const uint32_t s = t % STAGES, b = t & 1;
+        // ring stage of the tile's first train sub-tile, taken before the accumulator wait.  In this form the issue loop of the
+        // nsub = 1 kinds compiles to the same instructions as a loop over one tile counter; deriving the stage after the wait
+        // compiled to a slightly different schedule that measured 13 % slower on long 1-NN Hamming items (B200, 1000 W).
+        const uint32_t r0 = t * nsub, s0 = r0 % ns, b = t & 1;
         mbar_wait(BAR(TEMPTY + b), ((t >> 1) & 1) ^ 1);    // the epilogue has drained this accumulator buffer
-        mbar_wait(BAR(FULL + s), (t / STAGES) & 1);        // the train tile has landed
-        tc_fence_after();
-        const uint64_t db = smem_desc(smem_u32(sB) + s * TILE_BYTES);
-        if (elect_one()) {
-#pragma unroll
-          for (int kk = 0; kk < KB / 32; ++kk)
-            tc_mma<KIND>(tmem + (b * 2 + qt) * TILE, da + (uint64_t)(16 * kk), db + (uint64_t)(16 * kk), KIND == KIND_L2 ? IDESC_L2 : IDESC, kk > 0);
-          tc_commit(BAR(EMPTY + s));    // shared-memory stage free once both warps' MMAs have read it
-          tc_commit(BAR(TFULL + b));    // this query tile's accumulator complete
+        for (int j = 0; j < nsub; ++j) {
+          const uint32_t r = r0 + j, s = j == 0 ? s0 : r % ns;
+          mbar_wait(BAR(FULL + s), (r / ns) & 1);          // the train sub-tile has landed
+          tc_fence_after();
+          const uint64_t da = smem_desc(smem_u32(sA) + (qt * nsub + j) * TILE_BYTES);
+          const uint64_t db = smem_desc(smem_u32(sB) + s * TILE_BYTES);
+          if (elect_one()) {
+            issue_tile_pair<KIND>(tmem + (b * 2 + qt) * TILE, da, db, j, a.dim);
+            tc_commit(BAR(EMPTY + s));                            // shared-memory stage free once both warps' MMAs have read it
+            if (j == nsub - 1) tc_commit(BAR(TFULL + b));         // this query tile's accumulator complete
+          }
+          __syncwarp();
         }
-        __syncwarp();
       }
       if (elect_one()) tc_commit(BAR(AEMPTY));         // every MMA of this item has read the query tiles
       __syncwarp();
@@ -808,43 +760,101 @@ l2f_redecide_kernel(const float* __restrict__ q, const float* __restrict__ t, in
 
 }  // namespace sos_hamming_mma
 
-// Host side, called by sos_hamming_top2 (hamming.cu).  `ws` holds the partial keys + work items (already planned);
-// `exp` is scratch for the expanded tiles.
-size_t sos_hamming_mma_scratch_bytes(int n_seg, int max_nq, int max_nt) {
+int sos_tc_match(sos_ctx* ctx, int kind, const void* q, const void* t, int dim, const int32_t* q_start, const int32_t* q_len,
+                 const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int32_t* idx0, void* d0,
+                 int32_t* idx1, void* d1, int32_t* flag, int32_t* stats) {
   using namespace sos_hamming_mma;
-  const size_t qt = (size_t)((max_nq + 255) / 256) * 2, tt = (size_t)((max_nt + TILE - 1) / TILE);
-  return (size_t)n_seg * (qt + tt) * TILE_BYTES + 256;
-}
+  const bool top2 = idx1 != nullptr || d1 != nullptr;
+  const int nsub = kind == KIND_L2F && dim > 64 ? 2 : 1;
+  const int q_items = sos_div_up(max_nq, ITEM_QROWS), qt = 2 * q_items, tt = sos_div_up(max_nt, TILE);
+  // a work item is 256 query rows x (train tiles / splits); keep >= 4 train tiles per item (the two query tiles of an
+  // item are fetched once per item) unless that starves the SMs
+  int splits = sos_div_up(2 * ctx->sm_count, q_items * n_seg);
+  if (splits > tt / 4) splits = tt / 4;
+  if (splits > (1 << ITEM_SPLIT_BITS)) splits = 1 << ITEM_SPLIT_BITS;
+  if (splits < 1) splits = 1;
+  const size_t max_items = (size_t)q_items * splits * n_seg;
+  SOS_CHECK_ARG(max_items < ((size_t)1 << 31), "too many work items");
 
-int sos_hamming_mma_launch(sos_ctx* ctx, const uint32_t* q, const uint32_t* t, const int32_t* q_start,
-                           const int32_t* q_len, const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq,
-                           int max_nt, int splits, const uint32_t* items, const int32_t* n_items, unsigned max_items,
-                           bool top2, void* exp, uint2* partial) {
-  using namespace sos_hamming_mma;
-  const int qt = ((max_nq + 255) / 256) * 2, tt = (max_nt + TILE - 1) / TILE;
-  uint8_t* a_exp = (uint8_t*)exp;
-  uint8_t* b_exp = a_exp + (size_t)n_seg * qt * TILE_BYTES;
-  if (qt > 0 || tt > 0) {
+  // Scratch, each piece 256-byte aligned: partial keys (per query row and split: uint2 Hamming, ulonglong2 L2, 2 x
+  // ulonglong2 L2F) | work items | their count | L2F: list of undecided queries | its count | |q|^2 per expanded query row
+  // (L2: int32, L2F: float64) | L2F: max |t|^2 per segment | expanded query tiles | expanded train tiles
+  const bool l2f = kind == KIND_L2F;
+  const size_t rows = (size_t)max_nq * n_seg, q_rows = (size_t)n_seg * qt * TILE;
+  const size_t key_bytes = kind == KIND_HAMMING ? sizeof(uint2) : kind == KIND_L2 ? sizeof(ulonglong2) : 2 * sizeof(ulonglong2);
+  const size_t piece[] = {rows * splits * key_bytes, max_items * sizeof(uint32_t), sizeof(int32_t),
+                          l2f ? rows * sizeof(int2) : 0, l2f ? sizeof(int32_t) : 0,
+                          kind == KIND_L2 ? q_rows * sizeof(int32_t) : l2f ? q_rows * sizeof(double) : 0,
+                          l2f ? n_seg * sizeof(double) : 0, (size_t)n_seg * qt * nsub * TILE_BYTES,
+                          (size_t)n_seg * tt * nsub * TILE_BYTES};
+  constexpr int N_PIECES = sizeof(piece) / sizeof(piece[0]);
+  size_t off[N_PIECES + 1] = {0};
+  for (int i = 0; i < N_PIECES; ++i) off[i + 1] = off[i] + sos_align_up(piece[i], 256);
+  char* ws = nullptr;
+  int rc = sos_arena_get(ctx, off[N_PIECES], (void**)&ws);
+  if (rc != SOS_OK) return rc;
+  void* partial = ws;
+  uint32_t* items = (uint32_t*)(ws + off[1]);
+  int32_t* n_items = (int32_t*)(ws + off[2]);
+  int2* list = (int2*)(ws + off[3]);
+  int32_t* list_n = (int32_t*)(ws + off[4]);
+  void* qnorm = ws + off[5];
+  double* tmax2 = (double*)(ws + off[6]);
+  uint8_t* a_exp = (uint8_t*)(ws + off[7]);
+  uint8_t* b_exp = (uint8_t*)(ws + off[8]);
+
+  hamming_plan_kernel<<<1, 256, 0, ctx->stream>>>(q_len, n_seg, max_nq, splits, items, n_items);
+  SOS_LAUNCHED_AS(ctx, "hamming_plan_kernel");
+  if (kind == KIND_HAMMING) {
     ExpandArgs e;
-    e.desc[0] = q; e.desc[1] = t; e.start[0] = q_start; e.start[1] = t_start; e.len[0] = q_len; e.len[1] = t_len;
-    e.max_rows[0] = max_nq; e.max_rows[1] = max_nt; e.tiles_per_seg[0] = qt; e.tiles_per_seg[1] = tt;
-    e.out[0] = a_exp; e.out[1] = b_exp;
+    e.desc[0] = (const uint32_t*)q; e.desc[1] = (const uint32_t*)t; e.start[0] = q_start; e.start[1] = t_start;
+    e.len[0] = q_len; e.len[1] = t_len; e.max_rows[0] = max_nq; e.max_rows[1] = max_nt; e.tiles_per_seg[0] = qt;
+    e.tiles_per_seg[1] = tt; e.out[0] = a_exp; e.out[1] = b_exp;
     expand_kernel<<<dim3(qt > tt ? qt : tt, n_seg, 2), 256, 0, ctx->stream>>>(e);
     SOS_LAUNCHED_AS(ctx, "hamming_expand_kernel");
+  } else if (kind == KIND_L2) {
+    expand_l2_kernel<<<dim3(qt, n_seg), 256, 0, ctx->stream>>>((const float*)q, dim, q_start, q_len, max_nq, qt, 0, a_exp,
+                                                               (int32_t*)qnorm, flag);
+    SOS_LAUNCHED_AS(ctx, "l2_expand_kernel");
+    if (tt > 0) {
+      expand_l2_kernel<<<dim3(tt, n_seg), 256, 0, ctx->stream>>>((const float*)t, dim, t_start, t_len, max_nt, tt, 1, b_exp,
+                                                                 nullptr, flag);
+      SOS_LAUNCHED_AS(ctx, "l2_expand_kernel");
+    }
+  } else {
+    SOS_CUDA(cudaMemsetAsync(list_n, 0, sizeof(int32_t), ctx->stream));
+    SOS_CUDA(cudaMemsetAsync(tmax2, 0, (size_t)n_seg * sizeof(double), ctx->stream));
+    if (stats) SOS_CUDA(cudaMemsetAsync(stats, 0, SOS_L2F_STATS * sizeof(int32_t), ctx->stream));
+    l2f_expand_kernel<<<dim3(qt, n_seg), 256, 0, ctx->stream>>>((const float*)q, dim, q_start, q_len, max_nq, qt, nsub, 0,
+                                                                a_exp, (double*)qnorm, flag);
+    SOS_LAUNCHED_AS(ctx, "l2f_expand_kernel");
+    if (tt > 0) {
+      l2f_expand_kernel<<<dim3(tt, n_seg), 256, 0, ctx->stream>>>((const float*)t, dim, t_start, t_len, max_nt, tt, nsub, 1,
+                                                                  b_exp, tmax2, flag);
+      SOS_LAUNCHED_AS(ctx, "l2f_expand_kernel");
+    }
   }
+
   Args a;
+  a.a_norm = kind == KIND_L2 ? (const int32_t*)qnorm : nullptr;
   a.a_exp = a_exp; a.b_exp = b_exp; a.q_len = q_len; a.t_len = t_len;
   a.max_nq = max_nq; a.max_nt = max_nt; a.splits = splits; a.q_tiles_per_seg = qt; a.t_tiles_per_seg = tt;
   a.items = items; a.n_items = n_items; a.partial = partial;
-  a.a_norm = nullptr;
-  // ring depth 4 (221 KB of shared memory); 3 stages measured the same (profiles/r02/score_variants_and_ring_depth_ab.log)
+  a.dim = dim; a.nsub = nsub;
+  // ring depth 4 (221 KB of shared memory); 3 stages measured the same (profiles/r02/score_variants_and_ring_depth_ab.log).
+  // L2F: the six 36 KB buffers are 2 nsub query sub-tiles and a ring of 4 (dim <= 64) or 2 (dim <= 128) train sub-tiles.
   constexpr int ST = 4;
-  static bool attr_set[64][2] = {};     // per device: the opt-in to > 48 KB of dynamic shared memory
-  const int dev = ctx->device & 63, v = top2 ? 1 : 0;
-  if (!attr_set[dev][v]) {
-    if (top2) SOS_CUDA(cudaFuncSetAttribute(mma_kernel<true, ST, KIND_HAMMING>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
-    else SOS_CUDA(cudaFuncSetAttribute(mma_kernel<false, ST, KIND_HAMMING>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
-    attr_set[dev][v] = true;
+  using Kernel = void (*)(Args);
+  static const Kernel kernels[3][2] = {{mma_kernel<false, ST, KIND_HAMMING>, mma_kernel<true, ST, KIND_HAMMING>},
+                                       {mma_kernel<false, ST, KIND_L2>, mma_kernel<true, ST, KIND_L2>},
+                                       {mma_kernel<false, ST, KIND_L2F>, mma_kernel<true, ST, KIND_L2F>}};
+  static const char* const names[3] = {"hamming_mma_kernel", "l2_mma_kernel", "l2f_mma_kernel"};
+  static bool smem_opt_in[64][3][2] = {};   // per device: the opt-in to > 48 KB of dynamic shared memory
+  const Kernel kernel = kernels[kind][top2];
+  bool& opted_in = smem_opt_in[ctx->device & 63][kind][top2];
+  if (!opted_in) {
+    SOS_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
+    opted_in = true;
   }
   // One kernel, two launch shapes.  Short items (stereo buckets: a handful of train tiles each) run PERSISTENT — one CTA per
   // SM walks the work list, so barriers, tensor memory and the pipelines survive from item to item (measured: 0.083 ->
@@ -852,124 +862,30 @@ int sos_hamming_mma_launch(sos_ctx* ctx, const uint32_t* q, const uint32_t* t, c
   // the balancing to the hardware scheduler: the fixed striding of the persistent shape loses more to unequal SMs than the
   // per-item set-up costs (0.285 vs 0.300 ms; profiles/r02/hamming_ab_persistent.log).
   const bool persistent = max_nt <= 2048;
-  const unsigned grid = (persistent && max_items > (unsigned)ctx->sm_count) ? (unsigned)ctx->sm_count : max_items;
-  if (top2) mma_kernel<true, ST, KIND_HAMMING><<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
-  else mma_kernel<false, ST, KIND_HAMMING><<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
-  SOS_LAUNCHED_AS(ctx, "hamming_mma_kernel");
-  return SOS_OK;
-}
+  const unsigned grid = (persistent && max_items > (size_t)ctx->sm_count) ? (unsigned)ctx->sm_count : (unsigned)max_items;
+  kernel<<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
+  SOS_LAUNCHED_AS(ctx, names[kind]);
 
-// The float-descriptor L2 engine (sos_l2_top2 in hamming.cu).  `exp` = expanded tiles followed by the query norms.
-size_t sos_l2_mma_scratch_bytes(int n_seg, int max_nq, int max_nt) {
-  using namespace sos_hamming_mma;
-  const size_t qt = (size_t)((max_nq + 255) / 256) * 2;
-  return sos_hamming_mma_scratch_bytes(n_seg, max_nq, max_nt) + (size_t)n_seg * qt * TILE * sizeof(int32_t) + 256;
-}
-
-int sos_l2_mma_launch(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start, const int32_t* q_len,
-                      const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int splits,
-                      const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* exp,
-                      ulonglong2* partial, int32_t* flag) {
-  using namespace sos_hamming_mma;
-  const int qt = ((max_nq + 255) / 256) * 2, tt = (max_nt + TILE - 1) / TILE;
-  uint8_t* a_exp = (uint8_t*)exp;
-  uint8_t* b_exp = a_exp + (size_t)n_seg * qt * TILE_BYTES;
-  int32_t* norms = (int32_t*)(b_exp + sos_align_up((size_t)n_seg * tt * TILE_BYTES, 256));
-  if (qt > 0) {
-    expand_l2_kernel<<<dim3(qt, n_seg), 256, 0, ctx->stream>>>(q, dim, q_start, q_len, max_nq, qt, 0, a_exp, norms, flag);
-    SOS_LAUNCHED_AS(ctx, "l2_expand_kernel");
+  const dim3 mgrid(sos_div_up(max_nq, 256), n_seg);
+  if (kind == KIND_HAMMING) {
+    merge_kernel<<<mgrid, 256, 0, ctx->stream>>>((const uint2*)partial, q_start, q_len, max_nq, splits, idx0, (int32_t*)d0,
+                                                 idx1, (int32_t*)d1);
+    SOS_LAUNCHED_AS(ctx, "hamming_merge_kernel");
+  } else if (kind == KIND_L2) {
+    merge_kernel<<<mgrid, 256, 0, ctx->stream>>>((const ulonglong2*)partial, q_start, q_len, max_nq, splits, idx0, (float*)d0,
+                                                 idx1, (float*)d1);
+    SOS_LAUNCHED_AS(ctx, "l2_merge_kernel");
+  } else {
+    l2f_decide_kernel<<<mgrid, 256, 0, ctx->stream>>>((const ulonglong2*)partial, (const float*)q, (const float*)t, dim, q_start,
+                                                      q_len, t_start, t_len, max_nq, max_nt, splits, qt * TILE,
+                                                      (const double*)qnorm, tmax2, idx0, (float*)d0, idx1, (float*)d1, list,
+                                                      list_n, stats);
+    SOS_LAUNCHED_AS(ctx, "l2f_decide_kernel");
+    const size_t rd_grid = rows < (size_t)(8 * ctx->sm_count) ? rows : (size_t)(8 * ctx->sm_count);
+    l2f_redecide_kernel<<<(unsigned)rd_grid, RD_THREADS, 0, ctx->stream>>>((const float*)q, (const float*)t, dim, q_start,
+                                                                          t_start, t_len, max_nt, list, list_n, idx0,
+                                                                          (float*)d0, idx1, (float*)d1, stats);
+    SOS_LAUNCHED_AS(ctx, "l2f_redecide_kernel");
   }
-  if (tt > 0) {
-    expand_l2_kernel<<<dim3(tt, n_seg), 256, 0, ctx->stream>>>(t, dim, t_start, t_len, max_nt, tt, 1, b_exp, nullptr, flag);
-    SOS_LAUNCHED_AS(ctx, "l2_expand_kernel");
-  }
-  Args a;
-  a.a_norm = norms;
-  a.a_exp = a_exp; a.b_exp = b_exp; a.q_len = q_len; a.t_len = t_len;
-  a.max_nq = max_nq; a.max_nt = max_nt; a.splits = splits; a.q_tiles_per_seg = qt; a.t_tiles_per_seg = tt;
-  a.items = items; a.n_items = n_items; a.partial = partial;
-  constexpr int ST = 4;
-  static bool attr_set[64][2] = {};
-  const int dev = ctx->device & 63, v = top2 ? 1 : 0;
-  if (!attr_set[dev][v]) {
-    if (top2) SOS_CUDA(cudaFuncSetAttribute(mma_kernel<true, ST, KIND_L2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
-    else SOS_CUDA(cudaFuncSetAttribute(mma_kernel<false, ST, KIND_L2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
-    attr_set[dev][v] = true;
-  }
-  const bool persistent = max_nt <= 2048;
-  const unsigned grid = (persistent && max_items > (unsigned)ctx->sm_count) ? (unsigned)ctx->sm_count : max_items;
-  if (top2) mma_kernel<true, ST, KIND_L2><<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
-  else mma_kernel<false, ST, KIND_L2><<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
-  SOS_LAUNCHED_AS(ctx, "l2_mma_kernel");
-  return SOS_OK;
-}
-
-// The general float-descriptor L2 engine (sos_l2f_top2 in hamming.cu): expansion, GEMM, decision and float64 re-decision.
-// Scratch: partial keys (2 x ulonglong2 per query row and split) | list of undecided queries | its count | |q|^2 per expanded
-// query row | max |t|^2 per segment | expanded query tiles | expanded train tiles.
-static size_t l2f_align(size_t b) { return sos_align_up(b, 256); }
-size_t sos_l2f_scratch_bytes(int n_seg, int max_nq, int max_nt, int dim, int splits) {
-  using namespace sos_hamming_mma;
-  const size_t qt = (size_t)((max_nq + 255) / 256) * 2, tt = (size_t)((max_nt + TILE - 1) / TILE), nsub = dim > 64 ? 2 : 1;
-  const size_t rows = (size_t)max_nq * n_seg;
-  return l2f_align(rows * splits * 2 * sizeof(ulonglong2)) + l2f_align(rows * sizeof(int2)) + 256 +
-         l2f_align((size_t)n_seg * qt * TILE * sizeof(double)) + l2f_align((size_t)n_seg * sizeof(double)) +
-         (size_t)n_seg * (qt + tt) * nsub * TILE_BYTES;
-}
-
-int sos_l2f_launch(sos_ctx* ctx, const float* q, const float* t, int dim, const int32_t* q_start, const int32_t* q_len,
-                   const int32_t* t_start, const int32_t* t_len, int n_seg, int max_nq, int max_nt, int splits,
-                   const uint32_t* items, const int32_t* n_items, unsigned max_items, bool top2, void* scratch,
-                   int32_t* idx0, float* d0, int32_t* idx1, float* d1, int32_t* flag, int32_t* stats) {
-  using namespace sos_hamming_mma;
-  const int qt = ((max_nq + 255) / 256) * 2, tt = (max_nt + TILE - 1) / TILE, nsub = dim > 64 ? 2 : 1;
-  const size_t rows = (size_t)max_nq * n_seg;
-  char* p = (char*)scratch;
-  ulonglong2* partial = (ulonglong2*)p;            p += l2f_align(rows * splits * 2 * sizeof(ulonglong2));
-  int2* list = (int2*)p;                           p += l2f_align(rows * sizeof(int2));
-  int32_t* list_n = (int32_t*)p;                   p += 256;
-  double* qnorm2 = (double*)p;                     p += l2f_align((size_t)n_seg * qt * TILE * sizeof(double));
-  double* tmax2 = (double*)p;                      p += l2f_align((size_t)n_seg * sizeof(double));
-  uint8_t* a_exp = (uint8_t*)p;
-  uint8_t* b_exp = a_exp + (size_t)n_seg * qt * nsub * TILE_BYTES;
-  SOS_CUDA(cudaMemsetAsync(list_n, 0, sizeof(int32_t), ctx->stream));
-  SOS_CUDA(cudaMemsetAsync(tmax2, 0, (size_t)n_seg * sizeof(double), ctx->stream));
-  if (stats) SOS_CUDA(cudaMemsetAsync(stats, 0, SOS_L2F_STATS * sizeof(int32_t), ctx->stream));
-  if (qt > 0) {
-    l2f_expand_kernel<<<dim3(qt, n_seg), 256, 0, ctx->stream>>>(q, dim, q_start, q_len, max_nq, qt, nsub, 0, a_exp, qnorm2, flag);
-    SOS_LAUNCHED_AS(ctx, "l2f_expand_kernel");
-  }
-  if (tt > 0) {
-    l2f_expand_kernel<<<dim3(tt, n_seg), 256, 0, ctx->stream>>>(t, dim, t_start, t_len, max_nt, tt, nsub, 1, b_exp, tmax2, flag);
-    SOS_LAUNCHED_AS(ctx, "l2f_expand_kernel");
-  }
-  Args a;
-  a.a_norm = nullptr;
-  a.dim = dim; a.nsub = nsub;
-  a.a_exp = a_exp; a.b_exp = b_exp; a.q_len = q_len; a.t_len = t_len;
-  a.max_nq = max_nq; a.max_nt = max_nt; a.splits = splits; a.q_tiles_per_seg = qt; a.t_tiles_per_seg = tt;
-  a.items = items; a.n_items = n_items; a.partial = partial;
-  // six 36 KB buffers: 2 nsub for the query tiles, the rest a ring of train sub-tiles (4 for dim <= 64, 2 above)
-  constexpr int ST = 4;
-  static bool attr_set[64][2] = {};
-  const int dev = ctx->device & 63, v = top2 ? 1 : 0;
-  if (!attr_set[dev][v]) {
-    if (top2) SOS_CUDA(cudaFuncSetAttribute(mma_kernel<true, ST, KIND_L2F>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
-    else SOS_CUDA(cudaFuncSetAttribute(mma_kernel<false, ST, KIND_L2F>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(ST)));
-    attr_set[dev][v] = true;
-  }
-  const bool persistent = max_nt <= 2048;
-  const unsigned grid = (persistent && max_items > (unsigned)ctx->sm_count) ? (unsigned)ctx->sm_count : max_items;
-  if (top2) mma_kernel<true, ST, KIND_L2F><<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
-  else mma_kernel<false, ST, KIND_L2F><<<grid, THREADS, smem_bytes(ST), ctx->stream>>>(a);
-  SOS_LAUNCHED_AS(ctx, "l2f_mma_kernel");
-  dim3 mgrid((max_nq + 255) / 256, n_seg);
-  l2f_decide_kernel<<<mgrid, 256, 0, ctx->stream>>>(partial, q, t, dim, q_start, q_len, t_start, t_len, max_nq, max_nt, splits,
-                                                    qt * TILE, qnorm2, tmax2, idx0, d0, idx1, d1, list, list_n, stats);
-  SOS_LAUNCHED_AS(ctx, "l2f_decide_kernel");
-  const size_t rd_grid = rows < (size_t)(8 * ctx->sm_count) ? rows : (size_t)(8 * ctx->sm_count);
-  l2f_redecide_kernel<<<(unsigned)rd_grid, RD_THREADS, 0, ctx->stream>>>(q, t, dim, q_start, t_start, t_len, max_nt, list,
-                                                                        list_n, idx0, d0, idx1, d1, stats);
-  SOS_LAUNCHED_AS(ctx, "l2f_redecide_kernel");
   return SOS_OK;
 }
