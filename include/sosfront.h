@@ -471,7 +471,8 @@ int sos_refine_pose(sos_ctx* ctx, const float* p_ref, const float* f_cur, const 
 /* One step chains the five hot-path steps for a batch of frames exactly as
  * StereoPanoramicFrame.establish_stereo_correspondences (pose_est_tools.py:320-402) and
  * TrackerStereoSE3.track_frame (pose_est_tools.py:736-847) do for one frame; defaults in pose_est_tools.py:284-308,
- * 672-707, 862-878.  Feature detection is upstream of the hot path (SURVEY §2 row 5): features arrive as input. */
+ * 672-707, 862-878.  sos_frontend_step takes the features as input (feature detection is upstream of the hot path in
+ * the reference, SURVEY §2 row 5); sos_frontend_step_images detects them itself from the omni images (see below). */
 /* sos_frontend_config.refit */
 enum {
   SOS_REFINE_NONE = 0, /* pose = RANSAC model */
@@ -586,6 +587,43 @@ int sos_frontend_host_bytes(sos_frontend* fe, int64_t* h2d_bytes_per_step, int64
 int sos_frontend_step_host(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
                            const int32_t* bucket_off_top, const float* px_bot, const uint32_t* desc_bot,
                            const int32_t* bucket_off_bot, float* poses, int32_t* stats);
+
+/* Images-in steps: the front-end detects the features itself, on the step's own panoramas, with the reference's default
+ * detector (StereoPanoramicFrame -> OmniCamModel.detect_sparse_features_on_panorama, camera_models.py:1610-1797, "GFT"):
+ * 11 x 11 median, BGR2GRAY, goodFeaturesToTrack per azimuthal mask and view, ORB description, then the bucketed feature
+ * layout of sos_frontend_step — the same calls as sos_median_blur_11, sos_bgr_to_gray, sos_gft_detect and
+ * sos_orb_describe, bit for bit, inside the step (and its CUDA graph) with nothing read back to the host. */
+typedef struct sos_detect_config {
+  int32_t corners_per_bucket; /* maxCorners of goodFeaturesToTrack per azimuthal mask, 1..max_feat_per_bucket */
+  int32_t median;             /* 1: 11x11 median before BGR2GRAY (median_win_size = 11, pose_est_tools.py:297); 0: none */
+  double quality_level;       /* 0.01 */
+  double min_distance;        /* 5 */
+} sos_detect_config;
+
+/* Device arrays of the features the last images-in step detected (owned by the front-end). */
+typedef struct sos_frontend_features {
+  float* px_top;            /* [batch, max_feat_per_view, 2]: per frame, bucket by bucket, strongest corner first; zero rows */
+  uint32_t* desc_top;       /* [batch, max_feat_per_view, 8]   past the last feature                                       */
+  int32_t* boff_top;        /* [batch, n_buckets+1], clamped to max_feat_per_view                                          */
+  float* px_bot;
+  uint32_t* desc_bot;
+  int32_t* boff_bot;
+  int32_t* detect_stats;    /* [batch, 2 (top, bottom), 4]: corners accepted by the selection, corners ORB kept (border
+                               rule), rows dropped by the max_feat_per_view clamp, masks refused for more than 16384
+                               candidates (they contribute no corners to that frame and view) */
+} sos_frontend_features;
+
+/* masks_top / masks_bot: DEVICE uint8 [n_buckets, pano_rows, pano_cols], read by this call only (packed into bits here).
+ * Needs channels == 3 and n_buckets <= 32 (else SOS_ERR_UNSUPPORTED).  May be called again to change masks or parameters. */
+int sos_frontend_set_detector(sos_frontend* fe, const sos_detect_config* dcfg, const uint8_t* masks_top,
+                              const uint8_t* masks_bot);
+/* One step from DEVICE omni [batch, src_h, src_w, 3] alone (asynchronous; after the first call with a given omni pointer a
+ * captured graph is replayed and the host never waits).  SOS_ERR_INVALID without a detector. */
+int sos_frontend_step_images(sos_frontend* fe, const uint8_t* omni);
+/* The same from HOST omni (pinned for full copy bandwidth): only the LUT-reachable bands are uploaded, no feature arrays;
+ * then sos_frontend_wait_host. */
+int sos_frontend_submit_host_images(sos_frontend* fe, const uint8_t* omni, int* ticket);
+int sos_frontend_get_features(sos_frontend* fe, sos_frontend_features* out);
 
 /* ------------------------------------------------------------------------------------------------
  * Roofline denominators measured in-process (integer POPC pipe, FP32 FMA pipe) — bench.py only.

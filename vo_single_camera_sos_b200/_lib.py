@@ -86,6 +86,10 @@ PROTOTYPES = {
     "sos_frontend_wait_host": (I, [C.c_void_p, I, P, P]),
     "sos_frontend_host_bytes": (I, [C.c_void_p, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "sos_frontend_step_host": (I, [C.c_void_p, P, P, P, P, P, P, P, P, P]),
+    "sos_frontend_set_detector": (I, [C.c_void_p, P, P, P]),
+    "sos_frontend_step_images": (I, [C.c_void_p, P]),
+    "sos_frontend_submit_host_images": (I, [C.c_void_p, P, C.POINTER(I)]),
+    "sos_frontend_get_features": (I, [C.c_void_p, P]),
     "sos_peak_popc": (I, [c_ctx, C.POINTER(D)]),
     "sos_peak_ffma": (I, [c_ctx, C.POINTER(D)]),
     "sos_peak_dfma": (I, [c_ctx, C.POINTER(D)]),

@@ -173,6 +173,84 @@ __global__ void stats_kernel(const int32_t* __restrict__ n, const int32_t* __res
   stats[4 * i + 3] = best_hyp[i];
 }
 
+// Images-in step: the corners of one (frame, view) -> the bucketed feature rows sos_frontend_step reads, as
+// FeatureFront.detect (features.py) builds them.  One block per (frame, view); the nb * N slots (bucket-major, strongest
+// first) are scanned in tiles of the block: slot j of bucket k is kept iff j < count[k] and ORB kept it (border rule); kept
+// slot number p becomes feature row p if p < F.  Bucket offsets are the prefix sums of kept slots clamped to F; rows past
+// the last are zeroed.  A bucket whose selection refused its candidate list (count < 0) contributes nothing.
+// stats [B, 2, 4]: corners accepted, corners kept by ORB, rows dropped by the F clamp, refused masks.
+constexpr int DP_THREADS = 1024;
+
+__global__ void __launch_bounds__(DP_THREADS)
+detect_pack_kernel(const float2* __restrict__ xy, const int32_t* __restrict__ count, const uint8_t* __restrict__ keep,
+                   const uint4* __restrict__ desc, int B, int nb, int N, int F, float2* __restrict__ px_top,
+                   uint4* __restrict__ desc_top, int32_t* __restrict__ boff_top, float2* __restrict__ px_bot,
+                   uint4* __restrict__ desc_bot, int32_t* __restrict__ boff_bot, int32_t* __restrict__ stats) {
+  __shared__ int s_warp[DP_THREADS / 32];
+  __shared__ int s_bucket[32];
+  const int b = blockIdx.x, view = blockIdx.y;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const size_t list0 = ((size_t)view * B + b) * nb;               // xy / count / keep / desc are [2, B, nb, N, ...]
+  float2* px = (view == 0 ? px_top : px_bot) + (size_t)b * F;
+  uint4* ds = (view == 0 ? desc_top : desc_bot) + (size_t)b * F * 2;
+  int32_t* boff = (view == 0 ? boff_top : boff_bot) + (size_t)b * (nb + 1);
+  if (threadIdx.x < 32) s_bucket[threadIdx.x] = 0;
+  __syncthreads();
+  const int total_slots = nb * N;
+  int base = 0;
+  for (int i0 = 0; i0 < total_slots; i0 += DP_THREADS) {
+    const int i = i0 + threadIdx.x;
+    bool kept = false;
+    int k = 0;
+    if (i < total_slots) {
+      k = i / N;
+      kept = (i - k * N) < count[list0 + k] && keep[list0 * N + i] != 0;
+    }
+    const unsigned vote = __ballot_sync(0xFFFFFFFFu, kept);
+    if (lane == 0) s_warp[warp] = __popc(vote);
+    __syncthreads();
+    int before = 0, tile = 0;
+    for (int w = 0; w < DP_THREADS / 32; ++w) {
+      const int c = s_warp[w];
+      if (w < warp) before += c;
+      tile += c;
+    }
+    if (kept) {
+      atomicAdd(&s_bucket[k], 1);
+      const int pos = base + before + __popc(vote & ((1u << lane) - 1u));
+      if (pos < F) {
+        px[pos] = xy[list0 * N + i];
+        const uint4* src = desc + (list0 * N + i) * 2;
+        ds[2 * pos] = src[0];
+        ds[2 * pos + 1] = src[1];
+      }
+    }
+    base += tile;
+    __syncthreads();
+  }
+  for (int r = base + threadIdx.x; r < F; r += DP_THREADS) {
+    px[r] = make_float2(0.f, 0.f);
+    ds[2 * r] = make_uint4(0u, 0u, 0u, 0u);
+    ds[2 * r + 1] = make_uint4(0u, 0u, 0u, 0u);
+  }
+  if (threadIdx.x == 0) {
+    int acc = 0, accepted = 0, refused = 0;
+    boff[0] = 0;
+    for (int k = 0; k < nb; ++k) {
+      const int c = count[list0 + k];
+      accepted += max(c, 0);
+      refused += c < 0;
+      acc += s_bucket[k];
+      boff[k + 1] = min(acc, F);
+    }
+    int32_t* st = stats + ((size_t)b * 2 + view) * 4;
+    st[0] = accepted;
+    st[1] = base;
+    st[2] = max(0, base - F);
+    st[3] = refused;
+  }
+}
+
 }  // namespace
 
 struct sos_frontend {
@@ -213,13 +291,39 @@ struct sos_frontend {
   // graph cache keyed on the input pointers
   struct GraphKey {
     const void* p[7];
+    intptr_t images;   // 1: images-in step (its feature pointers are the front-end's own buffers)
   };
   struct GraphEntry {
     GraphKey key;
     cudaGraphExec_t exec = nullptr;
+    int launches = 0;
+    const void* arena = nullptr;   // fe->ctx->arena at capture
   };
   std::vector<GraphEntry> graphs;
   bool use_graph = true;
+  // images-in step (sos_frontend_set_detector): front-end-owned buffers, allocated by the first set_detector
+  struct Detector {
+    bool on = false;
+    sos_detect_config cfg;
+    int32_t overlap[2] = {0, 0};         // masks of the view share pixels (read back once, when they are packed)
+    uint8_t *med = nullptr, *gray = nullptr;   // [B, 2, rows, cols, 3] median output, [B, 2, rows, cols] gray
+    uint8_t* blur = nullptr;             // [B, 2, rows, cols] ORB's blurred gray (in the arena it could regrow
+                                         // the arena that the feature steps' graphs hold)
+    uint32_t* mask_bits[2] = {nullptr, nullptr};
+    int32_t* flags = nullptr;            // [2] overlap flags of the mask packing
+    // GFT scratch, shared by the two views (they run one after the other)
+    float* eig = nullptr;                // [B, rows, cols]
+    uint32_t* max_bits = nullptr;        // [B * nb]
+    int32_t* cand = nullptr;             // [B * nb] candidates per list
+    unsigned long long* keys = nullptr;  // [B * nb * SOS_GFT_CAP]
+    int32_t* rank = nullptr;             // [B, rows, cols], all -1: cleared once, the selection leaves it so
+    float* xy = nullptr;                 // [2, B, nb, N, 2]  corners, N = corners_per_bucket
+    int32_t* count = nullptr;            // [2, B, nb]
+    int32_t* kp_image = nullptr;         // [2, B, nb, N] image of each corner in gray (2 b + view)
+    uint32_t* kp_desc = nullptr;         // [2, B, nb, N, 8]
+    uint8_t* kp_keep = nullptr;          // [2, B, nb, N]
+    sos_frontend_features f;             // packed features + detect_stats
+  } det;
 };
 
 namespace {
@@ -239,9 +343,60 @@ int fe_alloc(sos_frontend* fe, T** out, size_t count) {
   return SOS_OK;
 }
 
+// Images-in step, ahead of stage A: remap, then the feature front of FeatureFront.detect (features.py) on the panoramas —
+// 11 x 11 median and BGR2GRAY over both views at once, Shi-Tomasi per view, ORB description over both views — and
+// detect_pack_kernel into the feature arrays stage A reads.  Nothing is read back: a candidate list over the selection's
+// capacity yields no corners (counted in detect_stats) instead of failing the step.
+int enqueue_detect(sos_frontend* fe, const uint8_t* omni) {
+  sos_ctx* ctx = fe->ctx;
+  const sos_frontend_config& c = fe->cfg;
+  sos_frontend::Detector& dt = fe->det;
+  const int B = c.batch, nb = c.n_buckets, N = dt.cfg.corners_per_bucket, H = c.pano_rows, W = c.pano_cols;
+  int rc = sos_remap_u8(ctx, omni, B, c.src_h, c.src_w, c.channels, fe->lut, 2, H, W, c.border, c.background, fe->d.pano);
+  if (rc) return rc;
+  const uint8_t* bgr = fe->d.pano;
+  if (dt.cfg.median) {
+    rc = sos_median_blur_11(ctx, fe->d.pano, 2 * B, H, W, 3, dt.med);
+    if (rc) return rc;
+    bgr = dt.med;
+  }
+  rc = sos_bgr_to_gray(ctx, bgr, (size_t)2 * B * H * W, dt.gray);
+  if (rc) return rc;
+  const size_t plane = (size_t)H * W;
+  for (int view = 0; view < 2; ++view) {
+    sos_gft_work w;
+    w.mask_bits = dt.mask_bits[view];
+    w.eig = dt.eig;
+    w.max_bits = dt.max_bits;
+    w.counts = dt.cand;
+    w.keys = dt.keys;
+    w.rank_img = dt.rank;
+    float* xy = dt.xy + (size_t)view * B * nb * N * 2;
+    int32_t* count = dt.count + (size_t)view * B * nb;
+    // the gray image of view v of frame b is plane 2 b + v
+    rc = sos_gft_candidates(ctx, w, dt.gray + view * plane, 2 * plane, B, H, W, nb, dt.cfg.quality_level);
+    // the counts are not known here: every block gets the shared memory of a full list (62 registers x 1024 threads leave
+    // room for one block per SM whatever the shared memory, so smaller lists would not share an SM anyway)
+    if (!rc) rc = sos_gft_select(ctx, w, B, H, W, nb, N, dt.cfg.min_distance, dt.overlap[view] != 0, SOS_GFT_CAP, xy, count);
+    if (rc) return rc;
+  }
+  rc = sos_orb_describe_into(ctx, dt.gray, 2 * B, H, W, dt.xy, nullptr, dt.kp_image, 2 * B * nb * N, dt.kp_desc, dt.kp_keep,
+                             dt.blur);
+  if (rc) return rc;
+  const sos_frontend_features& f = dt.f;
+  detect_pack_kernel<<<dim3(B, 2), DP_THREADS, 0, ctx->stream>>>((const float2*)dt.xy, dt.count, dt.kp_keep,
+                                                                 (const uint4*)dt.kp_desc, B, nb, N, c.max_feat_per_view,
+                                                                 (float2*)f.px_top, (uint4*)f.desc_top, f.boff_top,
+                                                                 (float2*)f.px_bot, (uint4*)f.desc_bot, f.boff_bot,
+                                                                 f.detect_stats);
+  SOS_LAUNCHED_AS(ctx, "detect_pack_kernel");
+  return SOS_OK;
+}
+
 // Stage A of a step (remap, stereo matching, lifting + triangulation into store slots 1..B), enqueued on ctx->stream.
+// images: the panoramas were already made by enqueue_detect.
 int enqueue_stage_a(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
-                 const int32_t* boff_top, const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot) {
+                 const int32_t* boff_top, const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot, bool images) {
   sos_ctx* ctx = fe->ctx;
   const sos_frontend_config& c = fe->cfg;
   sos_frontend_buffers& d = fe->d;
@@ -249,8 +404,9 @@ int enqueue_stage_a(sos_frontend* fe, const uint8_t* omni, const float* px_top, 
   int rc;
   // step 1, as a parallel branch (fork here, join at the end of the step).  Round 1 measured no gain from this — then the
   // chain was three long kernels that filled the GPU; now a fifth of the step is small launches that leave most SMs idle.
-  // Per-kernel profiling runs keep it in line so that every kernel is timed alone.
-  fe->remap_forked = fe->remap_stream != nullptr && !ctx->prof;
+  // Per-kernel profiling runs keep it in line so that every kernel is timed alone.  In an images-in step the remap feeds
+  // the detection and has already run.
+  fe->remap_forked = fe->remap_stream != nullptr && !ctx->prof && !images;
   if (fe->remap_forked) {
     SOS_CUDA(cudaEventRecord(fe->ev_fork, ctx->stream));
     SOS_CUDA(cudaStreamWaitEvent(fe->remap_stream, fe->ev_fork, 0));
@@ -261,7 +417,7 @@ int enqueue_stage_a(sos_frontend* fe, const uint8_t* omni, const float* px_top, 
     ctx->stream = main_stream;
     if (rc) return rc;
     SOS_CUDA(cudaEventRecord(fe->ev_join, fe->remap_stream));
-  } else {
+  } else if (!images) {
     rc = sos_remap_u8(ctx, omni, B, c.src_h, c.src_w, c.channels, fe->lut, 2, c.pano_rows, c.pano_cols, c.border,
                       c.background, d.pano);
     if (rc) return rc;
@@ -352,9 +508,11 @@ int enqueue_carry(sos_frontend* fe, int from) {
 
 // The kernel chain of one step.  Consecutive mode ends by carrying the last frame over as the reference of the next
 // step (slot B -> slot 0, one kernel instead of 8 copy nodes); in keyframe mode the caller promotes a slot itself.
+// images: the features are detected on the step's panoramas first (the px / desc / boff pointers are fe->det.f's).
 int enqueue_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
-                 const int32_t* boff_top, const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot) {
-  int rc = enqueue_stage_a(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot);
+                 const int32_t* boff_top, const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot, bool images) {
+  int rc = images ? enqueue_detect(fe, omni) : SOS_OK;
+  if (rc == SOS_OK) rc = enqueue_stage_a(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
   if (rc == SOS_OK) rc = enqueue_stage_b(fe);
   if (rc == SOS_OK && !fe->cfg.keyframe_mode) rc = enqueue_carry(fe, fe->cfg.batch);
   if (fe->remap_forked) {   // join the remap branch (also on an error path: a capture must not end with an open fork)
@@ -364,29 +522,49 @@ int enqueue_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, con
   return rc;
 }
 
+// images: an images-in step (the feature pointers are ignored, fe->det.f's are used)
 int run_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top, const int32_t* boff_top,
-             const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot) {
+             const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot, bool images = false) {
   sos_ctx* ctx = fe->ctx;
-  if (!fe->use_graph || ctx->prof) return enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot);
-  sos_frontend::GraphKey key = {{omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot}};
+  if (images) {
+    const sos_frontend_features& f = fe->det.f;
+    px_top = f.px_top; desc_top = f.desc_top; boff_top = f.boff_top;
+    px_bot = f.px_bot; desc_bot = f.desc_bot; boff_bot = f.boff_bot;
+  }
+  if (!fe->use_graph || ctx->prof) return enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
+  sos_frontend::GraphKey key;
+  memset(&key, 0, sizeof(key));
+  const void* ptrs[7] = {omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot};
+  memcpy(key.p, ptrs, sizeof(ptrs));
+  key.images = images ? 1 : 0;
+  // a graph holds the scratch arena's address: one captured before an eager run regrew the arena must not be replayed
+  for (size_t i = 0; i < fe->graphs.size();) {
+    if (fe->graphs[i].arena != ctx->arena) {
+      cudaGraphExecDestroy(fe->graphs[i].exec);
+      fe->graphs.erase(fe->graphs.begin() + i);
+    } else {
+      ++i;
+    }
+  }
   for (auto& g : fe->graphs) {
     if (memcmp(&g.key, &key, sizeof(key)) == 0) {
       SOS_CUDA(cudaGraphLaunch(g.exec, ctx->stream));
-      ctx->launches += fe->d.launches_per_step;
+      ctx->launches += g.launches;
       return SOS_OK;
     }
   }
   // first time with these buffers: run once eagerly (sizes the scratch arena), then capture
   const int64_t before = ctx->launches;
-  int rc = enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot);
+  int rc = enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
   if (rc) return rc;
-  fe->d.launches_per_step = (int)(ctx->launches - before);
+  const int launches = (int)(ctx->launches - before);
+  fe->d.launches_per_step = launches;
   SOS_CUDA(cudaStreamSynchronize(ctx->stream));
   // the eager run advanced the carried state; capturing does not execute anything
   cudaGraph_t graph = nullptr;
   SOS_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
   const int64_t l0 = ctx->launches;
-  rc = enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot);
+  rc = enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
   ctx->launches = l0;
   cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
   if (rc) {
@@ -399,6 +577,8 @@ int run_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const u
   }
   sos_frontend::GraphEntry ge;
   ge.key = key;
+  ge.launches = launches;
+  ge.arena = ctx->arena;   // the capture refuses to grow the arena, so this is the address the graph holds
   SOS_CUDA(cudaGraphInstantiate(&ge.exec, graph, 0));
   cudaGraphDestroy(graph);
   if (fe->graphs.size() >= 8) {
@@ -598,21 +778,114 @@ extern "C" int sos_frontend_get_buffers(sos_frontend* fe, sos_frontend_buffers* 
   return SOS_OK;
 }
 
-extern "C" int sos_frontend_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
-                                 const int32_t* bucket_off_top, const float* px_bot, const uint32_t* desc_bot,
-                                 const int32_t* bucket_off_bot) {
-  SOS_CHECK_ARG(fe, "fe is NULL");
-  SOS_CHECK_ARG(omni && px_top && desc_top && bucket_off_top && px_bot && desc_bot && bucket_off_bot, "NULL input");
+namespace {
+int step_device(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
+                const int32_t* bucket_off_top, const float* px_bot, const uint32_t* desc_bot, const int32_t* bucket_off_bot,
+                bool images) {
   SOS_CUDA(cudaSetDevice(fe->ctx->device));
   // inputs were produced on the caller's stream; results must be visible to it afterwards
   SOS_CUDA(cudaEventRecord(fe->ev_in, fe->parent->stream));
   SOS_CUDA(cudaStreamWaitEvent(fe->ctx->stream, fe->ev_in, 0));
   const int64_t before = fe->ctx->launches;
-  const int rc = run_step(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot);
+  const int rc = run_step(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, images);
   fe->parent->launches += fe->ctx->launches - before;
   if (rc) return rc;
   SOS_CUDA(cudaEventRecord(fe->ev_out, fe->ctx->stream));
   SOS_CUDA(cudaStreamWaitEvent(fe->parent->stream, fe->ev_out, 0));
+  return SOS_OK;
+}
+}  // namespace
+
+extern "C" int sos_frontend_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
+                                 const int32_t* bucket_off_top, const float* px_bot, const uint32_t* desc_bot,
+                                 const int32_t* bucket_off_bot) {
+  SOS_CHECK_ARG(fe, "fe is NULL");
+  SOS_CHECK_ARG(omni && px_top && desc_top && bucket_off_top && px_bot && desc_bot && bucket_off_bot, "NULL input");
+  return step_device(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, false);
+}
+
+extern "C" int sos_frontend_set_detector(sos_frontend* fe, const sos_detect_config* dcfg, const uint8_t* masks_top,
+                                         const uint8_t* masks_bot) {
+  SOS_CHECK_ARG(fe && dcfg, "NULL argument");
+  SOS_CHECK_ARG(masks_top && masks_bot, "NULL masks");
+  const sos_frontend_config& c = fe->cfg;
+  if (c.channels != 3 || c.n_buckets > 32) {
+    sos_set_error("sos_frontend_set_detector: the feature front needs 3-channel images and at most 32 buckets (channels %d, "
+                  "n_buckets %d)", c.channels, c.n_buckets);
+    return SOS_ERR_UNSUPPORTED;
+  }
+  SOS_CHECK_ARG(dcfg->corners_per_bucket >= 1 && dcfg->corners_per_bucket <= c.max_feat_per_bucket,
+                "corners_per_bucket must lie in [1, max_feat_per_bucket]");
+  SOS_CHECK_ARG(dcfg->median == 0 || dcfg->median == 1, "median must be 0 or 1");
+  SOS_CHECK_ARG(dcfg->quality_level > 0.0 && dcfg->min_distance >= 0.0 && dcfg->min_distance < 64.0,
+                "bad quality level / minimum distance");
+  SOS_CHECK_ARG(c.pano_rows > 62 && c.pano_cols > 62 && (size_t)c.pano_rows * c.pano_cols < (1ull << 31),
+                "panorama smaller than ORB's border or too large");
+  SOS_CHECK_ARG((long long)c.batch * c.n_buckets <= 65535, "too many (frame, bucket) lists");
+  SOS_CHECK_ARG(2ll * c.batch * c.n_buckets * c.max_feat_per_bucket < (1ll << 31), "too many corner slots");
+  SOS_CUDA(cudaSetDevice(fe->ctx->device));
+  Fence fence(fe);   // the masks may have been written on the caller's stream
+  sos_frontend::Detector& dt = fe->det;
+  const size_t B = c.batch, nb = c.n_buckets, Nmax = c.max_feat_per_bucket, F = c.max_feat_per_view;
+  const size_t plane = (size_t)c.pano_rows * c.pano_cols;
+  if (!dt.med) {
+    int rc = SOS_OK;
+    sos_frontend_features& f = dt.f;
+#define DT_ALLOC(ptr, count) \
+    if (rc == SOS_OK) rc = fe_alloc(fe, &(ptr), (count))
+    DT_ALLOC(dt.med, B * 2 * plane * 3); DT_ALLOC(dt.gray, B * 2 * plane); DT_ALLOC(dt.blur, B * 2 * plane);
+    DT_ALLOC(dt.mask_bits[0], plane); DT_ALLOC(dt.mask_bits[1], plane); DT_ALLOC(dt.flags, 2);
+    DT_ALLOC(dt.eig, B * plane); DT_ALLOC(dt.max_bits, B * nb); DT_ALLOC(dt.cand, B * nb);
+    DT_ALLOC(dt.keys, B * nb * SOS_GFT_CAP); DT_ALLOC(dt.rank, B * plane);
+    DT_ALLOC(dt.xy, 2 * B * nb * Nmax * 2); DT_ALLOC(dt.count, 2 * B * nb); DT_ALLOC(dt.kp_image, 2 * B * nb * Nmax);
+    DT_ALLOC(dt.kp_desc, 2 * B * nb * Nmax * 8); DT_ALLOC(dt.kp_keep, 2 * B * nb * Nmax);
+    DT_ALLOC(f.px_top, B * F * 2); DT_ALLOC(f.desc_top, B * F * 8); DT_ALLOC(f.boff_top, B * (nb + 1));
+    DT_ALLOC(f.px_bot, B * F * 2); DT_ALLOC(f.desc_bot, B * F * 8); DT_ALLOC(f.boff_bot, B * (nb + 1));
+    DT_ALLOC(f.detect_stats, B * 2 * 4);
+#undef DT_ALLOC
+    if (rc) return rc;
+    // the selection leaves every rank-image entry it sets back at -1, so one clear serves every later step
+    SOS_CUDA(cudaMemsetAsync(dt.rank, 0xFF, B * plane * sizeof(int32_t), fe->ctx->stream));
+  }
+  // corner slot (view, b, k, j) is described on gray plane 2 b + view
+  const size_t N = dcfg->corners_per_bucket;
+  std::vector<int32_t> img(2 * B * nb * N);
+  for (size_t i = 0; i < img.size(); ++i) {
+    const size_t vb = i / (nb * N);
+    img[i] = (int32_t)(2 * (vb % B) + vb / B);
+  }
+  SOS_CUDA(cudaMemcpyAsync(dt.kp_image, img.data(), img.size() * sizeof(int32_t), cudaMemcpyHostToDevice, fe->ctx->stream));
+  for (int view = 0; view < 2; ++view) {
+    const int rc = sos_gft_pack_masks(fe->ctx, view == 0 ? masks_top : masks_bot, c.pano_rows, c.pano_cols, c.n_buckets,
+                                      dt.mask_bits[view], dt.flags + view);
+    if (rc) return rc;
+  }
+  SOS_CUDA(cudaMemcpyAsync(dt.overlap, dt.flags, sizeof(dt.overlap), cudaMemcpyDeviceToHost, fe->ctx->stream));
+  SOS_CUDA(cudaStreamSynchronize(fe->ctx->stream));
+  dt.cfg = *dcfg;
+  dt.on = true;
+  // captured images-in steps bake the previous detector's parameters in
+  for (size_t i = 0; i < fe->graphs.size();) {
+    if (fe->graphs[i].key.images) {
+      cudaGraphExecDestroy(fe->graphs[i].exec);
+      fe->graphs.erase(fe->graphs.begin() + i);
+    } else {
+      ++i;
+    }
+  }
+  return SOS_OK;
+}
+
+extern "C" int sos_frontend_step_images(sos_frontend* fe, const uint8_t* omni) {
+  SOS_CHECK_ARG(fe && omni, "NULL argument");
+  SOS_CHECK_ARG(fe->det.on, "no detector: call sos_frontend_set_detector first");
+  return step_device(fe, omni, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, true);
+}
+
+extern "C" int sos_frontend_get_features(sos_frontend* fe, sos_frontend_features* out) {
+  SOS_CHECK_ARG(fe && out, "NULL argument");
+  SOS_CHECK_ARG(fe->det.on, "no detector: call sos_frontend_set_detector first");
+  *out = fe->det.f;
   return SOS_OK;
 }
 
@@ -699,11 +972,11 @@ extern "C" int sos_frontend_host_bytes(sos_frontend* fe, int64_t* h2d_bytes_per_
   return SOS_OK;
 }
 
-extern "C" int sos_frontend_submit_host(sos_frontend* fe, const uint8_t* omni, const float* px_top,
-                                        const uint32_t* desc_top, const int32_t* bucket_off_top, const float* px_bot,
-                                        const uint32_t* desc_bot, const int32_t* bucket_off_bot, int* ticket) {
-  SOS_CHECK_ARG(fe && ticket, "NULL argument");
-  SOS_CHECK_ARG(omni && px_top && desc_top && bucket_off_top && px_bot && desc_bot && bucket_off_bot, "NULL input");
+namespace {
+// H2D of one step's inputs on the copy stream (so that it overlaps the kernels of the previous step), the step, and the
+// D2H of poses and stats.  images: only the omni images are uploaded and the features are detected on the device.
+int submit(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top, const int32_t* bucket_off_top,
+           const float* px_bot, const uint32_t* desc_bot, const int32_t* bucket_off_bot, bool images, int* ticket) {
   SOS_CUDA(cudaSetDevice(fe->ctx->device));
   int rc = ensure_staging(fe);
   if (rc) return rc;
@@ -716,7 +989,6 @@ extern "C" int sos_frontend_submit_host(sos_frontend* fe, const uint8_t* omni, c
   const sos_frontend_config& c = fe->cfg;
   const size_t B = c.batch, F = c.max_feat_per_view;
   cudaStream_t cs = fe->copy_stream;
-  // H2D on the copy stream so that it overlaps the kernels of the previous step
   if (fe->bands.empty()) {
     SOS_CUDA(cudaMemcpyAsync(s.omni, omni, B * c.src_h * c.src_w * c.channels, cudaMemcpyHostToDevice, cs));
   } else {
@@ -733,16 +1005,18 @@ extern "C" int sos_frontend_submit_host(sos_frontend* fe, const uint8_t* omni, c
       SOS_CUDA(cudaMemcpy3DAsync(&p, cs));
     }
   }
-  SOS_CUDA(cudaMemcpyAsync(s.px_top, px_top, B * F * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
-  SOS_CUDA(cudaMemcpyAsync(s.px_bot, px_bot, B * F * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
-  SOS_CUDA(cudaMemcpyAsync(s.desc_top, desc_top, B * F * 32, cudaMemcpyHostToDevice, cs));
-  SOS_CUDA(cudaMemcpyAsync(s.desc_bot, desc_bot, B * F * 32, cudaMemcpyHostToDevice, cs));
-  SOS_CUDA(cudaMemcpyAsync(s.boff_top, bucket_off_top, B * (c.n_buckets + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
-  SOS_CUDA(cudaMemcpyAsync(s.boff_bot, bucket_off_bot, B * (c.n_buckets + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+  if (!images) {
+    SOS_CUDA(cudaMemcpyAsync(s.px_top, px_top, B * F * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.px_bot, px_bot, B * F * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.desc_top, desc_top, B * F * 32, cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.desc_bot, desc_bot, B * F * 32, cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.boff_top, bucket_off_top, B * (c.n_buckets + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.boff_bot, bucket_off_bot, B * (c.n_buckets + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+  }
   SOS_CUDA(cudaEventRecord(s.copied, cs));
   SOS_CUDA(cudaStreamWaitEvent(fe->ctx->stream, s.copied, 0));
   const int64_t before = fe->ctx->launches;
-  rc = run_step(fe, s.omni, s.px_top, s.desc_top, s.boff_top, s.px_bot, s.desc_bot, s.boff_bot);
+  rc = run_step(fe, s.omni, s.px_top, s.desc_top, s.boff_top, s.px_bot, s.desc_bot, s.boff_bot, images);
   fe->parent->launches += fe->ctx->launches - before;
   if (rc) return rc;
   SOS_CUDA(cudaMemcpyAsync(s.h_poses, fe->d.pose, B * 12 * sizeof(float), cudaMemcpyDeviceToHost, fe->ctx->stream));
@@ -753,6 +1027,21 @@ extern "C" int sos_frontend_submit_host(sos_frontend* fe, const uint8_t* omni, c
   *ticket = k;
   fe->next_stage = (k + 1) % sos_frontend::DEPTH;
   return SOS_OK;
+}
+}  // namespace
+
+extern "C" int sos_frontend_submit_host(sos_frontend* fe, const uint8_t* omni, const float* px_top,
+                                        const uint32_t* desc_top, const int32_t* bucket_off_top, const float* px_bot,
+                                        const uint32_t* desc_bot, const int32_t* bucket_off_bot, int* ticket) {
+  SOS_CHECK_ARG(fe && ticket, "NULL argument");
+  SOS_CHECK_ARG(omni && px_top && desc_top && bucket_off_top && px_bot && desc_bot && bucket_off_bot, "NULL input");
+  return submit(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, false, ticket);
+}
+
+extern "C" int sos_frontend_submit_host_images(sos_frontend* fe, const uint8_t* omni, int* ticket) {
+  SOS_CHECK_ARG(fe && ticket && omni, "NULL argument");
+  SOS_CHECK_ARG(fe->det.on, "no detector: call sos_frontend_set_detector first");
+  return submit(fe, omni, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, true, ticket);
 }
 
 extern "C" int sos_frontend_wait_host(sos_frontend* fe, int ticket, float* poses, int32_t* stats) {

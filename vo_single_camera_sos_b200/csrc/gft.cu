@@ -47,13 +47,13 @@ __device__ __forceinline__ int refl(int p, int n) {
 constexpr int GE_ROWS = 16;   // rows per block
 
 __global__ void __launch_bounds__(256, 3)
-gft_eig_kernel(const uint8_t* __restrict__ gray, int H, int W, float* __restrict__ eig, const uint32_t* __restrict__ mask_bits,
-               int n_masks, uint32_t* __restrict__ max_bits) {
+gft_eig_kernel(const uint8_t* __restrict__ gray, size_t img_stride, int H, int W, float* __restrict__ eig,
+               const uint32_t* __restrict__ mask_bits, int n_masks, uint32_t* __restrict__ max_bits) {
   const int xr = blockIdx.x * blockDim.x + threadIdx.x, img = blockIdx.z;
   const int y0 = blockIdx.y * GE_ROWS, y1 = min(H, y0 + GE_ROWS);
   const bool in = xr < W;
   const int x = in ? xr : W - 1;
-  const uint8_t* g = gray + (size_t)img * H * W;
+  const uint8_t* g = gray + (size_t)img * img_stride;
   // the three columns whose covariance terms enter this pixel's box sums (BORDER_REFLECT_101), each with its own Sobel taps
   int cx[3][3];
 #pragma unroll
@@ -275,7 +275,7 @@ gft_candidates_kernel(const float* __restrict__ eig, const uint32_t* __restrict_
   }
 }
 
-constexpr int GFT_CAP = 16384;      // candidates per (image, mask) kept for the selection (128 KB of shared memory)
+constexpr int GFT_CAP = SOS_GFT_CAP; // candidates per (image, mask) kept for the selection (128 KB of shared memory)
 constexpr int GFT_THREADS = 1024;
 constexpr int GFT_K = 4;            // stronger neighbours remembered per candidate (more: rescan the rank image)
 
@@ -519,9 +519,58 @@ extern "C" int sos_corner_min_eigenval(sos_ctx* ctx, const uint8_t* gray, int n_
   SOS_CHECK_ARG(gray && eig, "NULL array");
   SOS_CHECK_ARG(n_images <= 65535 && height <= 65535, "too many images / rows");
   SOS_CUDA(cudaSetDevice(ctx->device));
-  gft_eig_kernel<<<dim3(sos_div_up(width, 256), sos_div_up(height, GE_ROWS), n_images), 256, 0, ctx->stream>>>(gray, height, width, eig, nullptr, 0,
-                                                                                                                 nullptr);
+  gft_eig_kernel<<<dim3(sos_div_up(width, 256), sos_div_up(height, GE_ROWS), n_images), 256, 0, ctx->stream>>>(
+      gray, (size_t)height * width, height, width, eig, nullptr, 0, nullptr);
   SOS_LAUNCHED_AS(ctx, "gft_eig_kernel");
+  return SOS_OK;
+}
+
+int sos_gft_pack_masks(sos_ctx* ctx, const uint8_t* masks, int height, int width, int n_masks, uint32_t* bits,
+                       int32_t* overlap) {
+  const size_t per = (size_t)height * width;
+  SOS_CUDA(cudaMemsetAsync(overlap, 0, sizeof(int32_t), ctx->stream));
+  gft_pack_masks_kernel<<<(unsigned)((per + 255) / 256), 256, 0, ctx->stream>>>(masks, per, n_masks, bits, overlap);
+  SOS_LAUNCHED_AS(ctx, "gft_pack_masks_kernel");
+  return SOS_OK;
+}
+
+int sos_gft_candidates(sos_ctx* ctx, const sos_gft_work& w, const uint8_t* gray, size_t img_stride, int n_images, int height,
+                       int width, int n_masks, double quality_level) {
+  const size_t lists = (size_t)n_images * n_masks;
+  SOS_CUDA(cudaMemsetAsync(w.max_bits, 0, lists * sizeof(uint32_t), ctx->stream));
+  SOS_CUDA(cudaMemsetAsync(w.counts, 0, lists * sizeof(int32_t), ctx->stream));
+  gft_eig_kernel<<<dim3(sos_div_up(width, 256), sos_div_up(height, GE_ROWS), n_images), 256, 0, ctx->stream>>>(
+      gray, img_stride, height, width, w.eig, w.mask_bits, n_masks, w.max_bits);
+  SOS_LAUNCHED_AS(ctx, "gft_eig_kernel");
+  gft_candidates_kernel<<<dim3(sos_div_up(width, 256), sos_div_up(height, GC_ROWS), n_images), 256, 0, ctx->stream>>>(
+      w.eig, w.mask_bits, height, width, n_masks, w.max_bits, quality_level, GFT_CAP, w.keys, w.counts);
+  SOS_LAUNCHED_AS(ctx, "gft_candidates_kernel");
+  return SOS_OK;
+}
+
+int sos_gft_select(sos_ctx* ctx, const sos_gft_work& w, int n_images, int height, int width, int n_masks, int max_corners,
+                   double min_distance, bool overlap, int np2, float* out_xy, int32_t* out_count) {
+  // per device, so set on every call (a process may hold contexts on several devices)
+  SOS_CUDA(cudaFuncSetAttribute(gft_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gft_select_smem(GFT_CAP)));
+  const double md2 = min_distance * min_distance;
+  const int min_dist_sq = min_distance >= 1.0 ? (int)ceil(md2) : 0;   // integer offsets: dx^2 + dy^2 < minDistance^2
+  const int reach = (int)ceil(min_distance);
+  const size_t smem = gft_select_smem(np2);
+  // pixel-disjoint masks (the reference's default, overlap_degrees = 0): every list at once.  Overlapping masks: a pixel can
+  // be a candidate of two lists and each selection needs the rank image of its image to itself -> one launch per mask.
+  if (!overlap) {
+    gft_select_kernel<<<n_images * n_masks, GFT_THREADS, smem, ctx->stream>>>(w.keys, w.counts, GFT_CAP, height, width, n_masks,
+                                                                            -1, max_corners, min_dist_sq, reach, w.rank_img,
+                                                                            out_xy, out_count);
+    SOS_LAUNCHED_AS(ctx, "gft_select_kernel");
+    return SOS_OK;
+  }
+  for (int m = 0; m < n_masks; ++m) {
+    gft_select_kernel<<<n_images, GFT_THREADS, smem, ctx->stream>>>(w.keys, w.counts, GFT_CAP, height, width, n_masks, m,
+                                                                    max_corners, min_dist_sq, reach, w.rank_img, out_xy,
+                                                                    out_count);
+    SOS_LAUNCHED_AS(ctx, "gft_select_kernel");
+  }
   return SOS_OK;
 }
 
@@ -551,36 +600,22 @@ extern "C" int sos_gft_detect(sos_ctx* ctx, const uint8_t* gray, const uint8_t* 
   const size_t o_flag = take(sizeof(int32_t));
   const size_t o_bits = take((size_t)height * width * sizeof(uint32_t));
   void* ws = nullptr;
-  const int rc = sos_arena_get(ctx, off, &ws);
+  int rc = sos_arena_get(ctx, off, &ws);
   if (rc != SOS_OK) return rc;
   uint8_t* base = (uint8_t*)ws;
-  float* eig = (float*)(base + o_eig);
-  uint32_t* max_bits = (uint32_t*)(base + o_max);
-  int32_t* counts = (int32_t*)(base + o_cnt);
-  unsigned long long* keys = (unsigned long long*)(base + o_keys);
-  int32_t* rank_img = (int32_t*)(base + o_rank);
-
-  dim3 grid(sos_div_up(width, 256), height, n_images);
-  const size_t per = (size_t)height * width;
-  uint32_t* mask_bits = (uint32_t*)(base + o_bits);
+  sos_gft_work w;
+  w.mask_bits = (uint32_t*)(base + o_bits);
+  w.eig = (float*)(base + o_eig);
+  w.max_bits = (uint32_t*)(base + o_max);
+  w.counts = (int32_t*)(base + o_cnt);
+  w.keys = (unsigned long long*)(base + o_keys);
+  w.rank_img = (int32_t*)(base + o_rank);
   int32_t* flag = (int32_t*)(base + o_flag);
-  SOS_CUDA(cudaMemsetAsync(base + o_max, 0, (o_keys - o_max), ctx->stream));          // max_bits and counts
-  SOS_CUDA(cudaMemsetAsync(flag, 0, sizeof(int32_t), ctx->stream));
-  SOS_CUDA(cudaMemsetAsync(rank_img, 0xFF, px * sizeof(int32_t), ctx->stream));       // -1
-  gft_pack_masks_kernel<<<(unsigned)((per + 255) / 256), 256, 0, ctx->stream>>>(masks, per, n_masks, mask_bits, flag);
-  SOS_LAUNCHED_AS(ctx, "gft_pack_masks_kernel");
-  gft_eig_kernel<<<dim3(grid.x, sos_div_up(height, GE_ROWS), grid.z), 256, 0, ctx->stream>>>(gray, height, width, eig, mask_bits, n_masks, max_bits);
-  SOS_LAUNCHED_AS(ctx, "gft_eig_kernel");
-  if (eig_out) SOS_CUDA(cudaMemcpyAsync(eig_out, eig, px * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
-  gft_candidates_kernel<<<dim3(sos_div_up(width, 256), sos_div_up(height, GC_ROWS), n_images), 256, 0, ctx->stream>>>(
-      eig, mask_bits, height, width, n_masks, max_bits, quality_level, GFT_CAP, keys, counts);
-  SOS_LAUNCHED_AS(ctx, "gft_candidates_kernel");
-  const size_t smem = gft_select_smem(GFT_CAP);
-  // per device, so set on every call (a process may hold contexts on several devices)
-  SOS_CUDA(cudaFuncSetAttribute(gft_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const double md2 = min_distance * min_distance;
-  const int min_dist_sq = min_distance >= 1.0 ? (int)ceil(md2) : 0;   // integer offsets: dx^2 + dy^2 < minDistance^2
-  const int reach = (int)ceil(min_distance);
+  SOS_CUDA(cudaMemsetAsync(w.rank_img, 0xFF, px * sizeof(int32_t), ctx->stream));   // -1
+  rc = sos_gft_pack_masks(ctx, masks, height, width, n_masks, (uint32_t*)w.mask_bits, flag);
+  if (rc == SOS_OK) rc = sos_gft_candidates(ctx, w, gray, (size_t)height * width, n_images, height, width, n_masks, quality_level);
+  if (rc != SOS_OK) return rc;
+  if (eig_out) SOS_CUDA(cudaMemcpyAsync(eig_out, w.eig, px * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
   // One small read-back on every call: the overlap flag and the candidate counts.  A list with more candidates than the
   // buffer holds is refused (the atomics that filled the buffer kept a schedule-dependent subset), and the largest count
   // sizes the selection's shared memory (a block sorts next_pow2(count) keys: 64 KB instead of 128 KB lets three blocks
@@ -588,7 +623,7 @@ extern "C" int sos_gft_detect(sos_ctx* ctx, const uint8_t* gray, const uint8_t* 
   int overlap = 0;
   std::vector<int32_t> hc(lists);
   SOS_CUDA(cudaMemcpyAsync(&overlap, flag, sizeof(int32_t), cudaMemcpyDeviceToHost, ctx->stream));
-  SOS_CUDA(cudaMemcpyAsync(hc.data(), counts, sizeof(int32_t) * lists, cudaMemcpyDeviceToHost, ctx->stream));
+  SOS_CUDA(cudaMemcpyAsync(hc.data(), w.counts, sizeof(int32_t) * lists, cudaMemcpyDeviceToHost, ctx->stream));
   SOS_CUDA(cudaStreamSynchronize(ctx->stream));
   int mx = 1;
   for (int v : hc) {
@@ -600,19 +635,6 @@ extern "C" int sos_gft_detect(sos_ctx* ctx, const uint8_t* gray, const uint8_t* 
   }
   int np2 = 1024;
   while (np2 < mx) np2 <<= 1;
-  const size_t sel_smem = gft_select_smem(np2);
-  // pixel-disjoint masks (the reference's default, overlap_degrees = 0): every list at once.  Overlapping masks: a pixel can
-  // be a candidate of two lists and each selection needs the rank image of its image to itself -> one launch per mask.
-  if (!overlap) {
-    gft_select_kernel<<<lists, GFT_THREADS, sel_smem, ctx->stream>>>(keys, counts, GFT_CAP, height, width, n_masks, -1, max_corners,
-                                                                 min_dist_sq, reach, rank_img, out_xy, out_count);
-    SOS_LAUNCHED_AS(ctx, "gft_select_kernel");
-    return SOS_OK;
-  }
-  for (int m = 0; m < n_masks; ++m) {
-    gft_select_kernel<<<n_images, GFT_THREADS, sel_smem, ctx->stream>>>(keys, counts, GFT_CAP, height, width, n_masks, m, max_corners,
-                                                                    min_dist_sq, reach, rank_img, out_xy, out_count);
-    SOS_LAUNCHED_AS(ctx, "gft_select_kernel");
-  }
-  return SOS_OK;
+  return sos_gft_select(ctx, w, n_images, height, width, n_masks, max_corners, min_distance, overlap != 0, np2,
+                        out_xy, out_count);
 }

@@ -219,12 +219,18 @@ extern "C" int sos_orb_describe(sos_ctx* ctx, const uint8_t* gray, int n_images,
   SOS_CHECK_ARG(gray && kp_xy && desc, "NULL array");
   SOS_CHECK_ARG(n_images >= 1 && height > 2 * ORB_EDGE && width > 2 * ORB_EDGE, "image smaller than the ORB border");
   void* ws = nullptr;
-  int rc = sos_arena_get(ctx, sos_align_up((size_t)n_images * height * width, 256), &ws);
+  const int rc = sos_arena_get(ctx, sos_align_up((size_t)n_images * height * width, 256), &ws);
   if (rc != SOS_OK) return rc;
-  rc = sos_orb_blur(ctx, gray, n_images, height, width, (uint8_t*)ws);
+  return sos_orb_describe_into(ctx, gray, n_images, height, width, kp_xy, kp_angle_deg, kp_image, n, desc, keep, (uint8_t*)ws);
+}
+
+int sos_orb_describe_into(sos_ctx* ctx, const uint8_t* gray, int n_images, int height, int width, const float* kp_xy,
+                          const float* kp_angle_deg, const int32_t* kp_image, int n, uint32_t* desc, uint8_t* keep,
+                          uint8_t* blurred) {
+  const int rc = sos_orb_blur(ctx, gray, n_images, height, width, blurred);
   if (rc != SOS_OK) return rc;
-  orb_describe_kernel<<<sos_div_up(n, 8), 256, 0, ctx->stream>>>((const uint8_t*)ws, height, width, (const float2*)kp_xy,
-                                                                 kp_angle_deg, kp_image, n, desc, keep);
+  orb_describe_kernel<<<sos_div_up(n, 8), 256, 0, ctx->stream>>>(blurred, height, width, (const float2*)kp_xy, kp_angle_deg,
+                                                                 kp_image, n, desc, keep);
   SOS_LAUNCHED_AS(ctx, "orb_describe_kernel");
   return SOS_OK;
 }

@@ -1,7 +1,9 @@
 """Python handle on the batched GPU-resident SOS front-end (sos_frontend_* in include/sosfront.h).
 
 `Frontend.step(...)` takes device tensors, `Frontend.step_host(...)` / `submit_host` + `wait_host` take pinned host
-arrays (the end-to-end path: H2D, kernels, D2H).  All data-dependent sizes stay on the device; see csrc/frontend.cu.
+arrays (the end-to-end path: H2D, kernels, D2H).  After `set_detector(...)`, `step_images` / `step_host_images` take the
+omni images alone and detect the features inside the step.  All data-dependent sizes stay on the device; see
+csrc/frontend.cu.
 """
 from __future__ import annotations
 
@@ -114,6 +116,18 @@ class FrontendConfig:
         c.border[:] = [int(x) for x in b[:4]]
         c.background[:] = [int(x) for x in g[:4]]
         return c
+
+
+class _DetectConfig(C.Structure):
+    _fields_ = [("corners_per_bucket", C.c_int32), ("median", C.c_int32), ("quality_level", C.c_double),
+                ("min_distance", C.c_double)]
+
+
+_FEATURE_FIELDS = ["px_top", "desc_top", "boff_top", "px_bot", "desc_bot", "boff_bot", "detect_stats"]
+
+
+class _Features(C.Structure):
+    _fields_ = [(name, C.c_void_p) for name in _FEATURE_FIELDS]
 
 
 class _DeviceArray:
@@ -259,6 +273,78 @@ class Frontend:
 
     def step_host(self, *inputs):
         return self.wait_host(self.submit_host(*inputs))
+
+    # -- images-in steps (sos_frontend_set_detector) -------------------------------------------------------------------
+    def set_detector(self, masks_top, masks_bot, corners_per_bucket: int, quality_level: float = 0.01,
+                     min_distance: float = 5.0, median: bool = True):
+        """Detect the features inside the step, as features.FeatureFront does: masks uint8 [n_buckets, pano_rows,
+        pano_cols] per view (numpy or torch), goodFeaturesToTrack(maxCorners = corners_per_bucket, quality_level,
+        min_distance) per mask after an optional 11 x 11 median, then ORB description."""
+        c = self.cfg
+        ms = []
+        for name, m in (("masks_top", masks_top), ("masks_bot", masks_bot)):
+            t = (m if isinstance(m, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(m))).to(self.ctx.device)
+            if tuple(t.shape) != (c.n_buckets, c.pano_rows, c.pano_cols):
+                raise ValueError(f"{name} must be [n_buckets, pano_rows, pano_cols]")
+            ms.append(t.contiguous())
+        d = _DetectConfig(int(corners_per_bucket), int(bool(median)), float(quality_level), float(min_distance))
+        self.ctx._sync_stream()
+        # the masks are packed into bits by the call, which returns after that: they need not outlive it
+        check(self.ctx.lib.sos_frontend_set_detector(self._h, C.byref(d), *(self.ctx._t(m, torch.uint8, "masks") for m in ms)))
+
+    def _check_omni(self, omni, on_device: bool):
+        c = self.cfg
+        shape = (c.batch, c.src_h, c.src_w, c.channels)
+        if tuple(omni.shape) != shape:
+            raise ValueError(f"omni: expected shape {shape}, got {tuple(omni.shape)}")
+        if on_device:
+            return self.ctx._t(omni, torch.uint8, "omni")
+        if isinstance(omni, torch.Tensor):
+            if omni.is_cuda or omni.dtype != torch.uint8 or not omni.is_contiguous():
+                raise TypeError("omni: expected a contiguous host tensor of torch.uint8")
+            return omni.data_ptr()
+        if omni.dtype != np.uint8 or not omni.flags.c_contiguous:
+            raise TypeError("omni: expected a C-contiguous host array of uint8")
+        return omni.ctypes.data
+
+    def step_images(self, omni):
+        """Asynchronous images-in step on device omni [batch, src_h, src_w, 3]; results in `buffers()` / `features()`."""
+        p = self._check_omni(omni, True)
+        self.ctx._sync_stream()
+        check(self.ctx.lib.sos_frontend_step_images(self._h, p))
+
+    def submit_host_images(self, omni) -> int:
+        """Images-in step on host omni (pinned): only the LUT-reachable image bands go over PCIe.  -> ticket for wait_host."""
+        p = self._check_omni(omni, False)
+        t = C.c_int()
+        self.ctx._sync_stream()
+        check(self.ctx.lib.sos_frontend_submit_host_images(self._h, p, C.byref(t)))
+        return t.value
+
+    def step_host_images(self, omni):
+        return self.wait_host(self.submit_host_images(omni))
+
+    def host_images_bytes(self) -> int:
+        """H2D bytes of one submit_host_images: host_bytes() without the feature arrays."""
+        c = self.cfg
+        h2d, _ = self.host_bytes()
+        return h2d - c.batch * (2 * c.max_feat_per_view * (2 * 4 + 32) + 2 * (c.n_buckets + 1) * 4)
+
+    def features(self) -> dict:
+        """Zero-copy torch views of the features the last images-in step detected (layout of `step`'s inputs, desc as
+        uint8 [batch, max_feat_per_view, 32]) and detect_stats int32 [batch, 2, 4] (valid until close())."""
+        f = _Features()
+        check(self.ctx.lib.sos_frontend_get_features(self._h, C.byref(f)))
+        c = self.cfg
+        B, F, nb = c.batch, c.max_feat_per_view, c.n_buckets
+        shapes = {"px_top": ((B, F, 2), "f32"), "desc_top": ((B, F, 32), "u8"), "boff_top": ((B, nb + 1), "i32"),
+                  "px_bot": ((B, F, 2), "f32"), "desc_bot": ((B, F, 32), "u8"), "boff_bot": ((B, nb + 1), "i32"),
+                  "detect_stats": ((B, 2, 4), "i32")}
+        out = {}
+        for name in _FEATURE_FIELDS:
+            shape, kind = shapes[name]
+            out[name] = torch.as_tensor(_DeviceArray(getattr(f, name), shape, _TYPES[kind][0], self), device=self.ctx.device)
+        return out
 
     def buffers(self) -> dict:
         """Zero-copy torch views of the device buffers (valid until close())."""
