@@ -510,6 +510,9 @@ typedef struct sos_frontend_config {
 
 /* Device buffers of the front-end, exposed for parity tests and for consumers that keep working on the device.
  * "store" arrays hold batch+1 slots of `cap` rows: slot 0 = carried reference frame, slot i+1 = frame i of the step. */
+/* An RGB-D front-end (sos_frontend_create_rgbd) has one view: the store holds per slot the valid keypoints of a frame
+ * (uv = float keypoint coordinates, b_top = bearings, xyz, desc_c, src_top = input row), and pano, st_*, uv_bot, b_bot,
+ * src_bot, cam (central camera) and overflow are NULL. */
 typedef struct sos_frontend_buffers {
   uint8_t* pano;                                   /* [batch, 2, rows, cols, ch] */
   int32_t *st_q_start, *st_q_len, *st_t_start, *st_t_len; /* stereo segments [batch*n_buckets] */
@@ -534,6 +537,9 @@ typedef struct sos_frontend_buffers {
                                                       last step (bucket > max_feat_per_bucket, offsets > max_feat_per_view);
                                                       0 everywhere unless the configuration is too small for the input */
   int32_t batch, cap, launches_per_step;
+  int32_t views;                                   /* 2 (SOS: top, bottom) or 1 (RGB-D); the temporal-matching arrays hold
+                                                      `views` blocks and the RANSAC problems (p_ref .. inlier_mask) have
+                                                      a stride of views*cap rows */
 } sos_frontend_buffers;
 
 typedef struct sos_frontend sos_frontend;
@@ -624,6 +630,50 @@ int sos_frontend_step_images(sos_frontend* fe, const uint8_t* omni);
  * then sos_frontend_wait_host. */
 int sos_frontend_submit_host_images(sos_frontend* fe, const uint8_t* omni, int* ticket);
 int sos_frontend_get_features(sos_frontend* fe, sos_frontend_features* out);
+
+/* ------------------------------------------------------------------------------------------------
+ * The batched RGB-D front-end (BASELINE configuration 5): depth maps + keypoints in, frame-pair poses out
+ * ---------------------------------------------------------------------------------------------- */
+
+/* One step chains, for a batch of frames, what RGBDFrame.establish_keypoints (pose_est_tools.py:600-623) and
+ * TrackerRGBDSE3.track_frame (pose_est_tools.py:880-958) do for one frame:
+ *   store      per frame: pixel (trunc(x), trunc(y)) of every keypoint, depth lookup, back-projection and |Z| gate with
+ *              the arithmetic of sos_rgbd_backproject (bit-equal), ordered compaction of the valid keypoints into the
+ *              frame's store slot; a keypoint whose pixel lies outside the map is dropped;
+ *   matching   query = current frame, train = reference frame, 1-NN Hamming, sorted by (distance, query), |du| gate;
+ *   RANSAC     central camera, bearing score, on the shared hypothesis list (Arun or three-point hypotheses);
+ *   pose       refit as sos_frontend_config.refit.
+ * Pairs, reference slots, keyframe mode and the calls that work on either kind of front-end (destroy, reset, set_graph,
+ * set_ref_slots, promote, retrack, get_buffers, profile_begin / _end, host_bytes, wait_host) are those of the SOS
+ * front-end above.  sos_frontend_step, step_host, submit_host, set_detector, step_images, submit_host_images and
+ * get_features refuse an RGB-D front-end (SOS_ERR_INVALID), and the RGB-D calls below refuse an SOS front-end. */
+typedef struct sos_rgbd_frontend_config {
+  int32_t batch;               /* frames per step */
+  int32_t height, width;       /* depth map size */
+  int32_t max_kp;              /* keypoint rows per frame in the inputs, and the store capacity per frame */
+  int32_t n_hyp;               /* RANSAC hypotheses (210, pose_est_tools.py:709-720) */
+  int32_t solver;              /* SOS_SOLVER_ARUN (hyp [n_hyp,3]) or SOS_SOLVER_P3P (hyp [n_hyp,4]) */
+  int32_t refit;               /* SOS_REFINE_* */
+  int32_t refine_iters;        /* SOS_REFINE_LM: maximum cost evaluations (0 = 20) */
+  int32_t keyframe_mode;       /* as sos_frontend_config.keyframe_mode */
+  double cam[SOS_RGBD_NPARAMS]; /* intrinsics, as sos_rgbd_backproject */
+  double min_z, max_z;         /* |Z| gate in model units: 0.8, 7 m (pose_est_tools.py:429-430) */
+  double temporal_max_du;      /* 0.5 * 2 * cx (pose_est_tools.py:958) */
+  double ransac_threshold;     /* 1 - cos(5 deg) */
+} sos_rgbd_frontend_config;
+
+/* hyp is a DEVICE array that must outlive the front-end; destroy with sos_frontend_destroy. */
+int sos_frontend_create_rgbd(sos_ctx* ctx, const sos_rgbd_frontend_config* cfg, const uint32_t* hyp, sos_frontend** out);
+/* One step on DEVICE-resident inputs (asynchronous; after the first call with given pointers a captured graph is replayed):
+ *   depth [batch, height, width] float32     px [batch, max_kp, 2] float32 keypoint (x, y)
+ *   desc  [batch, max_kp, 8] uint32           n_kp [batch] int32: rows of frame b are 0 .. n_kp[b]-1
+ * n_kp is read on the device and clamped to [0, max_kp].  Output in the buffers: pose [batch,12], stats [batch,4] = valid
+ * keypoints of the frame, correspondences, inliers, best hypothesis. */
+int sos_frontend_step_rgbd(sos_frontend* fe, const float* depth, const float* px, const uint32_t* desc, const int32_t* n_kp);
+/* The same step on HOST inputs (pinned for full copy bandwidth), whole depth maps uploaded; n_kp[b] outside [0, max_kp]
+ * is refused.  Then sos_frontend_wait_host. */
+int sos_frontend_submit_host_rgbd(sos_frontend* fe, const float* depth, const float* px, const uint32_t* desc,
+                                  const int32_t* n_kp, int* ticket);
 
 /* ------------------------------------------------------------------------------------------------
  * Roofline denominators measured in-process (integer POPC pipe, FP32 FMA pipe) — bench.py only.

@@ -90,6 +90,9 @@ PROTOTYPES = {
     "sos_frontend_step_images": (I, [C.c_void_p, P]),
     "sos_frontend_submit_host_images": (I, [C.c_void_p, P, C.POINTER(I)]),
     "sos_frontend_get_features": (I, [C.c_void_p, P]),
+    "sos_frontend_create_rgbd": (I, [c_ctx, P, P, C.POINTER(C.c_void_p)]),
+    "sos_frontend_step_rgbd": (I, [C.c_void_p, P, P, P, P]),
+    "sos_frontend_submit_host_rgbd": (I, [C.c_void_p, P, P, P, P, C.POINTER(I)]),
     "sos_peak_popc": (I, [c_ctx, C.POINTER(D)]),
     "sos_peak_ffma": (I, [c_ctx, C.POINTER(D)]),
     "sos_peak_dfma": (I, [c_ctx, C.POINTER(D)]),

@@ -13,6 +13,10 @@
 //   temporal Hamming match top<->top, bottom<->bottom           pose_est_tools.py:741-749, 211-269
 //   stack correspondences (top first, then bottom)             pose_est_tools.py:752-778
 //   RANSAC over seeded Arun hypotheses (+ inlier refit)        pose_est_tools.py:785, 830
+//
+// The RGB-D front-end (sos_frontend_create_rgbd) runs the same stage B on one view and a central camera, after a store
+// stage of its own (rgbd_store_kernel): RGBDFrame.establish_keypoints (pose_est_tools.py:600-623) and
+// TrackerRGBDSE3.track_frame (pose_est_tools.py:880-958).
 #include <string.h>
 
 #include <vector>
@@ -20,6 +24,7 @@
 #include <algorithm>
 #include <climits>
 
+#include "rgbd.cuh"
 #include "sos_common.cuh"
 
 namespace {
@@ -73,12 +78,12 @@ __global__ void gather_desc_kernel(const uint4* __restrict__ desc_top, const uin
 }
 
 // Pair i tracks store slot i + 1 against its reference slot: slot i (consecutive frames) or ref_slot[i] (keyframe mode:
-// the slot of the tracking reference, pose_est_tools.py:1489; -1 = pair switched off).
+// the slot of the tracking reference, pose_est_tools.py:1489; -1 = pair switched off).  One segment per view and pair.
 __global__ void temporal_segments_kernel(const int32_t* __restrict__ n, const int32_t* __restrict__ ref_slot, int B, int cap,
-                                         int32_t* __restrict__ q_start, int32_t* __restrict__ q_len,
+                                         int views, int32_t* __restrict__ q_start, int32_t* __restrict__ q_len,
                                          int32_t* __restrict__ t_start, int32_t* __restrict__ t_len) {
   const int s = blockIdx.x * blockDim.x + threadIdx.x;
-  if (s >= 2 * B) return;
+  if (s >= views * B) return;
   const int view = s / B, i = s % B;
   const int r = ref_slot ? ref_slot[i] : i;
   const bool on = r >= 0 && r <= B && r != i + 1;
@@ -88,21 +93,22 @@ __global__ void temporal_segments_kernel(const int32_t* __restrict__ n, const in
   t_len[s] = on ? n[r] : 0;
 }
 
-// Stack the temporal matches of both views into one correspondence list per frame pair (pose_est_tools.py:752-778).
+// Stack the temporal matches of both views into one correspondence list per frame pair (pose_est_tools.py:752-778); with
+// one view (RGB-D, pose_est_tools.py:912-914) the list is that view's matches and cam is NULL (central camera).
 __global__ void __launch_bounds__(256)
 assemble_kernel(const int32_t* __restrict__ m_q, const int32_t* __restrict__ m_t, const int32_t* __restrict__ m_count,
-                const int32_t* __restrict__ q_start, int B, int cap, const float* __restrict__ xyz,
+                const int32_t* __restrict__ q_start, int B, int cap, int views, const float* __restrict__ xyz,
                 const float* __restrict__ b_top, const float* __restrict__ b_bot, float* __restrict__ p_ref,
                 float* __restrict__ p_cur, float* __restrict__ f_cur, uint8_t* __restrict__ cam,
                 int32_t* __restrict__ n_corr, int32_t* __restrict__ n_corr_top) {
   const int i = blockIdx.y;  // frame pair; blockIdx.x: 256 rows of its list (one block per pair left 116 of 148 SMs idle)
-  const int c_top = m_count[i], c_bot = m_count[B + i];
+  const int c_top = m_count[i], c_bot = views == 2 ? m_count[B + i] : 0;
   const int total = c_top + c_bot;
   if (blockIdx.x == 0 && threadIdx.x == 0) {
     n_corr[i] = total;
     n_corr_top[i] = c_top;
   }
-  const int cap2 = 2 * cap;
+  const int cap2 = views * cap;
   for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < total; k += gridDim.x * blockDim.x) {
     const int view = k < c_top ? 0 : 1;
     const int s = view * B + i;
@@ -118,12 +124,12 @@ assemble_kernel(const int32_t* __restrict__ m_q, const int32_t* __restrict__ m_t
       p_cur[o + d] = xyz[(size_t)rq * 3 + d];
       f_cur[o + d] = bq[d];
     }
-    cam[(size_t)i * cap2 + k] = (uint8_t)view;
+    if (cam) cam[(size_t)i * cap2 + k] = (uint8_t)view;
   }
 }
 
-// Store slot `from` -> slot 0 (the tracking reference of what follows).
-__global__ void carry_over_kernel(int B, int from, int cap, float* __restrict__ uv_top, float* __restrict__ uv_bot,
+// Store slot `from` -> slot 0 (the tracking reference of what follows).  views == 1: uv_bot and b_bot are not read.
+__global__ void carry_over_kernel(int B, int from, int cap, int views, float* __restrict__ uv_top, float* __restrict__ uv_bot,
                                   float* __restrict__ b_top, float* __restrict__ b_bot, float* __restrict__ xyz,
                                   uint32_t* __restrict__ desc_c, int32_t* __restrict__ n) {
   const int k = blockIdx.x * blockDim.x + threadIdx.x;
@@ -132,14 +138,14 @@ __global__ void carry_over_kernel(int B, int from, int cap, float* __restrict__ 
   if (k >= cnt) return;
   const size_t src = (size_t)from * cap + k, dst = k;
   ((float2*)uv_top)[dst] = ((const float2*)uv_top)[src];
-  ((float2*)uv_bot)[dst] = ((const float2*)uv_bot)[src];
+  if (views == 2) ((float2*)uv_bot)[dst] = ((const float2*)uv_bot)[src];
 #pragma unroll
   for (int c = 0; c < 3; ++c) {
     b_top[3 * dst + c] = b_top[3 * src + c];
-    b_bot[3 * dst + c] = b_bot[3 * src + c];
+    if (views == 2) b_bot[3 * dst + c] = b_bot[3 * src + c];
     xyz[3 * dst + c] = xyz[3 * src + c];
   }
-  for (int view = 0; view < 2; ++view) {
+  for (int view = 0; view < views; ++view) {
     uint4* base = (uint4*)(desc_c + (size_t)view * (B + 1) * cap * 8);
     base[2 * dst] = base[2 * src];
     base[2 * dst + 1] = base[2 * src + 1];
@@ -251,12 +257,81 @@ detect_pack_kernel(const float2* __restrict__ xy, const int32_t* __restrict__ co
   }
 }
 
+// RGB-D step, store stage (RGBDFrame.establish_keypoints, pose_est_tools.py:600-623): one block per frame b.  Keypoint row
+// k < n_kp[b] (clamped to [0, cap]) is looked up at its truncated pixel (astype(np.uint), :612) and back-projected by
+// rgbd_point, the arithmetic of sos_rgbd_backproject; a pixel outside the map (or a NaN coordinate) drops the keypoint.
+// The valid rows are compacted in row order (kpts[valid], :618-623) into store slot b + 1, tiles of the block as in
+// detect_pack_kernel: float keypoint coordinates (what the |du| gate reads), xyz, bearing, descriptor, input row; n[b + 1].
+constexpr int RS_THREADS = 1024;
+
+__global__ void __launch_bounds__(RS_THREADS)
+rgbd_store_kernel(RgbdP c, const float* __restrict__ depth, int h, int w, const float2* __restrict__ px,
+                  const uint4* __restrict__ desc, const int32_t* __restrict__ n_kp, int cap, double zmin, double zmax,
+                  float2* __restrict__ uv, float* __restrict__ bearing, float* __restrict__ xyz, uint4* __restrict__ desc_c,
+                  int32_t* __restrict__ src, int32_t* __restrict__ n) {
+  __shared__ int s_warp[RS_THREADS / 32];
+  const int b = blockIdx.x;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int rows = min(max(n_kp[b], 0), cap);
+  const float* dmap = depth + (size_t)b * h * w;
+  const size_t in0 = (size_t)b * cap, out0 = (size_t)(b + 1) * cap;
+  int base = 0;
+  for (int k0 = 0; k0 < rows; k0 += RS_THREADS) {
+    const int k = k0 + threadIdx.x;
+    float2 q = make_float2(0.f, 0.f);
+    float p[3], f[3];
+    bool ok = false;
+    if (k < rows) {
+      q = px[in0 + k];
+      const float tx = truncf(q.x), ty = truncf(q.y);
+      if (tx >= 0.f && tx < (float)w && ty >= 0.f && ty < (float)h)   // false for NaN; keeps the int conversion in range
+        ok = rgbd_point(c, dmap, h, w, (int)tx, (int)ty, zmin, zmax, p, f);
+    }
+    const unsigned vote = __ballot_sync(0xFFFFFFFFu, ok);
+    if (lane == 0) s_warp[warp] = __popc(vote);
+    __syncthreads();
+    int before = 0, tile = 0;
+    for (int wi = 0; wi < RS_THREADS / 32; ++wi) {
+      const int cnt = s_warp[wi];
+      if (wi < warp) before += cnt;
+      tile += cnt;
+    }
+    if (ok) {
+      const size_t o = out0 + base + before + __popc(vote & ((1u << lane) - 1u));
+      uv[o] = q;
+#pragma unroll
+      for (int d = 0; d < 3; ++d) {
+        xyz[3 * o + d] = p[d];
+        bearing[3 * o + d] = f[d];
+      }
+      desc_c[2 * o] = desc[2 * (in0 + k)];
+      desc_c[2 * o + 1] = desc[2 * (in0 + k) + 1];
+      src[o] = k;
+    }
+    base += tile;
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) n[b + 1] = base;
+}
+
 }  // namespace
+
+// The inputs of one step, which are also the key of its captured graph: a feature step (omni, px_top, desc_top, boff_top,
+// px_bot, desc_bot, boff_bot), an images-in step (omni; the feature pointers are the front-end's own buffers) or an RGB-D
+// step (depth, px, desc, n_kp).
+enum StepKind { STEP_FEATURES = 0, STEP_IMAGES = 1, STEP_RGBD = 2 };
+struct StepIn {
+  const void* p[7];
+  intptr_t kind;
+};
 
 struct sos_frontend {
   sos_ctx* ctx = nullptr;     // private (own scratch arena)
   sos_ctx* parent = nullptr;  // the caller's context (launch accounting)
-  sos_frontend_config cfg;
+  sos_frontend_config cfg;     // RGB-D: the fields stage B reads (batch, cap = max_kp, RANSAC and refinement, keyframe_mode)
+  bool rgbd = false;           // made by sos_frontend_create_rgbd
+  int views = 2;               // 2 (SOS) or 1 (RGB-D)
+  sos_rgbd_frontend_config rgbd_cfg;
   const sos_lut_entry* lut = nullptr;
   const uint32_t* hyp = nullptr;
   // device state
@@ -265,7 +340,8 @@ struct sos_frontend {
   // staging for the host API (double buffered)
   static constexpr int DEPTH = 2;
   struct Stage {
-    uint8_t* omni = nullptr;
+    uint8_t* omni = nullptr;      // RGB-D: depth maps (float32); px_top / desc_top hold the keypoints
+    int32_t* n_kp = nullptr;      // RGB-D
     float *px_top = nullptr, *px_bot = nullptr;
     uint32_t *desc_top = nullptr, *desc_bot = nullptr;
     int32_t *boff_top = nullptr, *boff_bot = nullptr;
@@ -288,13 +364,9 @@ struct sos_frontend {
   cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
   bool remap_forked = false;
   int next_stage = 0;
-  // graph cache keyed on the input pointers
-  struct GraphKey {
-    const void* p[7];
-    intptr_t images;   // 1: images-in step (its feature pointers are the front-end's own buffers)
-  };
+  // graph cache keyed on the inputs of a step
   struct GraphEntry {
-    GraphKey key;
+    StepIn key;
     cudaGraphExec_t exec = nullptr;
     int launches = 0;
     const void* arena = nullptr;   // fe->ctx->arena at capture
@@ -453,41 +525,44 @@ int enqueue_stage_a(sos_frontend* fe, const uint8_t* omni, const float* px_top, 
 }
 
 // Stage B: temporal matching against the reference slots, RANSAC, refinement.  Re-runnable on its own (sos_frontend_retrack).
+// SOS: two views and the two-mirror rig; RGB-D: one view and a central camera (rig NULL, pyopengv.absolute_pose_ransac).
 int enqueue_stage_b(sos_frontend* fe) {
   sos_ctx* ctx = fe->ctx;
   const sos_frontend_config& c = fe->cfg;
   sos_frontend_buffers& d = fe->d;
-  const int B = c.batch, cap = c.cap;
+  const int B = c.batch, cap = c.cap, V = fe->views, stride = V * cap;
+  const double* rig = V == 2 ? c.rig : nullptr;
+  const int n_cams = V == 2 ? 2 : 0;
   int rc;
-  // step 2b: temporal matching, 2 views x B pairs
-  temporal_segments_kernel<<<sos_div_up(2 * B, 128), 128, 0, ctx->stream>>>(d.n, c.keyframe_mode ? d.ref_slot : nullptr, B, cap,
-                                                                            d.tm_q_start, d.tm_q_len, d.tm_t_start, d.tm_t_len);
+  // step 2b: temporal matching, V views x B pairs
+  temporal_segments_kernel<<<sos_div_up(V * B, 128), 128, 0, ctx->stream>>>(d.n, c.keyframe_mode ? d.ref_slot : nullptr, B, cap,
+                                                                            V, d.tm_q_start, d.tm_q_len, d.tm_t_start, d.tm_t_len);
   SOS_LAUNCHED_AS(ctx, "temporal_segments_kernel");
-  rc = sos_hamming_top2(ctx, d.desc_c, d.desc_c, d.tm_q_start, d.tm_q_len, d.tm_t_start, d.tm_t_len, 2 * B, cap, cap,
+  rc = sos_hamming_top2(ctx, d.desc_c, d.desc_c, d.tm_q_start, d.tm_q_len, d.tm_t_start, d.tm_t_len, V * B, cap, cap,
                         d.tm_idx0, d.tm_d0, nullptr, nullptr);
   if (rc) return rc;
-  // pixel gate on u only (pose_est_tools.py:245-247): coordinates of the compacted store, both views in one array
+  // pixel gate on u only (pose_est_tools.py:245-247): coordinates of the compacted store, all views in one array
   rc = sos_match_select(ctx, SOS_MATCH_NN, 0.75, d.tm_idx0, d.tm_d0, nullptr, nullptr, d.tm_q_start, d.tm_q_len,
-                        d.tm_t_start, 2 * B, d.uv_c, d.uv_c, c.temporal_max_du, -1.0, d.tm_pair_q, d.tm_pair_t, d.tm_pair_d,
+                        d.tm_t_start, V * B, d.uv_c, d.uv_c, c.temporal_max_du, -1.0, d.tm_pair_q, d.tm_pair_t, d.tm_pair_d,
                         d.tm_pair_count);
   if (rc) return rc;
-  assemble_kernel<<<dim3(sos_div_up(2 * cap, 256), B), 256, 0, ctx->stream>>>(d.tm_pair_q, d.tm_pair_t, d.tm_pair_count, d.tm_q_start, B, cap, d.xyz, d.b_top,
+  assemble_kernel<<<dim3(sos_div_up(stride, 256), B), 256, 0, ctx->stream>>>(d.tm_pair_q, d.tm_pair_t, d.tm_pair_count, d.tm_q_start, B, cap, V, d.xyz, d.b_top,
                                               d.b_bot, d.p_ref, d.p_cur, d.f_cur, d.cam, d.n_corr, d.n_corr_top);
   SOS_LAUNCHED_AS(ctx, "assemble_kernel");
   // step 5
   rc = c.solver == SOS_SOLVER_P3P
-           ? sos_ransac_p3p(ctx, d.p_ref, d.f_cur, d.cam, d.n_corr, B, 2 * cap, c.rig, 2, fe->hyp, c.n_hyp, 0, c.ransac_threshold,
+           ? sos_ransac_p3p(ctx, d.p_ref, d.f_cur, d.cam, d.n_corr, B, stride, rig, n_cams, fe->hyp, c.n_hyp, 0, c.ransac_threshold,
                             d.ransac_pose, d.best_hyp, d.best_count, d.inlier_mask, nullptr, nullptr)
-           : sos_ransac_p3d(ctx, d.p_ref, d.p_cur, d.f_cur, d.cam, d.n_corr, B, 2 * cap, c.rig, 2, fe->hyp, c.n_hyp, 0,
+           : sos_ransac_p3d(ctx, d.p_ref, d.p_cur, d.f_cur, d.cam, d.n_corr, B, stride, rig, n_cams, fe->hyp, c.n_hyp, 0,
                             c.score_mode, c.ransac_threshold, d.ransac_pose, d.best_hyp, d.best_count, d.inlier_mask, nullptr,
                             nullptr);
   if (rc) return rc;
   if (c.refit == SOS_REFINE_LM) {
-    rc = sos_refine_pose(ctx, d.p_ref, d.f_cur, d.cam, d.inlier_mask, d.n_corr, B, 2 * cap, c.rig, 2, d.ransac_pose,
+    rc = sos_refine_pose(ctx, d.p_ref, d.f_cur, d.cam, d.inlier_mask, d.n_corr, B, stride, rig, n_cams, d.ransac_pose,
                          c.refine_iters > 0 ? c.refine_iters : 20, 0, d.pose, nullptr, d.refine_stats);
     if (rc) return rc;
   } else if (c.refit == SOS_REFINE_ARUN) {
-    rc = sos_refit_inliers(ctx, d.p_ref, d.p_cur, d.inlier_mask, d.n_corr, B, 2 * cap, d.pose, d.n_refit);
+    rc = sos_refit_inliers(ctx, d.p_ref, d.p_cur, d.inlier_mask, d.n_corr, B, stride, d.pose, d.n_refit);
     if (rc) return rc;
   } else {
     SOS_CUDA(cudaMemcpyAsync(d.pose, d.ransac_pose, (size_t)B * 12 * sizeof(float), cudaMemcpyDeviceToDevice, ctx->stream));
@@ -500,7 +575,7 @@ int enqueue_stage_b(sos_frontend* fe) {
 int enqueue_carry(sos_frontend* fe, int from) {
   sos_ctx* ctx = fe->ctx;
   sos_frontend_buffers& d = fe->d;
-  carry_over_kernel<<<sos_div_up(fe->cfg.cap, 256), 256, 0, ctx->stream>>>(fe->cfg.batch, from, fe->cfg.cap, d.uv_top, d.uv_bot,
+  carry_over_kernel<<<sos_div_up(fe->cfg.cap, 256), 256, 0, ctx->stream>>>(fe->cfg.batch, from, fe->cfg.cap, fe->views, d.uv_top, d.uv_bot,
                                                                             d.b_top, d.b_bot, d.xyz, d.desc_c, d.n);
   SOS_LAUNCHED_AS(ctx, "carry_over_kernel");
   return SOS_OK;
@@ -522,21 +597,58 @@ int enqueue_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, con
   return rc;
 }
 
-// images: an images-in step (the feature pointers are ignored, fe->det.f's are used)
-int run_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top, const int32_t* boff_top,
-             const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot, bool images = false) {
+// RGB-D step: store stage into slots 1..B, stage B, and in consecutive mode the carry-over of slot B.
+int enqueue_rgbd_step(sos_frontend* fe, const float* depth, const float* px, const uint32_t* desc, const int32_t* n_kp) {
   sos_ctx* ctx = fe->ctx;
-  if (images) {
-    const sos_frontend_features& f = fe->det.f;
-    px_top = f.px_top; desc_top = f.desc_top; boff_top = f.boff_top;
-    px_bot = f.px_bot; desc_bot = f.desc_bot; boff_bot = f.boff_bot;
-  }
-  if (!fe->use_graph || ctx->prof) return enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
-  sos_frontend::GraphKey key;
-  memset(&key, 0, sizeof(key));
+  const sos_rgbd_frontend_config& r = fe->rgbd_cfg;
+  sos_frontend_buffers& d = fe->d;
+  RgbdP cam;
+  for (int i = 0; i < SOS_RGBD_NPARAMS; ++i) cam.v[i] = r.cam[i];
+  rgbd_store_kernel<<<r.batch, RS_THREADS, 0, ctx->stream>>>(cam, depth, r.height, r.width, (const float2*)px, (const uint4*)desc,
+                                                              n_kp, r.max_kp, r.min_z, r.max_z, (float2*)d.uv_c, d.b_top, d.xyz,
+                                                              (uint4*)d.desc_c, d.src_top, d.n);
+  SOS_LAUNCHED_AS(ctx, "rgbd_store_kernel");
+  int rc = enqueue_stage_b(fe);
+  if (rc == SOS_OK && !fe->cfg.keyframe_mode) rc = enqueue_carry(fe, fe->cfg.batch);
+  return rc;
+}
+
+int enqueue_any(sos_frontend* fe, const StepIn& in) {
+  const void* const* p = in.p;
+  if (in.kind == STEP_RGBD)
+    return enqueue_rgbd_step(fe, (const float*)p[0], (const float*)p[1], (const uint32_t*)p[2], (const int32_t*)p[3]);
+  return enqueue_step(fe, (const uint8_t*)p[0], (const float*)p[1], (const uint32_t*)p[2], (const int32_t*)p[3],
+                      (const float*)p[4], (const uint32_t*)p[5], (const int32_t*)p[6], in.kind == STEP_IMAGES);
+}
+
+StepIn sos_step_in(const uint8_t* omni, const float* px_top, const uint32_t* desc_top, const int32_t* boff_top,
+                   const float* px_bot, const uint32_t* desc_bot, const int32_t* boff_bot, bool images) {
+  StepIn in;
+  memset(&in, 0, sizeof(in));
   const void* ptrs[7] = {omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot};
-  memcpy(key.p, ptrs, sizeof(ptrs));
-  key.images = images ? 1 : 0;
+  memcpy(in.p, ptrs, sizeof(ptrs));
+  in.kind = images ? STEP_IMAGES : STEP_FEATURES;
+  return in;
+}
+
+StepIn rgbd_step_in(const float* depth, const float* px, const uint32_t* desc, const int32_t* n_kp) {
+  StepIn in;
+  memset(&in, 0, sizeof(in));
+  in.p[0] = depth; in.p[1] = px; in.p[2] = desc; in.p[3] = n_kp;
+  in.kind = STEP_RGBD;
+  return in;
+}
+
+// Eager run, or the captured graph of these inputs (captured after one eager run).  An images-in step's feature pointers
+// are replaced by fe->det.f's.
+int run_step(sos_frontend* fe, StepIn key) {
+  sos_ctx* ctx = fe->ctx;
+  if (key.kind == STEP_IMAGES) {
+    const sos_frontend_features& f = fe->det.f;
+    const void* ptrs[6] = {f.px_top, f.desc_top, f.boff_top, f.px_bot, f.desc_bot, f.boff_bot};
+    memcpy(key.p + 1, ptrs, sizeof(ptrs));
+  }
+  if (!fe->use_graph || ctx->prof) return enqueue_any(fe, key);
   // a graph holds the scratch arena's address: one captured before an eager run regrew the arena must not be replayed
   for (size_t i = 0; i < fe->graphs.size();) {
     if (fe->graphs[i].arena != ctx->arena) {
@@ -555,7 +667,7 @@ int run_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const u
   }
   // first time with these buffers: run once eagerly (sizes the scratch arena), then capture
   const int64_t before = ctx->launches;
-  int rc = enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
+  int rc = enqueue_any(fe, key);
   if (rc) return rc;
   const int launches = (int)(ctx->launches - before);
   fe->d.launches_per_step = launches;
@@ -564,7 +676,7 @@ int run_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const u
   cudaGraph_t graph = nullptr;
   SOS_CUDA(cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
   const int64_t l0 = ctx->launches;
-  rc = enqueue_step(fe, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, images);
+  rc = enqueue_any(fe, key);
   ctx->launches = l0;
   cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
   if (rc) {
@@ -591,22 +703,16 @@ int run_step(sos_frontend* fe, const uint8_t* omni, const float* px_top, const u
 
 }  // namespace
 
-extern "C" int sos_frontend_create(sos_ctx* ctx, const sos_frontend_config* cfg, const sos_lut_entry* lut,
-                                   const uint32_t* hyp, sos_frontend** out) {
-  SOS_CHECK_ARG(ctx && cfg && lut && hyp && out, "NULL argument");
-  SOS_CHECK_ARG(cfg->batch > 0 && cfg->batch <= 4096, "batch out of range");
-  SOS_CHECK_ARG(cfg->channels == 1 || cfg->channels == 3 || cfg->channels == 4, "channels must be 1, 3 or 4");
-  SOS_CHECK_ARG(cfg->n_buckets > 0 && cfg->max_feat_per_view > 0 && cfg->max_feat_per_bucket > 0 && cfg->cap > 0, "bad capacity");
-  SOS_CHECK_ARG(cfg->n_hyp >= 0, "negative n_hyp");
-  SOS_CHECK_ARG(cfg->solver == SOS_SOLVER_ARUN || cfg->solver == SOS_SOLVER_P3P, "unknown solver");
-  SOS_CHECK_ARG(cfg->solver != SOS_SOLVER_P3P || cfg->score_mode == SOS_SCORE_BEARING, "the bearing-only solver scores bearings");
+namespace {
+// A front-end without buffers: private context (same device, but its own scratch arena — the arena address is baked into
+// the captured graphs, so no other caller may regrow it), its own compute stream (the caller's may be the legacy default
+// stream, which cannot be captured; every step is fenced against the caller's current stream with events, so the caller
+// sees ordinary stream semantics) and, for SOS, the remap branch.  On failure everything made so far is destroyed.
+int fe_open(sos_ctx* ctx, bool remap_branch, sos_frontend** out) {
   SOS_CUDA(cudaSetDevice(ctx->device));
   sos_frontend* fe = new sos_frontend();
-  // private context: same device, but its own scratch arena — the arena address is baked into the captured graphs, so
-  // no other caller may regrow it
   fe->ctx = new sos_ctx();
   fe->ctx->device = ctx->device;
-  // every failure below goes through sos_frontend_destroy (streams, events, allocations made so far)
 #define FE_CUDA(call)                                                                               \
   do {                                                                                              \
     cudaError_t e__ = (call);                                                                       \
@@ -616,29 +722,64 @@ extern "C" int sos_frontend_create(sos_ctx* ctx, const sos_frontend_config* cfg,
       return SOS_ERR_CUDA;                                                                          \
     }                                                                                               \
   } while (0)
-  // ... and its own compute stream (the caller's may be the legacy default stream, which cannot be captured); every
-  // step is fenced against the caller's current stream with events, so the caller sees ordinary stream semantics
   int prio_lo = 0, prio_hi = 0;   // (numerically lower = higher priority)
   FE_CUDA(cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
   FE_CUDA(cudaStreamCreateWithPriority(&fe->ctx->stream, cudaStreamNonBlocking, prio_hi));
   fe->ctx->own_stream = true;
   FE_CUDA(cudaEventCreateWithFlags(&fe->ev_in, cudaEventDisableTiming));
   FE_CUDA(cudaEventCreateWithFlags(&fe->ev_out, cudaEventDisableTiming));
-  // lowest priority for the remap branch: the chain's kernels take the SMs they can use first, the remap's blocks fill
-  // what is left (measured: 1.321 -> 1.303 ms per C2 step; shorter remap blocks to free SMs sooner were slower)
-  FE_CUDA(cudaStreamCreateWithPriority(&fe->remap_stream, cudaStreamNonBlocking, prio_lo));
-  FE_CUDA(cudaEventCreateWithFlags(&fe->ev_fork, cudaEventDisableTiming));
-  FE_CUDA(cudaEventCreateWithFlags(&fe->ev_join, cudaEventDisableTiming));
+  if (remap_branch) {
+    // lowest priority for the remap branch: the chain's kernels take the SMs they can use first, the remap's blocks fill
+    // what is left (measured: 1.321 -> 1.303 ms per C2 step; shorter remap blocks to free SMs sooner were slower)
+    FE_CUDA(cudaStreamCreateWithPriority(&fe->remap_stream, cudaStreamNonBlocking, prio_lo));
+    FE_CUDA(cudaEventCreateWithFlags(&fe->ev_fork, cudaEventDisableTiming));
+    FE_CUDA(cudaEventCreateWithFlags(&fe->ev_join, cudaEventDisableTiming));
+  }
+#undef FE_CUDA
   fe->ctx->sm_count = ctx->sm_count;
   fe->parent = ctx;
+  memset(&fe->d, 0, sizeof(fe->d));
+  *out = fe;
+  return SOS_OK;
+}
+
+// The zero fills of fe_alloc were queued on the private stream: finish them before anybody can look at the buffers.
+int fe_finish(sos_frontend* fe, sos_ctx* ctx, int rc, sos_frontend** out) {
+  if (rc == SOS_OK) {
+    cudaError_t e = cudaStreamSynchronize(fe->ctx->stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
+    if (e != cudaSuccess) {
+      sos_set_error("sos_frontend_create: cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
+      rc = SOS_ERR_CUDA;
+    }
+  }
+  if (rc != SOS_OK) {
+    sos_frontend_destroy(fe);
+    return rc;
+  }
+  *out = fe;
+  return SOS_OK;
+}
+}  // namespace
+
+extern "C" int sos_frontend_create(sos_ctx* ctx, const sos_frontend_config* cfg, const sos_lut_entry* lut,
+                                   const uint32_t* hyp, sos_frontend** out) {
+  SOS_CHECK_ARG(ctx && cfg && lut && hyp && out, "NULL argument");
+  SOS_CHECK_ARG(cfg->batch > 0 && cfg->batch <= 4096, "batch out of range");
+  SOS_CHECK_ARG(cfg->channels == 1 || cfg->channels == 3 || cfg->channels == 4, "channels must be 1, 3 or 4");
+  SOS_CHECK_ARG(cfg->n_buckets > 0 && cfg->max_feat_per_view > 0 && cfg->max_feat_per_bucket > 0 && cfg->cap > 0, "bad capacity");
+  SOS_CHECK_ARG(cfg->n_hyp >= 0, "negative n_hyp");
+  SOS_CHECK_ARG(cfg->solver == SOS_SOLVER_ARUN || cfg->solver == SOS_SOLVER_P3P, "unknown solver");
+  SOS_CHECK_ARG(cfg->solver != SOS_SOLVER_P3P || cfg->score_mode == SOS_SCORE_BEARING, "the bearing-only solver scores bearings");
+  sos_frontend* fe = nullptr;
+  int rc = fe_open(ctx, true, &fe);
+  if (rc) return rc;
   fe->cfg = *cfg;
   fe->lut = lut;
   fe->hyp = hyp;
-  memset(&fe->d, 0, sizeof(fe->d));
   const sos_frontend_config& c = fe->cfg;
   const size_t B = c.batch, F = c.max_feat_per_view, cap = c.cap, S = B * c.n_buckets, slots = B + 1;
   sos_frontend_buffers& d = fe->d;
-  int rc = SOS_OK;
 #define FE_ALLOC(field, count) \
   if (rc == SOS_OK) rc = fe_alloc(fe, &d.field, (count))
   FE_ALLOC(pano, B * 2 * c.pano_rows * c.pano_cols * c.channels);
@@ -661,18 +802,62 @@ extern "C" int sos_frontend_create(sos_ctx* ctx, const sos_frontend_config* cfg,
   FE_ALLOC(ransac_pose, B * 12); FE_ALLOC(pose, B * 12); FE_ALLOC(best_hyp, B); FE_ALLOC(best_count, B);
   FE_ALLOC(n_refit, B); FE_ALLOC(inlier_mask, B * 2 * cap); FE_ALLOC(stats, B * 4); FE_ALLOC(refine_stats, B * 4); FE_ALLOC(ref_slot, B); FE_ALLOC(overflow, B);
 #undef FE_ALLOC
-  if (rc != SOS_OK) {
-    sos_frontend_destroy(fe);
-    return rc;
-  }
   d.batch = c.batch;
   d.cap = c.cap;
-  // the zero fills above were queued on the private stream: finish them before anybody can look at the buffers
-  FE_CUDA(cudaStreamSynchronize(fe->ctx->stream));
-  FE_CUDA(cudaStreamSynchronize(ctx->stream));
-#undef FE_CUDA
-  *out = fe;
-  return SOS_OK;
+  d.views = 2;
+  return fe_finish(fe, ctx, rc, out);
+}
+
+extern "C" int sos_frontend_create_rgbd(sos_ctx* ctx, const sos_rgbd_frontend_config* cfg, const uint32_t* hyp,
+                                        sos_frontend** out) {
+  SOS_CHECK_ARG(ctx && cfg && hyp && out, "NULL argument");
+  SOS_CHECK_ARG(cfg->batch > 0 && cfg->batch <= 4096, "batch out of range");
+  SOS_CHECK_ARG(cfg->height > 0 && cfg->width > 0 && (long long)cfg->height * cfg->width < (1ll << 31), "bad depth map size");
+  SOS_CHECK_ARG(cfg->max_kp > 0 && (long long)(cfg->batch + 1) * cfg->max_kp < (1ll << 31), "bad max_kp");
+  SOS_CHECK_ARG(cfg->n_hyp >= 0, "negative n_hyp");
+  SOS_CHECK_ARG(cfg->solver == SOS_SOLVER_ARUN || cfg->solver == SOS_SOLVER_P3P, "unknown solver");
+  SOS_CHECK_ARG(cfg->refit == SOS_REFINE_NONE || cfg->refit == SOS_REFINE_ARUN || cfg->refit == SOS_REFINE_LM, "unknown refit");
+  sos_frontend* fe = nullptr;
+  int rc = fe_open(ctx, false, &fe);
+  if (rc) return rc;
+  fe->rgbd = true;
+  fe->views = 1;
+  fe->rgbd_cfg = *cfg;
+  fe->hyp = hyp;
+  // what stage B, the keyframe calls and the host path read
+  sos_frontend_config& c = fe->cfg;
+  memset(&c, 0, sizeof(c));
+  c.batch = cfg->batch;
+  c.cap = cfg->max_kp;
+  c.n_hyp = cfg->n_hyp;
+  c.score_mode = SOS_SCORE_BEARING;
+  c.refit = cfg->refit;
+  c.refine_iters = cfg->refine_iters;
+  c.keyframe_mode = cfg->keyframe_mode;
+  c.solver = cfg->solver;
+  c.ransac_threshold = cfg->ransac_threshold;
+  c.temporal_max_du = cfg->temporal_max_du;
+  const size_t B = c.batch, cap = c.cap, slots = B + 1;
+  sos_frontend_buffers& d = fe->d;
+#define FE_ALLOC(field, count) \
+  if (rc == SOS_OK) rc = fe_alloc(fe, &d.field, (count))
+  FE_ALLOC(uv_c, slots * cap * 2);
+  d.uv_top = d.uv_c;
+  FE_ALLOC(b_top, slots * cap * 3); FE_ALLOC(xyz, slots * cap * 3); FE_ALLOC(src_top, slots * cap); FE_ALLOC(n, slots);
+  FE_ALLOC(desc_c, slots * cap * 8);
+  FE_ALLOC(tm_q_start, B); FE_ALLOC(tm_q_len, B); FE_ALLOC(tm_t_start, B); FE_ALLOC(tm_t_len, B);
+  FE_ALLOC(tm_idx0, slots * cap); FE_ALLOC(tm_d0, slots * cap);
+  FE_ALLOC(tm_pair_q, slots * cap); FE_ALLOC(tm_pair_t, slots * cap); FE_ALLOC(tm_pair_d, slots * cap);
+  FE_ALLOC(tm_pair_count, B);
+  FE_ALLOC(p_ref, B * cap * 3); FE_ALLOC(p_cur, B * cap * 3); FE_ALLOC(f_cur, B * cap * 3);
+  FE_ALLOC(n_corr, B); FE_ALLOC(n_corr_top, B);
+  FE_ALLOC(ransac_pose, B * 12); FE_ALLOC(pose, B * 12); FE_ALLOC(best_hyp, B); FE_ALLOC(best_count, B);
+  FE_ALLOC(n_refit, B); FE_ALLOC(inlier_mask, B * cap); FE_ALLOC(stats, B * 4); FE_ALLOC(refine_stats, B * 4); FE_ALLOC(ref_slot, B);
+#undef FE_ALLOC
+  d.batch = c.batch;
+  d.cap = c.cap;
+  d.views = 1;
+  return fe_finish(fe, ctx, rc, out);
 }
 
 extern "C" int sos_frontend_destroy(sos_frontend* fe) {
@@ -778,16 +963,17 @@ extern "C" int sos_frontend_get_buffers(sos_frontend* fe, sos_frontend_buffers* 
   return SOS_OK;
 }
 
+#define SOS_CHECK_SOS(fe) SOS_CHECK_ARG(!(fe)->rgbd, "not available on an RGB-D front-end")
+#define SOS_CHECK_RGBD(fe) SOS_CHECK_ARG((fe)->rgbd, "needs an RGB-D front-end (sos_frontend_create_rgbd)")
+
 namespace {
-int step_device(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top,
-                const int32_t* bucket_off_top, const float* px_bot, const uint32_t* desc_bot, const int32_t* bucket_off_bot,
-                bool images) {
+int step_device(sos_frontend* fe, const StepIn& in) {
   SOS_CUDA(cudaSetDevice(fe->ctx->device));
   // inputs were produced on the caller's stream; results must be visible to it afterwards
   SOS_CUDA(cudaEventRecord(fe->ev_in, fe->parent->stream));
   SOS_CUDA(cudaStreamWaitEvent(fe->ctx->stream, fe->ev_in, 0));
   const int64_t before = fe->ctx->launches;
-  const int rc = run_step(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, images);
+  const int rc = run_step(fe, in);
   fe->parent->launches += fe->ctx->launches - before;
   if (rc) return rc;
   SOS_CUDA(cudaEventRecord(fe->ev_out, fe->ctx->stream));
@@ -800,13 +986,23 @@ extern "C" int sos_frontend_step(sos_frontend* fe, const uint8_t* omni, const fl
                                  const int32_t* bucket_off_top, const float* px_bot, const uint32_t* desc_bot,
                                  const int32_t* bucket_off_bot) {
   SOS_CHECK_ARG(fe, "fe is NULL");
+  SOS_CHECK_SOS(fe);
   SOS_CHECK_ARG(omni && px_top && desc_top && bucket_off_top && px_bot && desc_bot && bucket_off_bot, "NULL input");
-  return step_device(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, false);
+  return step_device(fe, sos_step_in(omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, false));
+}
+
+extern "C" int sos_frontend_step_rgbd(sos_frontend* fe, const float* depth, const float* px, const uint32_t* desc,
+                                      const int32_t* n_kp) {
+  SOS_CHECK_ARG(fe, "fe is NULL");
+  SOS_CHECK_RGBD(fe);
+  SOS_CHECK_ARG(depth && px && desc && n_kp, "NULL input");
+  return step_device(fe, rgbd_step_in(depth, px, desc, n_kp));
 }
 
 extern "C" int sos_frontend_set_detector(sos_frontend* fe, const sos_detect_config* dcfg, const uint8_t* masks_top,
                                          const uint8_t* masks_bot) {
   SOS_CHECK_ARG(fe && dcfg, "NULL argument");
+  SOS_CHECK_SOS(fe);
   SOS_CHECK_ARG(masks_top && masks_bot, "NULL masks");
   const sos_frontend_config& c = fe->cfg;
   if (c.channels != 3 || c.n_buckets > 32) {
@@ -866,7 +1062,7 @@ extern "C" int sos_frontend_set_detector(sos_frontend* fe, const sos_detect_conf
   dt.on = true;
   // captured images-in steps bake the previous detector's parameters in
   for (size_t i = 0; i < fe->graphs.size();) {
-    if (fe->graphs[i].key.images) {
+    if (fe->graphs[i].key.kind == STEP_IMAGES) {
       cudaGraphExecDestroy(fe->graphs[i].exec);
       fe->graphs.erase(fe->graphs.begin() + i);
     } else {
@@ -878,12 +1074,14 @@ extern "C" int sos_frontend_set_detector(sos_frontend* fe, const sos_detect_conf
 
 extern "C" int sos_frontend_step_images(sos_frontend* fe, const uint8_t* omni) {
   SOS_CHECK_ARG(fe && omni, "NULL argument");
+  SOS_CHECK_SOS(fe);
   SOS_CHECK_ARG(fe->det.on, "no detector: call sos_frontend_set_detector first");
-  return step_device(fe, omni, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, true);
+  return step_device(fe, sos_step_in(omni, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, true));
 }
 
 extern "C" int sos_frontend_get_features(sos_frontend* fe, sos_frontend_features* out) {
   SOS_CHECK_ARG(fe && out, "NULL argument");
+  SOS_CHECK_SOS(fe);
   SOS_CHECK_ARG(fe->det.on, "no detector: call sos_frontend_set_detector first");
   *out = fe->det.f;
   return SOS_OK;
@@ -894,6 +1092,22 @@ static int ensure_staging(sos_frontend* fe) {
   const sos_frontend_config& c = fe->cfg;
   const size_t B = c.batch, F = c.max_feat_per_view;
   SOS_CUDA(cudaStreamCreateWithFlags(&fe->copy_stream, cudaStreamNonBlocking));
+  if (fe->rgbd) {   // whole depth maps, keypoints, descriptors and counts
+    const sos_rgbd_frontend_config& r = fe->rgbd_cfg;
+    for (auto& s : fe->stage) {
+      int rc = fe_alloc(fe, &s.omni, B * r.height * r.width * sizeof(float));
+      if (!rc) rc = fe_alloc(fe, &s.px_top, B * r.max_kp * 2);
+      if (!rc) rc = fe_alloc(fe, &s.desc_top, B * r.max_kp * 8);
+      if (!rc) rc = fe_alloc(fe, &s.n_kp, B);
+      if (rc) return rc;
+      SOS_CUDA(cudaMallocHost((void**)&s.h_poses, B * 12 * sizeof(float)));
+      SOS_CUDA(cudaMallocHost((void**)&s.h_stats, B * 4 * sizeof(int32_t)));
+      SOS_CUDA(cudaEventCreateWithFlags(&s.copied, cudaEventDisableTiming));
+      SOS_CUDA(cudaEventCreateWithFlags(&s.done, cudaEventDisableTiming));
+    }
+    SOS_CUDA(cudaStreamSynchronize(fe->ctx->stream));
+    return SOS_OK;
+  }
   for (auto& s : fe->stage) {
     int rc = fe_alloc(fe, &s.omni, B * c.src_h * c.src_w * c.channels);
     if (!rc) rc = fe_alloc(fe, &s.px_top, B * F * 2);
@@ -966,17 +1180,21 @@ extern "C" int sos_frontend_host_bytes(sos_frontend* fe, int64_t* h2d_bytes_per_
   if (rc) return rc;
   const sos_frontend_config& c = fe->cfg;
   const int64_t B = c.batch, F = c.max_feat_per_view;
-  if (h2d_bytes_per_step)
+  if (h2d_bytes_per_step && fe->rgbd) {
+    const sos_rgbd_frontend_config& r = fe->rgbd_cfg;
+    *h2d_bytes_per_step = B * ((int64_t)r.height * r.width * 4 + (int64_t)r.max_kp * (2 * 4 + 32) + 4);
+  } else if (h2d_bytes_per_step) {
     *h2d_bytes_per_step = B * (fe->omni_bytes_per_frame + 2 * F * 2 * 4 + 2 * F * 32 + 2 * (c.n_buckets + 1) * 4);
+  }
   if (d2h_bytes_per_step) *d2h_bytes_per_step = B * (12 * 4 + 4 * 4);
   return SOS_OK;
 }
 
 namespace {
 // H2D of one step's inputs on the copy stream (so that it overlaps the kernels of the previous step), the step, and the
-// D2H of poses and stats.  images: only the omni images are uploaded and the features are detected on the device.
-int submit(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uint32_t* desc_top, const int32_t* bucket_off_top,
-           const float* px_bot, const uint32_t* desc_bot, const int32_t* bucket_off_bot, bool images, int* ticket) {
+// D2H of poses and stats.  in: HOST pointers; images-in step: only the omni images are uploaded and the features are
+// detected on the device; RGB-D step: whole depth maps, then keypoints, descriptors and counts.
+int submit(sos_frontend* fe, const StepIn& in, int* ticket) {
   SOS_CUDA(cudaSetDevice(fe->ctx->device));
   int rc = ensure_staging(fe);
   if (rc) return rc;
@@ -989,7 +1207,20 @@ int submit(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uin
   const sos_frontend_config& c = fe->cfg;
   const size_t B = c.batch, F = c.max_feat_per_view;
   cudaStream_t cs = fe->copy_stream;
-  if (fe->bands.empty()) {
+  const bool images = in.kind == STEP_IMAGES;
+  const uint8_t* omni = (const uint8_t*)in.p[0];
+  const float *px_top = (const float*)in.p[1], *px_bot = (const float*)in.p[4];
+  const uint32_t *desc_top = (const uint32_t*)in.p[2], *desc_bot = (const uint32_t*)in.p[5];
+  const int32_t *bucket_off_top = (const int32_t*)in.p[3], *bucket_off_bot = (const int32_t*)in.p[6];
+  StepIn dev;
+  if (in.kind == STEP_RGBD) {
+    const sos_rgbd_frontend_config& r = fe->rgbd_cfg;
+    SOS_CUDA(cudaMemcpyAsync(s.omni, in.p[0], B * r.height * r.width * sizeof(float), cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.px_top, in.p[1], B * r.max_kp * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.desc_top, in.p[2], B * r.max_kp * 32, cudaMemcpyHostToDevice, cs));
+    SOS_CUDA(cudaMemcpyAsync(s.n_kp, in.p[3], B * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
+    dev = rgbd_step_in((const float*)s.omni, s.px_top, s.desc_top, s.n_kp);
+  } else if (fe->bands.empty()) {
     SOS_CUDA(cudaMemcpyAsync(s.omni, omni, B * c.src_h * c.src_w * c.channels, cudaMemcpyHostToDevice, cs));
   } else {
     // one strided copy per band of rows, covering that band in every frame of the batch (depth = frames)
@@ -1005,7 +1236,7 @@ int submit(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uin
       SOS_CUDA(cudaMemcpy3DAsync(&p, cs));
     }
   }
-  if (!images) {
+  if (in.kind == STEP_FEATURES) {
     SOS_CUDA(cudaMemcpyAsync(s.px_top, px_top, B * F * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
     SOS_CUDA(cudaMemcpyAsync(s.px_bot, px_bot, B * F * 2 * sizeof(float), cudaMemcpyHostToDevice, cs));
     SOS_CUDA(cudaMemcpyAsync(s.desc_top, desc_top, B * F * 32, cudaMemcpyHostToDevice, cs));
@@ -1013,10 +1244,11 @@ int submit(sos_frontend* fe, const uint8_t* omni, const float* px_top, const uin
     SOS_CUDA(cudaMemcpyAsync(s.boff_top, bucket_off_top, B * (c.n_buckets + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
     SOS_CUDA(cudaMemcpyAsync(s.boff_bot, bucket_off_bot, B * (c.n_buckets + 1) * sizeof(int32_t), cudaMemcpyHostToDevice, cs));
   }
+  if (in.kind != STEP_RGBD) dev = sos_step_in(s.omni, s.px_top, s.desc_top, s.boff_top, s.px_bot, s.desc_bot, s.boff_bot, images);
   SOS_CUDA(cudaEventRecord(s.copied, cs));
   SOS_CUDA(cudaStreamWaitEvent(fe->ctx->stream, s.copied, 0));
   const int64_t before = fe->ctx->launches;
-  rc = run_step(fe, s.omni, s.px_top, s.desc_top, s.boff_top, s.px_bot, s.desc_bot, s.boff_bot, images);
+  rc = run_step(fe, dev);
   fe->parent->launches += fe->ctx->launches - before;
   if (rc) return rc;
   SOS_CUDA(cudaMemcpyAsync(s.h_poses, fe->d.pose, B * 12 * sizeof(float), cudaMemcpyDeviceToHost, fe->ctx->stream));
@@ -1034,14 +1266,25 @@ extern "C" int sos_frontend_submit_host(sos_frontend* fe, const uint8_t* omni, c
                                         const uint32_t* desc_top, const int32_t* bucket_off_top, const float* px_bot,
                                         const uint32_t* desc_bot, const int32_t* bucket_off_bot, int* ticket) {
   SOS_CHECK_ARG(fe && ticket, "NULL argument");
+  SOS_CHECK_SOS(fe);
   SOS_CHECK_ARG(omni && px_top && desc_top && bucket_off_top && px_bot && desc_bot && bucket_off_bot, "NULL input");
-  return submit(fe, omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, false, ticket);
+  return submit(fe, sos_step_in(omni, px_top, desc_top, bucket_off_top, px_bot, desc_bot, bucket_off_bot, false), ticket);
+}
+
+extern "C" int sos_frontend_submit_host_rgbd(sos_frontend* fe, const float* depth, const float* px, const uint32_t* desc,
+                                             const int32_t* n_kp, int* ticket) {
+  SOS_CHECK_ARG(fe && ticket, "NULL argument");
+  SOS_CHECK_RGBD(fe);
+  SOS_CHECK_ARG(depth && px && desc && n_kp, "NULL input");
+  for (int b = 0; b < fe->cfg.batch; ++b) SOS_CHECK_ARG(n_kp[b] >= 0 && n_kp[b] <= fe->rgbd_cfg.max_kp, "n_kp outside [0, max_kp]");
+  return submit(fe, rgbd_step_in(depth, px, desc, n_kp), ticket);
 }
 
 extern "C" int sos_frontend_submit_host_images(sos_frontend* fe, const uint8_t* omni, int* ticket) {
   SOS_CHECK_ARG(fe && ticket && omni, "NULL argument");
+  SOS_CHECK_SOS(fe);
   SOS_CHECK_ARG(fe->det.on, "no detector: call sos_frontend_set_detector first");
-  return submit(fe, omni, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, true, ticket);
+  return submit(fe, sos_step_in(omni, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, true), ticket);
 }
 
 extern "C" int sos_frontend_wait_host(sos_frontend* fe, int ticket, float* poses, int32_t* stats) {

@@ -6,6 +6,7 @@
 // where the hot path stores them (pixel coordinates are float32 cv2.KeyPoint.pt values, so nothing is lost on input).
 #include <math_constants.h>
 
+#include "rgbd.cuh"
 #include "sos_common.cuh"
 
 namespace {
@@ -399,18 +400,7 @@ __global__ void lift_gum_kernel(GumP g, const double* __restrict__ uv, int n, do
   if (el) el[i] = asin(sz);
 }
 
-// ---- F12: RGB-D, camera_models.py:781-799, 835-860, 203-212; pose_est_tools.py:612-620 ------------------------
-struct RgbdP {
-  double v[SOS_RGBD_NPARAMS];
-};
-
-__device__ __forceinline__ double rgbd_depth_z(const RgbdP& c, double d, double u, double v) {
-  if (c.v[SOS_RGBD_DEPTH_IS_Z] != 0.0) return d;
-  const double f = c.v[SOS_RGBD_FOCAL_M];
-  const double xi = (f / c.v[SOS_RGBD_FX]) * (u - c.v[SOS_RGBD_CX]);
-  const double yi = (f / c.v[SOS_RGBD_FY]) * (v - c.v[SOS_RGBD_CY]);
-  return f * d / sqrt(xi * xi + yi * yi + f * f);
-}
+// ---- F12: RGB-D, camera_models.py:781-799, 835-860, 203-212; pose_est_tools.py:612-620 (rgbd.cuh) -------------
 
 // One thread per pixel position, looping over the frames: the double-precision square root of the radial model depends on
 // (x, y) only, so it is taken once per thread and the per-frame work is one multiply and one divide (first version: sqrt and
@@ -441,27 +431,13 @@ __global__ void rgbd_backproject_kernel(RgbdP c, const float* __restrict__ depth
   if (i >= n) return;
   const int b = blockIdx.y;
   const size_t o = (size_t)b * n + i;
-  const int u = us[o], v = vs[o];
-  double Z = CUDART_NAN;
-  if (u >= 0 && u < w && v >= 0 && v < h) {
-    const double d = (double)depth[((size_t)b * h + v) * w + u];
-    const double zz = rgbd_depth_z(c, d, (double)u, (double)v);
-    if (zz != 0.0) Z = zz;  // camera_models.py:846: zero depth -> NaN
-  }
-  const double X = ((double)u - c.v[SOS_RGBD_CX]) * Z / c.v[SOS_RGBD_FX];
-  const double Y = ((double)v - c.v[SOS_RGBD_CY]) * Z / c.v[SOS_RGBD_FY];
-  const double nrm = sqrt(X * X + Y * Y + Z * Z);
-  xyz[3 * o] = (float)X; xyz[3 * o + 1] = (float)Y; xyz[3 * o + 2] = (float)Z;
+  float p[3], f[3];
+  const bool ok = rgbd_point(c, depth + (size_t)b * h * w, h, w, us[o], vs[o], zmin, zmax, p, f);
+  xyz[3 * o] = p[0]; xyz[3 * o + 1] = p[1]; xyz[3 * o + 2] = p[2];
   if (bearing) {
-    bearing[3 * o] = (float)(X / nrm); bearing[3 * o + 1] = (float)(Y / nrm); bearing[3 * o + 2] = (float)(Z / nrm);
+    bearing[3 * o] = f[0]; bearing[3 * o + 1] = f[1]; bearing[3 * o + 2] = f[2];
   }
-  if (valid) {
-    bool ok = !isnan(Z);
-    const double az = fabs(Z);  // pose_est_tools.py:570-592 gates |Z| (norm over a length-1 axis)
-    if (zmin > 0.0) ok = ok && az >= zmin;
-    if (zmax > 0.0) ok = ok && az <= zmax;
-    valid[o] = ok ? 1 : 0;
-  }
+  if (valid) valid[o] = ok ? 1 : 0;
 }
 
 static GumP load_gum(const double* g) {

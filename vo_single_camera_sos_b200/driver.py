@@ -7,6 +7,8 @@ the current keyframe in one captured kernel chain; the host then walks the batch
 keyframe policy.  When frame j becomes a keyframe, its store slot is promoted on the device and only stage B (temporal
 matching, RANSAC, refinement) is re-run for the frames after j — their remap / stereo matching / triangulation is
 reused.  The sequence of poses and keyframes is the one the sequential loop produces.
+
+The same driver runs the RGB-D front-end (an RgbdFrontendConfig): one camera, depth maps and keypoints per frame.
 """
 from __future__ import annotations
 
@@ -20,9 +22,10 @@ import numpy as np
 import torch
 
 from . import ops
-from .frontend import Frontend, FrontendConfig
+from .frontend import Frontend, FrontendConfig, RgbdFrontendConfig
 
 INPUT_KEYS = ("omni", "px_top", "desc_top", "boff_top", "px_bot", "desc_bot", "boff_bot")
+RGBD_INPUT_KEYS = ("depth", "px", "desc", "n_kp")
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -166,30 +169,45 @@ class TrackingState:
 # ---------------------------------------------------------------------------------------------------------------------
 # the batched driver
 # ---------------------------------------------------------------------------------------------------------------------
-class BatchedVO:
-    """frames: sequence of per-frame dicts with the front-end's inputs for ONE frame each
-    (omni [H,W,C] u8, px_* [F,2] f32, desc_* [F,32] u8, boff_* [n_buckets+1] i32)."""
+def frontend_layout(cfg):
+    """What the driver takes from the kind of front-end: (input keys, {key: (batch shape, dtype)}, number_of_cams,
+    default minimum of correspondences).  The trackers refuse fewer than 2 * 3 * 0.33 * 2 (TrackerStereoSE3,
+    pose_est_tools.py:779-781) or 2 * 3 * 1 (TrackerRGBDSE3.track_frame) correspondences."""
+    c = cfg
+    if isinstance(cfg, RgbdFrontendConfig):
+        return RGBD_INPUT_KEYS, {
+            "depth": ((c.batch, c.height, c.width), torch.float32),
+            "px": ((c.batch, c.max_kp, 2), torch.float32),
+            "desc": ((c.batch, c.max_kp, 32), torch.uint8),
+            "n_kp": ((c.batch,), torch.int32),
+        }, 1, 2 * 3 * 1
+    return INPUT_KEYS, {
+        "omni": ((c.batch, c.src_h, c.src_w, c.channels), torch.uint8),
+        "px_top": ((c.batch, c.max_feat_per_view, 2), torch.float32),
+        "px_bot": ((c.batch, c.max_feat_per_view, 2), torch.float32),
+        "desc_top": ((c.batch, c.max_feat_per_view, 32), torch.uint8),
+        "desc_bot": ((c.batch, c.max_feat_per_view, 32), torch.uint8),
+        "boff_top": ((c.batch, c.n_buckets + 1), torch.int32),
+        "boff_bot": ((c.batch, c.n_buckets + 1), torch.int32),
+    }, 2, 2 * 3 * (0.33 * 2)
 
-    def __init__(self, ctx: ops.Context, cfg: FrontendConfig, lut: torch.Tensor, hyp: torch.Tensor,
+
+class BatchedVO:
+    """frames: sequence of per-frame dicts with the front-end's inputs for ONE frame each: SOS (FrontendConfig)
+    omni [H,W,C] u8, px_* [F,2] f32, desc_* [F,32] u8, boff_* [n_buckets+1] i32; RGB-D (RgbdFrontendConfig, lut None)
+    depth [height,width] f32, px [max_kp,2] f32, desc [max_kp,32] u8, n_kp (int)."""
+
+    def __init__(self, ctx: ops.Context, cfg, lut: Optional[torch.Tensor], hyp: torch.Tensor,
                  policy: Optional[KeyframePolicy] = None, units_to_m: float = 1.0, min_correspondences: Optional[int] = None):
         if not cfg.keyframe_mode:
-            raise ValueError("BatchedVO needs a FrontendConfig with keyframe_mode=True")
+            raise ValueError("BatchedVO needs a front-end configuration with keyframe_mode=True")
         self.ctx, self.cfg = ctx, cfg
         self.fe = Frontend(ctx, cfg, lut, hyp)
         self.policy = policy or KeyframePolicy()
         self.units_to_m = units_to_m
-        # TrackerStereoSE3.track_frame refuses fewer than 2 * 3 * 0.33 * 2 correspondences (pose_est_tools.py:779-781)
-        self.min_correspondences = 2 * 3 * (0.33 * 2) if min_correspondences is None else min_correspondences
-        c = cfg
-        shapes = {
-            "omni": ((c.batch, c.src_h, c.src_w, c.channels), torch.uint8),
-            "px_top": ((c.batch, c.max_feat_per_view, 2), torch.float32),
-            "px_bot": ((c.batch, c.max_feat_per_view, 2), torch.float32),
-            "desc_top": ((c.batch, c.max_feat_per_view, 32), torch.uint8),
-            "desc_bot": ((c.batch, c.max_feat_per_view, 32), torch.uint8),
-            "boff_top": ((c.batch, c.n_buckets + 1), torch.int32),
-            "boff_bot": ((c.batch, c.n_buckets + 1), torch.int32),
-        }
+        self.input_keys, shapes, self.number_of_cams, default_min = frontend_layout(cfg)
+        self._step = self.fe.step_rgbd if isinstance(cfg, RgbdFrontendConfig) else self.fe.step
+        self.min_correspondences = default_min if min_correspondences is None else min_correspondences
         # pinned staging (one batch) + its device twin; frames are packed into the staging arrays on the host
         # two sets, so that the next batch is packed while the current one is copied, tracked and resolved
         self._pinned = [{k: torch.zeros(shape, dtype=dt).pin_memory() for k, (shape, dt) in shapes.items()} for _ in range(2)]
@@ -210,12 +228,12 @@ class BatchedVO:
         host = self._host[s]
 
         def pack(i):                        # numpy copies release the GIL
-            for k in INPUT_KEYS:
+            for k in self.input_keys:
                 host[k][i] = frames[i][k]
         # packing a batch of images is the driver's largest host cost (118 MB per 32 C1 frames): spread it over the cores
         list(self._pool.map(pack, range(len(frames))))
         if len(frames) < B:
-            for k in INPUT_KEYS:
+            for k in self.input_keys:
                 host[k][len(frames):] = 0   # unused slots: empty frames (no features -> no work after the remap)
 
     def _predict(self, i0: int, chain: bool, token: int):
@@ -233,7 +251,7 @@ class BatchedVO:
         return refs, assume
 
     def _h2d(self, s: int):
-        for k in INPUT_KEYS:
+        for k in self.input_keys:
             self._dev[s][k].copy_(self._pinned[s][k], non_blocking=True)
 
     def _read(self):
@@ -246,7 +264,7 @@ class BatchedVO:
         frames = list(frames)
         ids = list(range(len(frames))) if frame_ids is None else list(frame_ids)
         B = self.cfg.batch
-        state = TrackingState(self.policy, 2, self.units_to_m)
+        state = TrackingState(self.policy, self.number_of_cams, self.units_to_m)
         res = state.result
         self.fe.reset()
         nxt = 0                                   # next frame to resolve
@@ -271,7 +289,7 @@ class BatchedVO:
             else:
                 refs, assume = self._predict(0, chain, token)
             self.fe.set_ref_slots(refs)
-            self.fe.step(*[self._dev[cur][k] for k in INPUT_KEYS])
+            self._step(*[self._dev[cur][k] for k in self.input_keys])
             res.device_steps += 1
             pose, stats, n_slots = self._read()
             i = 0

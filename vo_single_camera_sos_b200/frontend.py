@@ -2,8 +2,9 @@
 
 `Frontend.step(...)` takes device tensors, `Frontend.step_host(...)` / `submit_host` + `wait_host` take pinned host
 arrays (the end-to-end path: H2D, kernels, D2H).  After `set_detector(...)`, `step_images` / `step_host_images` take the
-omni images alone and detect the features inside the step.  All data-dependent sizes stay on the device; see
-csrc/frontend.cu.
+omni images alone and detect the features inside the step.  A `Frontend` made from an `RgbdFrontendConfig` is the RGB-D
+front-end (BASELINE configuration 5): `step_rgbd` / `step_host_rgbd` take depth maps and keypoints.  All data-dependent
+sizes stay on the device; see csrc/frontend.cu.
 """
 from __future__ import annotations
 
@@ -49,7 +50,50 @@ _BUF_FIELDS = [
 
 class _Buffers(C.Structure):
     _fields_ = [(name, C.c_void_p) for name, _ in _BUF_FIELDS] + [
-        ("batch", C.c_int32), ("cap", C.c_int32), ("launches_per_step", C.c_int32)]
+        ("batch", C.c_int32), ("cap", C.c_int32), ("launches_per_step", C.c_int32), ("views", C.c_int32)]
+
+
+class _RgbdConfig(C.Structure):
+    _fields_ = [
+        ("batch", C.c_int32), ("height", C.c_int32), ("width", C.c_int32), ("max_kp", C.c_int32), ("n_hyp", C.c_int32),
+        ("solver", C.c_int32), ("refit", C.c_int32), ("refine_iters", C.c_int32), ("keyframe_mode", C.c_int32),
+        ("cam", C.c_double * len(ops.RGBD_FIELDS)), ("min_z", C.c_double), ("max_z", C.c_double),
+        ("temporal_max_du", C.c_double), ("ransac_threshold", C.c_double),
+    ]
+
+
+@dataclass
+class RgbdFrontendConfig:
+    """The RGB-D front-end (sos_rgbd_frontend_config); defaults follow RGBDFrame / TrackerRGBDSE3
+    (pose_est_tools.py:429-430, 672-707, 880-958)."""
+    batch: int
+    cam: Sequence[float]               # ops.RGBD_FIELDS order: fx, fy, center_x, center_y, focal_length_m, depth_is_Z
+    height: int = 480
+    width: int = 640
+    max_kp: int = 2000                 # keypoint rows per frame, and the store capacity
+    n_hyp: int = 210
+    solver: int = 0                    # ops.SOLVER_ARUN (hyp [n_hyp,3]) / ops.SOLVER_P3P (hyp [n_hyp,4])
+    refit: int = 2                     # ops.REFINE_LM: the tracker's absolute_pose_optimize_nonlinear
+    refine_iters: int = 0              # REFINE_LM: maximum cost evaluations (0 -> 20)
+    keyframe_mode: bool = False
+    min_z: float = 0.8
+    max_z: float = 7.0
+    temporal_max_du: Optional[float] = None    # None -> 0.5 * 2 * center_x (pose_est_tools.py:958)
+    ransac_threshold: float = 1.0 - math.cos(math.radians(5.0))
+
+    def to_c(self) -> _RgbdConfig:
+        c = _RgbdConfig()
+        for k in ("batch", "height", "width", "max_kp", "n_hyp", "solver", "refit", "refine_iters"):
+            setattr(c, k, int(getattr(self, k)))
+        c.keyframe_mode = int(bool(self.keyframe_mode))
+        cam = [float(x) for x in self.cam]
+        if len(cam) != len(ops.RGBD_FIELDS):
+            raise ValueError(f"cam must hold {len(ops.RGBD_FIELDS)} values ({', '.join(ops.RGBD_FIELDS)})")
+        c.cam[:] = cam
+        c.min_z, c.max_z = float(self.min_z), float(self.max_z)
+        c.temporal_max_du = float(0.5 * 2.0 * cam[2] if self.temporal_max_du is None else self.temporal_max_du)
+        c.ransac_threshold = float(self.ransac_threshold)
+        return c
 
 
 @dataclass
@@ -143,21 +187,33 @@ _TYPES = {"u8": ("|u1", torch.uint8), "i32": ("<i4", torch.int32), "f32": ("<f4"
 
 
 class Frontend:
-    def __init__(self, ctx: ops.Context, cfg: FrontendConfig, lut: torch.Tensor, hyp: torch.Tensor):
-        """lut [2, rows, cols] int64 (packed LUT of the top and bottom view); hyp [n_hyp, 3] int32 (uint32 bits; [n_hyp, 4] for SOLVER_P3P)."""
+    def __init__(self, ctx: ops.Context, cfg, lut: Optional[torch.Tensor], hyp: torch.Tensor):
+        """SOS (cfg: FrontendConfig): lut [2, rows, cols] int64 (packed LUT of the top and bottom view).  RGB-D (cfg:
+        RgbdFrontendConfig): lut is None.  hyp [n_hyp, 3] int32 (uint32 bits; [n_hyp, 4] for SOLVER_P3P)."""
         self.ctx, self.cfg = ctx, cfg
+        self.rgbd = isinstance(cfg, RgbdFrontendConfig)
         ctx._sync_stream()
-        if tuple(lut.shape) != (2, cfg.pano_rows, cfg.pano_cols):
+        if self.rgbd:
+            if lut is not None:
+                raise ValueError("the RGB-D front-end takes no LUT")
+        elif tuple(lut.shape) != (2, cfg.pano_rows, cfg.pano_cols):
             raise ValueError("lut must be [2, pano_rows, pano_cols]")
         if hyp.shape[0] != cfg.n_hyp or hyp.shape[1] != (4 if cfg.solver == ops.SOLVER_P3P else 3):
             raise ValueError("hyp must be [n_hyp, 3] (SOLVER_ARUN) or [n_hyp, 4] (SOLVER_P3P)")
         self._lut, self._hyp = lut, hyp  # keep alive
         self._c = cfg.to_c()
         h = C.c_void_p()
-        check(ctx.lib.sos_frontend_create(ctx._h, C.byref(self._c), ctx._t(lut, torch.int64, "lut"),
-                                          ctx._t(hyp, torch.int32, "hyp"), C.byref(h)))
+        if self.rgbd:
+            check(ctx.lib.sos_frontend_create_rgbd(ctx._h, C.byref(self._c), ctx._t(hyp, torch.int32, "hyp"), C.byref(h)))
+        else:
+            check(ctx.lib.sos_frontend_create(ctx._h, C.byref(self._c), ctx._t(lut, torch.int64, "lut"),
+                                              ctx._t(hyp, torch.int32, "hyp"), C.byref(h)))
         self._h = h
         self._stream = torch.cuda.current_stream(ctx.device)
+
+    def _need(self, rgbd: bool, what: str):
+        if self.rgbd != rgbd:
+            raise TypeError(f"{what} needs {'an RGB-D' if rgbd else 'an SOS'} front-end")
 
     def close(self):
         if getattr(self, "_h", None):
@@ -190,6 +246,7 @@ class Frontend:
         return [(nm[i], float(ms[i])) for i in range(n.value)]
 
     def _check_inputs(self, omni, px_top, desc_top, boff_top, px_bot, desc_bot, boff_bot, on_device: bool):
+        self._need(False, "step / submit_host")
         c = self.cfg
         shapes = {
             "omni": ((c.batch, c.src_h, c.src_w, c.channels), (torch.uint8, np.uint8)),
@@ -280,6 +337,7 @@ class Frontend:
         """Detect the features inside the step, as features.FeatureFront does: masks uint8 [n_buckets, pano_rows,
         pano_cols] per view (numpy or torch), goodFeaturesToTrack(maxCorners = corners_per_bucket, quality_level,
         min_distance) per mask after an optional 11 x 11 median, then ORB description."""
+        self._need(False, "set_detector")
         c = self.cfg
         ms = []
         for name, m in (("masks_top", masks_top), ("masks_bot", masks_bot)):
@@ -293,6 +351,7 @@ class Frontend:
         check(self.ctx.lib.sos_frontend_set_detector(self._h, C.byref(d), *(self.ctx._t(m, torch.uint8, "masks") for m in ms)))
 
     def _check_omni(self, omni, on_device: bool):
+        self._need(False, "step_images / submit_host_images")
         c = self.cfg
         shape = (c.batch, c.src_h, c.src_w, c.channels)
         if tuple(omni.shape) != shape:
@@ -326,6 +385,7 @@ class Frontend:
 
     def host_images_bytes(self) -> int:
         """H2D bytes of one submit_host_images: host_bytes() without the feature arrays."""
+        self._need(False, "host_images_bytes")
         c = self.cfg
         h2d, _ = self.host_bytes()
         return h2d - c.batch * (2 * c.max_feat_per_view * (2 * 4 + 32) + 2 * (c.n_buckets + 1) * 4)
@@ -333,6 +393,7 @@ class Frontend:
     def features(self) -> dict:
         """Zero-copy torch views of the features the last images-in step detected (layout of `step`'s inputs, desc as
         uint8 [batch, max_feat_per_view, 32]) and detect_stats int32 [batch, 2, 4] (valid until close())."""
+        self._need(False, "features")
         f = _Features()
         check(self.ctx.lib.sos_frontend_get_features(self._h, C.byref(f)))
         c = self.cfg
@@ -346,29 +407,85 @@ class Frontend:
             out[name] = torch.as_tensor(_DeviceArray(getattr(f, name), shape, _TYPES[kind][0], self), device=self.ctx.device)
         return out
 
+    # -- RGB-D steps ---------------------------------------------------------------------------------------------------
+    def _check_rgbd(self, depth, px, desc, n_kp, on_device: bool):
+        self._need(True, "step_rgbd / submit_host_rgbd")
+        c = self.cfg
+        shapes = {"depth": ((c.batch, c.height, c.width), (torch.float32, np.float32)),
+                  "px": ((c.batch, c.max_kp, 2), (torch.float32, np.float32)),
+                  "desc": ((c.batch, c.max_kp, 32), (torch.uint8, np.uint8)),
+                  "n_kp": ((c.batch,), (torch.int32, np.int32))}
+        ptrs = []
+        for k, v in (("depth", depth), ("px", px), ("desc", desc), ("n_kp", n_kp)):
+            shape, (tdt, ndt) = shapes[k]
+            if tuple(v.shape) != shape:
+                raise ValueError(f"{k}: expected shape {shape}, got {tuple(v.shape)}")
+            if on_device:
+                ptrs.append(self.ctx._t(v, tdt, k))
+                continue
+            if isinstance(v, torch.Tensor):
+                if v.is_cuda or v.dtype != tdt or not v.is_contiguous():
+                    raise TypeError(f"{k}: expected a contiguous host tensor of {tdt}")
+                ptrs.append(v.data_ptr())
+            else:
+                if v.dtype != ndt or not v.flags.c_contiguous:
+                    raise TypeError(f"{k}: expected a C-contiguous host array of {ndt}")
+                ptrs.append(v.ctypes.data)
+            if k == "n_kp":
+                # host path: the counts are at hand, so refuse what the device path can only clamp to [0, max_kp]
+                n = np.asarray(v)
+                if n.min() < 0 or n.max() > c.max_kp:
+                    raise ValueError(f"n_kp must lie in [0, max_kp = {c.max_kp}], got [{int(n.min())}, {int(n.max())}]")
+        return ptrs
+
+    def step_rgbd(self, depth, px, desc, n_kp):
+        """Asynchronous RGB-D step on device tensors: depth [batch, height, width] float32, px [batch, max_kp, 2] float32,
+        desc [batch, max_kp, 32] uint8, n_kp [batch] int32 (read on the device and clamped to [0, max_kp]); results are
+        read through `buffers()`."""
+        p = self._check_rgbd(depth, px, desc, n_kp, True)
+        self.ctx._sync_stream()
+        check(self.ctx.lib.sos_frontend_step_rgbd(self._h, *p))
+
+    def submit_host_rgbd(self, depth, px, desc, n_kp) -> int:
+        """RGB-D step on host arrays (pinned for full copy bandwidth; whole depth maps are uploaded).  -> ticket for
+        wait_host."""
+        p = self._check_rgbd(depth, px, desc, n_kp, False)
+        t = C.c_int()
+        self.ctx._sync_stream()
+        check(self.ctx.lib.sos_frontend_submit_host_rgbd(self._h, *p, C.byref(t)))
+        return t.value
+
+    def step_host_rgbd(self, depth, px, desc, n_kp):
+        return self.wait_host(self.submit_host_rgbd(depth, px, desc, n_kp))
+
     def buffers(self) -> dict:
-        """Zero-copy torch views of the device buffers (valid until close())."""
+        """Zero-copy torch views of the device buffers (valid until close()).  An RGB-D front-end has one view and no
+        panorama / stereo / second-view / camera-index / overflow buffers (they are absent from the dict)."""
         b = _Buffers()
         check(self.ctx.lib.sos_frontend_get_buffers(self._h, C.byref(b)))
         c = self.cfg
-        B, cap, slots, F, S = c.batch, c.cap, c.batch + 1, c.max_feat_per_view, c.batch * c.n_buckets
+        V = int(b.views)
+        B, cap, slots = c.batch, int(b.cap), c.batch + 1
+        F, S = (0, 0) if self.rgbd else (c.max_feat_per_view, c.batch * c.n_buckets)
         shapes = {
-            "pano": (B, 2, c.pano_rows, c.pano_cols, c.channels),
+            "pano": None if self.rgbd else (B, 2, c.pano_rows, c.pano_cols, c.channels),
             "st_q_start": (S,), "st_q_len": (S,), "st_t_start": (S,), "st_t_len": (S,),
             "st_idx0": (B * F,), "st_d0": (B * F,), "st_pair_q": (B * F,), "st_pair_t": (B * F,), "st_pair_d": (B * F,),
-            "st_pair_count": (S,), "uv_c": (2, slots * cap, 2), "uv_top": (slots, cap, 2), "uv_bot": (slots, cap, 2),
+            "st_pair_count": (S,), "uv_c": (V, slots * cap, 2), "uv_top": (slots, cap, 2), "uv_bot": (slots, cap, 2),
             "b_top": (slots, cap, 3), "b_bot": (slots, cap, 3), "xyz": (slots, cap, 3), "src_top": (slots, cap),
-            "src_bot": (slots, cap), "n": (slots,), "desc_c": (2, slots, cap, 8),
-            "tm_q_start": (2 * B,), "tm_q_len": (2 * B,), "tm_t_start": (2 * B,), "tm_t_len": (2 * B,),
-            "tm_idx0": (2 * slots * cap,), "tm_d0": (2 * slots * cap,), "tm_pair_q": (2 * slots * cap,),
-            "tm_pair_t": (2 * slots * cap,), "tm_pair_d": (2 * slots * cap,), "tm_pair_count": (2 * B,),
-            "p_ref": (B, 2 * cap, 3), "p_cur": (B, 2 * cap, 3), "f_cur": (B, 2 * cap, 3), "cam": (B, 2 * cap),
+            "src_bot": (slots, cap), "n": (slots,), "desc_c": (V, slots, cap, 8),
+            "tm_q_start": (V * B,), "tm_q_len": (V * B,), "tm_t_start": (V * B,), "tm_t_len": (V * B,),
+            "tm_idx0": (V * slots * cap,), "tm_d0": (V * slots * cap,), "tm_pair_q": (V * slots * cap,),
+            "tm_pair_t": (V * slots * cap,), "tm_pair_d": (V * slots * cap,), "tm_pair_count": (V * B,),
+            "p_ref": (B, V * cap, 3), "p_cur": (B, V * cap, 3), "f_cur": (B, V * cap, 3), "cam": (B, V * cap),
             "n_corr": (B,), "n_corr_top": (B,), "ransac_pose": (B, 3, 4), "pose": (B, 3, 4), "best_hyp": (B,),
-            "best_count": (B,), "n_refit": (B,), "inlier_mask": (B, 2 * cap), "stats": (B, 4), "refine_stats": (B, 4), "ref_slot": (B,),
+            "best_count": (B,), "n_refit": (B,), "inlier_mask": (B, V * cap), "stats": (B, 4), "refine_stats": (B, 4), "ref_slot": (B,),
             "overflow": (B,),
         }
         out = {}
         for name, kind in _BUF_FIELDS:
+            if not getattr(b, name):
+                continue
             typestr, _ = _TYPES[kind]
             out[name] = torch.as_tensor(_DeviceArray(getattr(b, name), shapes[name], typestr, self), device=self.ctx.device)
         out["launches_per_step"] = int(b.launches_per_step)

@@ -267,3 +267,104 @@ def render_omni(rig: Rig, scene: Scene, T_c_wrt_w: np.ndarray, lift=None) -> np.
         iv = np.mod(np.floor(hit[np.arange(len(d)), b] / cell).astype(int), T)
         img[m] = scene.texture[face, iu, iv]
     return img
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# RGB-D sequences (BASELINE configuration 5, demo_vo_rgbd.py)
+# ---------------------------------------------------------------------------------------------------------------
+RGBD_FIELDS = ("fx", "fy", "center_x", "center_y", "focal_length_m", "depth_is_Z")
+
+
+@dataclass
+class RgbdSequence:
+    cam: dict                  # RGBD_FIELDS -> value (RGBDCamModel's intrinsics, camera_models.py:752-779)
+    trajectory: np.ndarray     # T_C_wrt_W [n, 4, 4]
+    landmarks: np.ndarray      # [L, 3] world points
+    frames: list               # per frame: depth [480, 640] float32, px [n, 2] float32, desc [n, 32] uint8, landmark [n]
+                               # int64 (-1 = distractor)
+    background: float = 0.0
+
+    def cam_vector(self) -> np.ndarray:
+        return np.array([float(self.cam[k]) for k in RGBD_FIELDS], np.float64)
+
+    def inputs(self, ids, max_kp: int) -> dict:
+        """The frames `ids` as the RGB-D front-end's step inputs: depth [B,h,w] f32, px [B,max_kp,2] f32, desc
+        [B,max_kp,32] u8 (rows past a frame's keypoints are zero), n_kp [B] int32."""
+        fr = [self.frames[i] for i in ids]
+        h, w = fr[0]["depth"].shape
+        out = dict(depth=np.stack([f["depth"] for f in fr]), px=np.zeros((len(fr), max_kp, 2), np.float32),
+                   desc=np.zeros((len(fr), max_kp, 32), np.uint8), n_kp=np.zeros(len(fr), np.int32))
+        for b, f in enumerate(fr):
+            n = min(len(f["px"]), max_kp)
+            out["px"][b, :n], out["desc"][b, :n], out["n_kp"][b] = f["px"][:n], f["desc"][:n], n
+        return out
+
+
+def rgbd_depth_value(cam: dict, Z: np.ndarray, u: np.ndarray, v: np.ndarray) -> np.ndarray:
+    """What the sensor stores at integer pixel (u, v) for a point at depth Z: Z itself, or for radial maps the distance
+    along the pixel's ray, the inverse of RGBDCamModel.get_depth_Z (camera_models.py:781-799)."""
+    if cam["depth_is_Z"]:
+        return np.asarray(Z, np.float64)
+    ray = np.sqrt(((u - cam["center_x"]) / cam["fx"]) ** 2 + ((v - cam["center_y"]) / cam["fy"]) ** 2 + 1.0)
+    return Z * ray
+
+
+def make_rgbd_sequence(n_frames: int, n_kp: int = 2000, depth_is_Z: bool = True, seed: int = 0, flip: float = 0.04,
+                       distractors: float = 0.25, width: int = 640, height: int = 480,
+                       background: float = 0.0) -> RgbdSequence:
+    """A pinhole RGB-D camera moving along make_trajectory through a room of landmarks (walls, and points floating inside
+    at 0.7 .. 3 m), intrinsics of demo_vo_rgbd.py: fx = fy = 525 for Z depth maps, 554.256258 for radial ones (the
+    synthetic branch), c = (319.5, 239.5).
+
+    Per frame, n_kp keypoints in random order: about (1 - distractors) of them are landmarks in view (pixel = the float32
+    projection, descriptor = the landmark's with per-view bit flips of probability `flip`), the rest distractors (uniform
+    pixel, random descriptor); the landmarks chosen are the strongest in view by a fixed per-landmark strength, so that
+    consecutive frames share most of them.  The depth map is `background` everywhere except at the truncated pixel of every
+    landmark keypoint, which holds that landmark's depth; of two landmarks that truncate to the same pixel the nearer
+    one (then the lower id) is kept and the other is not a keypoint.  The default background 0 is "no reading": a keypoint
+    there has no 3D point (camera_models.py:846), so distractors mostly drop out at the range gate and the temporal
+    correspondences are nearly outlier-free (one outlier inside the 5 degree RANSAC threshold already pulls the LM pose
+    of the reference's bearing residual away from the true motion)."""
+    cam = dict(fx=525.0 if depth_is_Z else 554.256258, fy=525.0 if depth_is_Z else 554.256258, center_x=319.5,
+               center_y=239.5, focal_length_m=1.0 / 1000.0, depth_is_Z=1.0 if depth_is_Z else 0.0)
+    rng = np.random.default_rng(seed + 3000)
+    half = np.array([4.0, 4.0, 2.5])
+    n_land = max(24 * n_kp, 2000)
+    d = rng.normal(size=(n_land, 3))
+    d /= np.linalg.norm(d, axis=1, keepdims=True)
+    walls = d * np.min(half / np.abs(d), axis=1, keepdims=True)
+    inside = d * rng.uniform(0.7, 3.0, (n_land, 1))
+    land = np.where((np.arange(n_land) % 5 < 3)[:, None], walls, inside)   # 60 % walls, 40 % inside
+    land_desc = rng.integers(0, 256, (n_land, 32), dtype=np.uint8)
+    strength = rng.random(n_land)      # a detector finds the same strong corners again from frame to frame
+    traj = make_trajectory(n_frames, seed)
+    n_true = int(round(n_kp * (1.0 - distractors)))
+    frames = []
+    for fi, T in enumerate(traj):
+        fr = np.random.default_rng([seed, fi, 17])
+        P = (land - T[:3, 3]) @ T[:3, :3]                     # R^T (p - t): world -> camera
+        Z = P[:, 2]
+        with np.errstate(divide="ignore", invalid="ignore"):
+            uv = np.stack([cam["fx"] * P[:, 0] / Z + cam["center_x"], cam["fy"] * P[:, 1] / Z + cam["center_y"]], 1)
+        uv32 = uv.astype(np.float32)
+        tu, tv = np.trunc(uv32[:, 0]), np.trunc(uv32[:, 1])
+        vis = (Z > 0.5) & (tu >= 0) & (tu < width) & (tv >= 0) & (tv < height)
+        vis_ids = np.flatnonzero(vis)
+        ids = vis_ids[np.argsort(-strength[vis_ids], kind="stable")[:n_true]]   # the strongest corners in view
+        # one landmark per truncated pixel: nearest first, then lowest id
+        pix = tv[ids].astype(np.int64) * width + tu[ids].astype(np.int64)
+        order = np.lexsort((ids, Z[ids]))
+        _, first = np.unique(pix[order], return_index=True)
+        ids = ids[np.sort(order[first])]
+        ui, vi = tu[ids].astype(np.int64), tv[ids].astype(np.int64)
+        depth = np.full((height, width), background, np.float32)
+        depth[vi, ui] = rgbd_depth_value(cam, Z[ids], ui, vi).astype(np.float32)
+        n_dis = n_kp - len(ids)
+        px = np.concatenate([uv32[ids], np.stack([fr.uniform(0, width, n_dis), fr.uniform(0, height, n_dis)], 1)])
+        px = px.astype(np.float32)
+        desc = np.concatenate([land_desc[ids] ^ np.packbits(fr.random((len(ids), 256)) < flip, axis=1),
+                               fr.integers(0, 256, (n_dis, 32), dtype=np.uint8)])
+        lid = np.concatenate([ids, np.full(n_dis, -1)]).astype(np.int64)
+        perm = fr.permutation(n_kp)
+        frames.append(dict(depth=depth, px=px[perm], desc=desc[perm], landmark=lid[perm]))
+    return RgbdSequence(cam, traj, land, frames, background)
